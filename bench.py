@@ -2,6 +2,7 @@
 """bench.py -- env-steps/sec of the batched RLToyEnv step path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N \
         --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
@@ -25,6 +26,10 @@ Prints ONE JSON line (rank 0):
   e2e                host buffers in, host buffers out (public API)
   step_api           the gym-style step() call itself, eager and graphed
   cpu_baseline       the reference's own RLToyEnv loop on one host core
+`--dump-outputs DIR` writes what the last timed launch returned (rank 0) as
+DIR/<name>.npy, every step of a fixed, seeded sample of envs, so that two
+builds can be compared output for output (the inputs depend on the arguments
+only).
 `--impl reference` times the reference's RLToyEnv (oracle/_ref, vendored by
 oracle/make_ref.py; else the CPU port oracle/scalar_env.py) on all host cores.
 """
@@ -48,6 +53,7 @@ ALGO_BYTES_ROLLOUT = 22   # SURVEY.md 8d (ii): action in + outputs out
 ALGO_BYTES_STEP = 58      # SURVEY.md 8d table, config C2 single step
 NORMAL_NAMES = {"fp64": "fp64 ziggurat (numpy's Generator.normal algorithm)",
                 "boxmuller": "fp64 Box-Muller", "fast": "fp32 SFU Box-Muller"}
+DUMP_BYTES = 48 << 20     # cap of what --dump-outputs writes
 
 
 def workload_config():
@@ -563,6 +569,31 @@ def parity_check(env, snap, actions, out_rows, idx, n_launches, T, rank, N):
             "oracle_seconds": round(time.perf_counter() - t0, 1)}
 
 
+def dump_outputs(path, out):
+    """Write the [T, N] arrays of one rollout as path/<name>.npy: obs and
+    reward as float64, the flags as float32, restricted to a seeded sample of
+    envs (and of steps, should one env's column alone exceed DUMP_BYTES)."""
+    import numpy as np
+    import torch
+    T, N = out["obs"].shape
+    per_step = 8 + 8 + 4 + 4
+    n_envs = max(1, min(N, DUMP_BYTES // (T * per_step)))
+    n_steps = min(T, DUMP_BYTES // (n_envs * per_step))
+
+    def sample(n, k, seed):
+        if k >= n:
+            return np.arange(n)
+        return np.sort(np.random.default_rng(seed).choice(n, size=k, replace=False))
+    dev = out["obs"].device
+    rows = torch.as_tensor(sample(T, n_steps, 1), device=dev)
+    cols = torch.as_tensor(sample(N, n_envs, 0), device=dev)
+    os.makedirs(path, exist_ok=True)
+    for k, v in out.items():
+        a = v.index_select(0, rows).index_select(1, cols).cpu().numpy()
+        dt = np.float64 if k in ("obs", "reward") else np.float32
+        np.save(os.path.join(path, k + ".npy"), a.astype(dt))
+
+
 def run_gpu_arm(args):
     import numpy as np
     import torch
@@ -651,6 +682,9 @@ def run_gpu_arm(args):
     per_gpu_steps_per_s = N * T / (ms_per_step * 1e-3)
     achieved = per_gpu_steps_per_s * ALGO_BYTES_ROLLOUT / 1e9
     jit_used = env.jit_last_used
+    # the legs below reuse `out`: save the last timed launch's outputs first
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
     # rows of the timed output buffers, for the oracle comparison below
     parity = None
     if snap is not None:
@@ -917,7 +951,14 @@ def main():
     ap.add_argument("--no-jit", action="store_true",
                     help="use the ahead-of-time kernels instead of the "
                          "NVRTC-specialised one")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed launch (a "
+                         "seeded sample of envs, every step) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's outputs")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference_arm(args)

@@ -41,7 +41,12 @@ def main():
             shutil.copytree(s, d, ignore=shutil.ignore_patterns("__pycache__", "*.pyc"))
         else:
             shutil.copy2(s, d)
-    for root, _, files in os.walk(out):
+    # the experiment files tests/test_sweep.py reads (REFERENCE_ROOT/experiments)
+    exps = os.path.join(SRC, "experiments")
+    if os.path.isdir(exps):
+        shutil.copytree(exps, os.path.join(DST, "experiments"),
+                        ignore=shutil.ignore_patterns("__pycache__", "*.pyc"))
+    for root, _, files in os.walk(DST):
         for f in sorted(files):
             p = os.path.join(root, f)
             manifest.append((hashlib.sha256(open(p, "rb").read()).hexdigest(),

@@ -175,15 +175,23 @@ class VectorRLToyEnv:
     def _check(self, rc):
         _lib.check(self._lib, self._ctx, rc)
 
-    def _reseed(self, seed, mask=None):
-        """reset(seed=s) / seed(s) in Philox mode: re-key the streams AND
-        rewind what they are indexed by (global step, episode counters of the
-        envs being reset), so that the same seed gives the same trajectory --
-        the gym reset(seed) contract the reference meets by re-seeding
-        `_np_random`.  CUDA graphs captured before keep the old key baked into
-        their kernel parameters: they refuse to replay (make_graphed_step)."""
+    def _reseed(self, seed, mask=None, rewind=False):
+        """reset(seed=s) / seed(s) in Philox mode: re-key the streams and zero
+        the episode counters of the envs in `mask` (all when None).
+
+        `rewind` (an unmasked reset(seed=s)) also sets the global step back to
+        0, so that the same seed gives the same trajectory -- the gym
+        reset(seed) contract the reference meets by re-seeding `_np_random`.
+        Every env's delay ring and state history are dead at that point.  A
+        masked reset(seed) or a bare seed(s) keeps the step index: the envs
+        it does not reset still find their ring, history and line-window slots
+        from it (slot = step mod depth).  It re-keys every env, so it does not
+        promise a reproducible trajectory.  CUDA graphs captured before keep
+        the old key baked into their kernel parameters: they refuse to replay
+        (make_graphed_step)."""
         self.philox_seed = int(seed) & (2**64 - 1)
-        self._step_index = 0
+        if rewind:
+            self._step_index = 0
         if mask is None:
             self._episode.zero_()
         else:
@@ -407,7 +415,7 @@ class VectorRLToyEnv:
         elif (seed is not None and self.noise == "philox"
               and not options.get("_ctor")):
             # re-keying the counter-based streams is the analogue of re-seeding
-            self._reseed(seed, mask)
+            self._reseed(seed, mask, rewind=mask is None)
         if reset_u is not None:
             reset_u = torch.as_tensor(reset_u, dtype=torch.float64,
                                       device=dev).contiguous()
@@ -434,15 +442,26 @@ class VectorRLToyEnv:
     def _check_state_range(self, states):
         """Caller-supplied discrete states index the tables on the device:
         reject anything outside [0, S) (rows (relevant, irrelevant) with
-        irrelevant_features) instead of reading out of bounds."""
-        hi = [max(t.n_states for t in self.group_tables)]
-        if self._irr:
-            hi.append(max(t.n_states_irr for t in self.group_tables))
+        irrelevant_features) instead of reading out of bounds.  Each env is
+        checked against the state count of its own config group."""
         st = states.reshape(self.num_envs, -1)
-        for k, n in enumerate(hi):
-            col = st[:, k]
-            if bool(((col < 0) | (col >= n)).any()):
-                raise ValueError(f"state out of range [0, {n}) in column {k}")
+        for k in range(2 if self._irr else 1):
+            self._check_column(st[:, k:k + 1], irr=k == 1,
+                               what=f"state in column {k}")
+
+    def _check_column(self, states, irr, what):
+        """Raise unless every entry of row i of `states` [N, k] lies in
+        [0, S) of env i's config group (S of the irrelevant sub-MDP when
+        `irr`): the kernels index that group's tables with it."""
+        n = torch.tensor([t.n_states_irr if irr else t.n_states
+                          for t in self.group_tables], device=states.device)
+        hi = torch.repeat_interleave(
+            n, torch.tensor(self._group_sizes, device=states.device))[:, None]
+        bad = ((states < 0) | (states >= hi)).any(dim=1)
+        if bool(bad.any()):
+            i = int(bad.nonzero()[0, 0])
+            raise ValueError(f"{what} out of range [0, {int(hi[i, 0])}) at env "
+                             f"{i} (its config group's state count)")
 
     def _observe(self, state, image_params=None, reset=False, ctor=False):
         """Underlying state -> observation (identity, dtype_o cast, or the
@@ -684,7 +703,11 @@ class VectorRLToyEnv:
     def set_obs_dtype(self, dtype):
         """Override dtype_o for the observations rollout() / step() write
         (torch.int64 / int32 / uint8): 8 -> 1 byte per env-step of output for
-        the toy state spaces."""
+        the toy state spaces.  Not for image envs: their observations are
+        the images, and the renderer reads the int64 states."""
+        if self.spec.image_representations:
+            raise ValueError("set_obs_dtype: image observations are uint8 "
+                             "images already; the states stay int64")
         assert dtype in self._OBS_CODES
         if dtype == torch.uint8:
             assert max(self.tables.n_states, self.tables.n_states_irr or 0) <= 256
@@ -1047,7 +1070,10 @@ class VectorRLToyEnv:
             self._d2h_stream = torch.cuda.Stream(dev)
             self._stage = {}
         chunk = max(1, min(int(chunk_steps), T))
-        key = (chunk,) + tuple(actions_host.shape[1:]) + (actions_host.dtype,)
+        # the staging mirrors one chunk of the caller's buffers: any change of
+        # their names, dtypes or trailing shapes needs new staging
+        key = (chunk, tuple(actions_host.shape[1:]), actions_host.dtype) + tuple(
+            (k, v.dtype, tuple(v.shape[1:])) for k, v in sorted(out_host.items()))
         if self._stage.get("key") != key:
             acts = [torch.empty((chunk,) + tuple(actions_host.shape[1:]),
                                 dtype=actions_host.dtype, device=dev)
@@ -1312,7 +1338,7 @@ class VectorRLToyEnv:
                     init[i] = self._host_box_sample(self._rng_F[i])
         elif (seed is not None and self.noise == "philox"
               and not options.get("_ctor")):
-            self._reseed(seed, mask)
+            self._reseed(seed, mask, rewind=mask is None)
         if init is not None:
             init = torch.as_tensor(init, device=dev).to(self._real).reshape(
                 N, D).contiguous()
@@ -1533,7 +1559,7 @@ class VectorRLToyEnv:
                         low=np.zeros(nd), high=hi, size=(nd,))).astype(np.int64)
         elif (seed is not None and self.noise == "philox"
               and not options.get("_ctor")):
-            self._reseed(seed, mask)
+            self._reseed(seed, mask, rewind=mask is None)
         if init is not None:
             init = torch.as_tensor(init, device=dev).to(torch.int64).reshape(
                 N, nd).contiguous()
@@ -1699,10 +1725,7 @@ class VectorRLToyEnv:
         if self._irr:
             full = torch.as_tensor(state["curr_state"] if isinstance(state, dict)
                                    else state, device=dev).reshape(N, 2)
-            n_irr = max(t.n_states_irr for t in self.group_tables)
-            if bool(((full[:, 1] < 0) | (full[:, 1] >= n_irr)).any()):
-                raise ValueError(f"irrelevant state out of range [0, {n_irr})")
-            self._cur_irr.copy_(full[:, 1].to(torch.int32))
+            self._check_column(full[:, 1:], irr=True, what="irrelevant state")
             if not isinstance(state, dict):
                 state = full[:, 0]
         if isinstance(state, dict):
@@ -1714,9 +1737,9 @@ class VectorRLToyEnv:
         valid = ~torch.isnan(aug)
         n_valid = valid.to(torch.int32).sum(dim=1)          # trailing entries
         states = torch.nan_to_num(aug, nan=0.0).to(torch.int64)
-        n_rel = max(t.n_states for t in self.group_tables)
-        if bool(((states < 0) | (states >= n_rel)).any()):
-            raise ValueError(f"augmented_state entry out of range [0, {n_rel})")
+        self._check_column(states, irr=False, what="augmented_state entry")
+        if self._irr:  # (only once both columns have passed the checks)
+            self._cur_irr.copy_(full[:, 1].to(torch.int32))
         self._cur.copy_(states[:, -1].to(torch.int32))
         bits = max(1, int(np.ceil(np.log2(max(self.tables.n_states, 2)))))
         key = torch.zeros(N, dtype=torch.int64, device=dev)

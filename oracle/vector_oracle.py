@@ -67,6 +67,10 @@ class VectorDiscreteOracle:
         self.t = np.zeros(self.N, dtype=np.int64)
         self.episode = np.zeros(self.N, dtype=np.int64)
         self.window = [[] for _ in range(self.N)]   # last L states
+        # states since the reset, newest last, at most L + d + 1 (the window
+        # of get_augmented_state)
+        self.H = self.L + self.d + 1
+        self.hist = [[] for _ in range(self.N)]
         self.fifo = [[0.0] * self.d for _ in range(self.N)]
         self.stats = dict(episodes=0, transitions=0, reward=0.0,
                           noisy_transitions=0, abs_reward_noise=0.0,
@@ -92,6 +96,42 @@ class VectorDiscreteOracle:
             self.fifo[i] = [
                 float(ring[(self.step_index - (self.d - k)) % self.d][i])
                 if self.d - k <= self.t[i] else 0.0 for k in range(self.d)]
+
+    def reseed(self, seed, mask=None, rewind=False):
+        """reset(seed=...) / seed() of the CUDA path: a new Philox key and
+        the episode counters of the envs in `mask` (all when None) back to 0.
+        `rewind` (an unmasked reset(seed=...)) also sets the global step back
+        to 0; otherwise the step index carries on.  The per-env FIFO and
+        window here have no phase, so they are the reference for envs that a
+        reseed leaves running."""
+        self.seed = int(seed) & (2**64 - 1)
+        idx = np.arange(self.N) if mask is None else np.nonzero(mask)[0]
+        self.episode[idx] = 0
+        if rewind:
+            self.step_index = 0
+
+    def set_state(self, states):
+        """set_augmented_state with bare states ([N], or [N, 2] rows with
+        irrelevant_features): each env continues as from the start of an
+        episode in that state; episode counters and statistics unchanged."""
+        st = np.asarray(states, dtype=np.int64)
+        for i in range(self.N):
+            s = st[i]
+            if self.irr:
+                s, self.cur1[i] = int(s[0]), int(s[1])
+            self.cur[i] = int(s)
+            self.t[i] = 0
+            self.window[i] = [int(s)]
+            self.hist[i] = [int(s)]
+            self.fifo[i] = [0.0] * self.d
+
+    def augmented_state(self):
+        """get_augmented_state()["augmented_state"]: [N, L + d + 1] float64,
+        oldest first, NaN before the episode start."""
+        out = np.full((self.N, self.H), np.nan)
+        for i, h in enumerate(self.hist):
+            out[i, self.H - len(h):] = h
+        return out
 
     # -- draws -------------------------------------------------------------
     def _reset_u(self, idx):
@@ -131,6 +171,7 @@ class VectorDiscreteOracle:
         self.t[i] = 0
         self.episode[i] += 1
         self.window[i] = [s0]
+        self.hist[i] = [s0]
         self.fifo[i] = [0.0] * self.d
 
     def rollout(self, T, actions=None, replay=None):
@@ -246,6 +287,8 @@ class VectorDiscreteOracle:
                         self.cur1[i] = min(int(np.searchsorted(
                             self.init_cdf1, u1, side="right")), self.S1 - 1)
                 obs[t, i] = (self.cur[i], self.cur1[i]) if self.irr else self.cur[i]
+                if not (self.autoreset and (done or tr)):
+                    self.hist[i] = (self.hist[i] + [int(self.cur[i])])[-self.H:]
         self.step_index += T
         return dict(obs=obs, final_obs=final_obs, reward=reward,
                     terminated=term, truncated=trunc)
@@ -269,8 +312,24 @@ class VectorGroupedOracle:
             self.parts.append(VectorDiscreteOracle(
                 e, n, autoreset=autoreset, horizon=horizon, seed=seed, gids=gids, **kw))
 
-    def reset(self):
-        return np.concatenate([p.reset() for p in self.parts])
+    def _split(self, x):
+        """Per-group slices of an env-major array (None stays None)."""
+        if x is None:
+            return [None] * len(self.parts)
+        x, begin, out = np.asarray(x), 0, []
+        for n in self.sizes:
+            out.append(x[begin:begin + n])
+            begin += n
+        return out
+
+    def reset(self, mask=None, init_state=None):
+        return np.concatenate([
+            p.reset(mask=m, init_state=s) for p, m, s in
+            zip(self.parts, self._split(mask), self._split(init_state))])
+
+    def reseed(self, seed, mask=None, rewind=False):
+        for p, m in zip(self.parts, self._split(mask)):
+            p.reseed(seed, mask=m, rewind=rewind)
 
     def rollout(self, T, actions=None):
         outs, begin = [], 0

@@ -38,6 +38,11 @@ EXPORTED_SYMBOLS = (
 MDPP_MAX_DIM, MDPP_MAX_ORDER, MDPP_MAX_TERM_BOXES = 16, 4, 8
 
 
+def _ptr(t):
+    """Device pointer of a tensor for a struct field or argument (NULL for None)."""
+    return None if t is None else C.c_void_p(t.data_ptr())
+
+
 class DiscreteGroup(C.Structure):
     _fields_ = [
         ("n_states", C.c_int32), ("n_actions", C.c_int32),

@@ -80,6 +80,17 @@ class EnvSpec:
     terminal_cells: Any = None
 
 
+def state_space_kind(config):
+    """"discrete", "continuous" or "grid": the config's state_space_type,
+    lower-cased; {} is the reference's default discrete config (:227-235)."""
+    if config == {}:
+        return "discrete"
+    kind = config["state_space_type"].lower()
+    if kind not in ("discrete", "continuous", "grid"):
+        raise ValueError("Unknown state_space_type")
+    return kind
+
+
 def parse_config(config):
     """Fill defaults exactly like RLToyEnv.__init__ (:227-666)."""
     if config == {}:  # :227-235
@@ -100,10 +111,7 @@ def parse_config(config):
         for k in _SEED_KEYS:
             sp.seed_dict[k] = sp.env_rng.integers(sys.maxsize).item()
 
-    config["state_space_type"] = config["state_space_type"].lower()
-    kind = sp.kind = config["state_space_type"]
-    if kind not in ("discrete", "continuous", "grid"):
-        raise ValueError("Unknown state_space_type")
+    kind = sp.kind = config["state_space_type"] = state_space_kind(config)
     g = config.get
     sp.use_custom_mdp = bool(g("use_custom_mdp", False))
     if sp.use_custom_mdp:

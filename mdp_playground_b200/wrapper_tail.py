@@ -27,10 +27,7 @@ import numpy as np
 import torch
 
 from . import _lib
-
-
-def _ptr(t):
-    return None if t is None else C.c_void_p(t.data_ptr())
+from ._lib import _ptr
 
 
 class VectorGymEnvTail:

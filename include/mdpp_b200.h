@@ -490,6 +490,36 @@ int mdpp_render_discrete(mdpp_ctx* ctx, const mdpp_image_discrete_tables* tb,
                          const mdpp_step_opts* opts, void* cuda_stream);
 #endif
 
+/* Per-group renderer configurations of a heterogeneous launch (config groups
+ * that differ in image_transforms, sh_quant, ro_quant, scale range or state
+ * count): group g renders the envs [env_begin, env_begin + env_count) with
+ * its own tables `tb` (DEVICE pointers, borrowed until the next set call or
+ * mdpp_destroy).  Groups tile the env range in order (at most 65 535) and
+ * agree on width, height and n_sub_images.  The Philox id of env e of group
+ * g is opts->env_id_offset + global_id_base + (e - env_begin), like the step
+ * kernels' (mdpp_discrete_group), so a group's image transforms do not
+ * depend on how the job is sharded.                                          */
+typedef struct mdpp_image_discrete_group {
+  mdpp_image_discrete_tables tb;
+  int64_t env_begin, env_count;
+  int64_t global_id_base;
+} mdpp_image_discrete_group;
+
+#ifndef __CUDACC_RTC__ /* NVRTC sees the types only */
+/* Replaces any earlier set; the descriptors are copied.                      */
+int mdpp_set_image_discrete_groups(mdpp_ctx* ctx,
+                                   const mdpp_image_discrete_group* groups,
+                                   int32_t n_groups);
+/* mdpp_render_discrete with the tables of each image's group: image m is
+ * env (m / n_sub) % n_envs, the same indexing; n_envs must equal the
+ * groups' total.                                                            */
+int mdpp_render_discrete_groups(mdpp_ctx* ctx, const int64_t* states,
+                                const int32_t* params_in, int32_t* params_out,
+                                uint8_t* out, int64_t n_images, int64_t n_envs,
+                                int32_t image_stream, const mdpp_step_opts* opts,
+                                void* cuda_stream);
+#endif
+
 #define MDPP_MAX_STAMP_ROWS 32
 
 typedef struct mdpp_image_continuous_config {
@@ -521,6 +551,28 @@ typedef struct mdpp_image_continuous_config {
 int mdpp_render_continuous(mdpp_ctx* ctx, const mdpp_image_continuous_config* cfg,
                            const void* states, uint8_t* out, int64_t n_images,
                            void* cuda_stream);
+#endif
+
+/* Per-group configurations of continuous and grid image observations (the
+ * target, terminal rectangles, feature bounds and grid lines of each config
+ * group): group g renders the envs [env_begin, env_begin + env_count).
+ * Groups tile the env range in order (at most 65 535) and agree on width,
+ * height, n_sub_images, dim and is_f64.                                      */
+typedef struct mdpp_image_continuous_group {
+  mdpp_image_continuous_config cfg;
+  int64_t env_begin, env_count;
+} mdpp_image_continuous_group;
+
+#ifndef __CUDACC_RTC__ /* NVRTC sees the types only */
+/* Replaces any earlier set; the configurations are copied.                   */
+int mdpp_set_image_continuous_groups(mdpp_ctx* ctx,
+                                     const mdpp_image_continuous_group* groups,
+                                     int32_t n_groups);
+/* mdpp_render_continuous with the configuration of each image's group:
+ * image m is env m % n_envs; n_envs must equal the groups' total.           */
+int mdpp_render_continuous_groups(mdpp_ctx* ctx, const void* states,
+                                  uint8_t* out, int64_t n_images,
+                                  int64_t n_envs, void* cuda_stream);
 #endif
 
 /* ------------------------------------------------------------------------

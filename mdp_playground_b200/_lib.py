@@ -34,6 +34,8 @@ EXPORTED_SYMBOLS = (
     "mdpp_tail_actions", "mdpp_tail_post", "mdpp_tail_image_shift",
     "mdpp_set_continuous_groups",
     "mdpp_set_grid_groups",
+    "mdpp_set_image_discrete_groups", "mdpp_render_discrete_groups",
+    "mdpp_set_image_continuous_groups", "mdpp_render_continuous_groups",
 )
 MDPP_MAX_DIM, MDPP_MAX_ORDER, MDPP_MAX_TERM_BOXES = 16, 4, 8
 
@@ -161,6 +163,11 @@ class ImageDiscreteTables(C.Structure):
     ]
 
 
+class ImageDiscreteGroup(C.Structure):
+    _fields_ = [("tb", ImageDiscreteTables), ("env_begin", C.c_int64),
+                ("env_count", C.c_int64), ("global_id_base", C.c_int64)]
+
+
 MDPP_MAX_STAMP_ROWS = 32
 
 
@@ -178,6 +185,11 @@ class ImageContinuousConfig(C.Structure):
         ("stamp", (C.c_int32 * 2) * MDPP_MAX_STAMP_ROWS),
         ("vline", (C.c_uint64 * 4) * 2), ("hline", (C.c_uint64 * 4) * 2),
     ]
+
+
+class ImageContinuousGroup(C.Structure):
+    _fields_ = [("cfg", ImageContinuousConfig), ("env_begin", C.c_int64),
+                ("env_count", C.c_int64)]
 
 
 MDPP_MAX_GRID_DIMS = 4
@@ -288,6 +300,13 @@ def load():
         C.c_int32, C.POINTER(StepOpts), P]
     lib.mdpp_render_continuous.argtypes = [
         P, C.POINTER(ImageContinuousConfig), P, P, C.c_int64, P]
+    lib.mdpp_set_image_discrete_groups.argtypes = [
+        P, C.POINTER(ImageDiscreteGroup), C.c_int32]
+    lib.mdpp_render_discrete_groups.argtypes = [
+        P, P, P, P, P, C.c_int64, C.c_int64, C.c_int32, C.POINTER(StepOpts), P]
+    lib.mdpp_set_image_continuous_groups.argtypes = [
+        P, C.POINTER(ImageContinuousGroup), C.c_int32]
+    lib.mdpp_render_continuous_groups.argtypes = [P, P, P, C.c_int64, C.c_int64, P]
     lib.mdpp_set_grid_config.argtypes = [P, C.POINTER(GridConfig)]
     lib.mdpp_set_grid_groups.argtypes = [P, C.POINTER(GridGroup), C.c_int32]
     lib.mdpp_grid_rollout.argtypes = [

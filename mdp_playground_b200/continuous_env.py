@@ -115,6 +115,7 @@ class ContinuousEnv(VectorRLToyEnv):
                     "reward_function and image_representations (group %d)" % gi)
             cfgs.append(self._continuous_cfg(s_, s_.config, np_dt))
         c, self._term_lows, self._term_highs = cfgs[0]
+        self._group_terms = [(lo, hi) for _, lo, hi in cfgs]  # (the images')
         line = sp.reward_function == "move_along_a_line"
         # (the key's presence, not its value, turns transition noise on here)
         self.has_pnoise = any(s_.has_transition_noise for s_ in specs)
@@ -124,9 +125,9 @@ class ContinuousEnv(VectorRLToyEnv):
             return bool(self._real == torch.float32 and (
                 (cc.target_is_f64 and cc.dense) or line))
         if G > 1:
-            if sp.image_representations or self.noise == "numpy":
+            if self.noise == "numpy":
                 raise NotImplementedError(
-                    "config_groups of continuous envs: no images, no noise='numpy'")
+                    "config_groups of continuous envs: no noise='numpy'")
             if len({ring64(cc) for cc, _, _ in cfgs}) != 1 or (
                     line and len({s_.sequence_length for s_ in specs}) != 1):
                 raise ValueError(
@@ -230,20 +231,24 @@ class ContinuousEnv(VectorRLToyEnv):
 
     # ------------------------------------------------------------------
     def _init_images(self):
-        sp = self.spec
-        D = sp.state_space_dim
-        assert np.isfinite(sp.state_space_max), \
-            "image observations need a bounded state space"
+        """One renderer configuration per config group: its own target,
+        terminal regions and feature bounds (state_space_max)."""
+        D = self.spec.state_space_dim
         if D not in (2, 4):
             raise NotImplementedError(
                 "continuous image observations: 2 relevant (+ 0 or 2 "
                 "irrelevant) dimensions")
         dt = self._np_real
-        self._img_cfg = self._box_image_cfg(
-            D, np.full((2,), -sp.state_space_max).astype(dt),
-            np.full((2,), sp.state_space_max).astype(dt),
-            list(zip(self._term_lows, self._term_highs)),
-            np.asarray(sp.target_point, dtype=dt), self._real == torch.float64)
+        cfgs = []
+        for s_, (lows, highs) in zip(self._group_specs, self._group_terms):
+            assert np.isfinite(s_.state_space_max), \
+                "image observations need a bounded state space"
+            cfgs.append(self._box_image_cfg(
+                s_, D, np.full((2,), -s_.state_space_max).astype(dt),
+                np.full((2,), s_.state_space_max).astype(dt),
+                list(zip(lows, highs)),
+                np.asarray(s_.target_point, dtype=dt), self._real == torch.float64))
+        self._set_image_groups(cfgs)
 
     def _render_states(self, state):
         return state.to(self._real).contiguous()

@@ -101,6 +101,7 @@ extern "C" void mdpp_destroy(mdpp_ctx* ctx) {
   if (ctx->c_cta_map) cudaFree(ctx->c_cta_map);
   if (ctx->g_groups) cudaFree(ctx->g_groups);
   if (ctx->g_cta_map) cudaFree(ctx->g_cta_map);
+  render_release(ctx);
   delete ctx;
 }
 

@@ -45,6 +45,19 @@ struct mdpp_ctx {
   void* g_cta_map = nullptr;  // CtaMapEntry[g_n_ctas]
   int g_n_groups = 0;
   int64_t g_n_ctas = 0, g_total_envs = 0;
+  // per-group image renderers (mdpp_set_image_discrete_groups /
+  // mdpp_set_image_continuous_groups): the group descriptors and an
+  // env -> group map, one load per image
+  mdpp_image_discrete_group* img_d_groups = nullptr;  // [img_d_n_groups]
+  uint16_t* img_d_env_group = nullptr;                // [img_d_total_envs]
+  mdpp_image_discrete_tables img_d_first;  // group 0's (shared sizes), any-rotate
+  int img_d_n_groups = 0;
+  int64_t img_d_total_envs = 0;
+  mdpp_image_continuous_group* img_c_groups = nullptr;
+  uint16_t* img_c_env_group = nullptr;
+  mdpp_image_continuous_config img_c_first;
+  int img_c_n_groups = 0;
+  int64_t img_c_total_envs = 0;
   // runtime-specialised kernels (jit.cu), keyed by their define string
   std::map<std::string, void*> jit_functions;   // CUfunction
   std::vector<void*> jit_modules;               // CUmodule
@@ -70,6 +83,7 @@ int jit_try_rollout(mdpp_ctx* ctx, RolloutParams& p, int noise_mode,
 struct ContinuousParams;
 int jit_try_continuous(mdpp_ctx* ctx, ContinuousParams& p, cudaStream_t stream);
 void jit_release(mdpp_ctx* ctx);
+void render_release(mdpp_ctx* ctx);  // render.cu: the per-group image descriptors
 int smem_min_steps();  // MDPP_SMEM_MIN_T (default 1): shorter launches skip the smem staging
 int fail(mdpp_ctx* ctx, int code, const std::string& msg);
 int cuda_fail(mdpp_ctx* ctx, cudaError_t e, const char* what);

@@ -12,7 +12,10 @@
 // streaming stores first; the shape is then assembled as column bitmaps of the
 // FINAL image in shared memory and only its non-empty 4-byte words are stored
 // again.  K5: one CTA per (sub-)image, 16 output bytes per thread and store.
+#include <algorithm>
 #include <cstdlib>
+#include <string>
+#include <vector>
 
 #include "internal.h"
 #include "philox.cuh"
@@ -29,7 +32,11 @@ constexpr int kMaskPad = 24;
 constexpr int kMaskCols = kMaskRows + 2 * kMaskPad;
 
 struct RenderDParams {
+  // the tables of a single-config launch; in a grouped launch group 0's
+  // (width, height and n_sub_images are common) with has_rotate = any group's
   mdpp_image_discrete_tables tb;
+  const mdpp_image_discrete_group* groups;  // grouped launch: the descriptors
+  const uint16_t* env_group;                //   and the env -> group map
   const int64_t* states;
   const int32_t* params_in;
   int32_t* params_out;
@@ -94,9 +101,12 @@ __device__ __forceinline__ int scaled_radius(const mdpp_image_discrete_tables& t
 // The scalar set-up of image m (see ImageSetup).  Restates the draw order of
 // the reference (:149-181, :251, :258-259): one Philox call per image, w0
 // scale, w1 / w2 shifts, w3 rotation + flip bits.  Uniform over the warp.
-__device__ __forceinline__ ImageSetup image_setup(const RenderDParams& p, int64_t m,
+// `tb`: the image's tables; `id_base`: the Philox id of env 0 of them (mod
+// 2^32), the id of env e being id_base + e.
+__device__ __forceinline__ ImageSetup image_setup(const RenderDParams& p,
+                                                  const mdpp_image_discrete_tables& tb,
+                                                  uint32_t id_base, int64_t m,
                                                   int lane, double thr0) {
-  const mdpp_image_discrete_tables& tb = p.tb;
   const int W = tb.width, H = tb.height;
   ImageSetup g;
   int state = (int)p.states[m];
@@ -113,7 +123,7 @@ __device__ __forceinline__ ImageSetup image_setup(const RenderDParams& p, int64_
     else if (tb.n_sub_images > 2) { sub = e % (uint32_t)tb.n_sub_images; e /= (uint32_t)tb.n_sub_images; }
     uint32_t t_rel = 0;
     if (e >= (uint32_t)p.n_envs) { t_rel = e / (uint32_t)p.n_envs; e -= t_rel * (uint32_t)p.n_envs; }
-    const uint32_t gid = (uint32_t)p.env_id_offset + e;
+    const uint32_t gid = id_base + e;
     const uint64_t step = p.step_index + (uint64_t)t_rel +
                           (p.step_index_dev ? *p.step_index_dev : 0ull);
     U4 w = philox4x32_10(gid, (uint32_t)step, (uint32_t)(step >> 32),
@@ -207,11 +217,19 @@ __device__ __forceinline__ ImageSetup image_setup(const RenderDParams& p, int64_
 // us unrotated; 8 CTAs at 59 registers: 39.9 / 32.6 us.  Two warps or one per
 // CTA instead of four, so that a slow image does not hold its neighbours'
 // slots: 39.7 / 39.5 us rotated, i.e. within 1-2 %.)
-template <int V>  // experiment switches (MDPP_RENDER_VARIANT); none at present
+//
+// kGrouped: the tables come from the image's config group (p.groups, found
+// through p.env_group) instead of the kernel parameters.  Each warp copies
+// its group's 128-byte descriptor to shared memory before the
+// griddepcontrol.wait below -- static tables, like r_thresholds -- so the
+// overlap with the step kernel is kept.
+static_assert(sizeof(mdpp_image_discrete_group) == 128, "one word per lane");
+template <int V, bool kGrouped>  // V: experiment switches (MDPP_RENDER_VARIANT); none at present
 __global__ void __launch_bounds__(kRBlock, 10)
 render_discrete_kernel(const __grid_constant__ RenderDParams p) {
   __shared__ uint64_t mask_s[kImagesPerCta][kMaskCols];    // polygon column bitmaps
   __shared__ uint64_t fmask_s[kImagesPerCta][kRotCols][2];  // ... of the final image
+  __shared__ mdpp_image_discrete_group desc_s[kGrouped ? kImagesPerCta : 1];
   // The next kernel of the stream, when launched with programmatic stream
   // serialisation (the next step kernel), may start its prologue now; it
   // still waits for this grid to complete before touching the env state.
@@ -222,8 +240,16 @@ render_discrete_kernel(const __grid_constant__ RenderDParams p) {
   if (m >= p.n_images) return;  // whole warp; only warp-level barriers below
   uint64_t* mask = mask_s[warp] + kMaskPad;
   uint64_t (*fmask)[2] = fmask_s[warp];
-  const mdpp_image_discrete_tables& tb = p.tb;
-  const int W = tb.width, H = tb.height;
+  int gi = 0;
+  if (kGrouped) {  // the image's env (see image_setup) -> its group; used below
+    uint32_t e = (uint32_t)m;
+    if (p.tb.n_sub_images == 2) e >>= 1;
+    else if (p.tb.n_sub_images > 2) e /= (uint32_t)p.tb.n_sub_images;
+    if (e >= (uint32_t)p.n_envs) e %= (uint32_t)p.n_envs;  // a [T][N] block
+    gi = p.env_group[e];
+  }
+  const mdpp_image_discrete_tables& tb = kGrouped ? desc_s[warp].tb : p.tb;
+  const int W = p.tb.width, H = p.tb.height;
   const int total = W * H;
   uint8_t* out = p.out + m * (int64_t)total;
   // 16-byte zero fill + aligned 4-byte words per column
@@ -252,6 +278,13 @@ render_discrete_kernel(const __grid_constant__ RenderDParams p) {
   for (int w = lane; w < 2 * kRotCols; w += 32) (&fmask[0][0])[w] = 0ull;
   if (lane < kMaskPad) { mask[-1 - lane] = 0ull; mask[kMaskRows + lane] = 0ull; }
   // (static tables may be read ahead of the wait below)
+  uint32_t id_base = (uint32_t)p.env_id_offset;
+  if (kGrouped) {
+    reinterpret_cast<uint32_t*>(&desc_s[warp])[lane] =
+        reinterpret_cast<const uint32_t*>(p.groups + gi)[lane];
+    __syncwarp();
+    id_base += (uint32_t)(desc_s[warp].global_id_base - desc_s[warp].env_begin);
+  }
   const double thr0 = tb.has_scale && lane < tb.n_radii - 1 ? tb.r_thresholds[lane]
                                                             : __longlong_as_double(0x7ff0000000000000ll);
   // launched with MDPP_LAUNCH_OVERLAP_PREVIOUS: everything above overlapped the
@@ -259,7 +292,7 @@ render_discrete_kernel(const __grid_constant__ RenderDParams p) {
   // it now.  Returns at once in an ordinary launch.
   asm volatile("griddepcontrol.wait;" ::: "memory");
 
-  const ImageSetup g = image_setup(p, m, lane, thr0);
+  const ImageSetup g = image_setup(p, tb, id_base, m, lane, thr0);
   __syncwarp();  // fmask is cleared
   const int sw = g.sw, sh = g.sh, rot = g.rot, flip = g.flip;
   const int xbase = g.xbase, ybase = g.ybase;
@@ -383,18 +416,37 @@ render_discrete_kernel(const __grid_constant__ RenderDParams p) {
 }
 
 struct RenderCParams {
+  // single-config launch: the configuration; grouped: group 0's (the sizes,
+  // dim and dtype are common)
   mdpp_image_continuous_config cfg;
+  const mdpp_image_continuous_group* groups;  // grouped launch: the configs
+  const uint16_t* env_group;                  //   and the env -> group map
+  int64_t n_envs;
   const void* states;
   uint8_t* out;
 };
 
-template <typename R>
+// kGrouped: the CTA first stages its image's group configuration in shared
+// memory; everything after that is the single-config kernel.
+template <typename R, bool kGrouped>
 __global__ void __launch_bounds__(kRBlock)
 render_continuous_kernel(const __grid_constant__ RenderCParams p) {
-  const mdpp_image_continuous_config& c = p.cfg;
+  constexpr int kCfgWords = sizeof(mdpp_image_continuous_config) / 4;
+  static_assert(sizeof(mdpp_image_continuous_config) % 16 == 0, "uint4 copy");
+  __shared__ __align__(16) uint32_t cfg_s[kGrouped ? kCfgWords : 1];
+  const int n_sub = p.cfg.n_sub_images;
+  const int64_t m = blockIdx.x / n_sub;
+  const int sub = blockIdx.x % n_sub;  // 0 relevant, 1 irrelevant
+  if (kGrouped) {
+    const int gi = p.env_group[m % p.n_envs];
+    const uint4* src = reinterpret_cast<const uint4*>(&p.groups[gi].cfg);
+    for (int i = threadIdx.x; i < kCfgWords / 4; i += kRBlock)
+      reinterpret_cast<uint4*>(cfg_s)[i] = src[i];
+    __syncthreads();
+  }
+  const mdpp_image_continuous_config& c =
+      kGrouped ? *reinterpret_cast<const mdpp_image_continuous_config*>(cfg_s) : p.cfg;
   const int W = c.width, H = c.height;
-  const int64_t m = blockIdx.x / c.n_sub_images;
-  const int sub = blockIdx.x % c.n_sub_images;  // 0 relevant, 1 irrelevant
   const R* st = reinterpret_cast<const R*>(p.states) + m * c.dim;
   // convert_to_pixel (:248-277): ((v - lo) / (hi - lo)) in dtype_s, promoted
   // to float64 by the integer image shape, truncated
@@ -461,6 +513,134 @@ render_continuous_kernel(const __grid_constant__ RenderCParams p) {
 
 using namespace mdpp;
 
+namespace {
+
+// The parameters of a discrete render call that do not depend on where the
+// tables come from.
+void fill_render_params(RenderDParams& p, const int64_t* states,
+                        const int32_t* params_in, int32_t* params_out,
+                        uint8_t* out, int64_t n_images, int64_t n_envs,
+                        int32_t image_stream, const mdpp_step_opts* opts) {
+  p.states = states;
+  p.params_in = params_in;
+  p.params_out = params_out;
+  p.out = out;
+  p.n_images = n_images;
+  p.n_envs = n_envs;
+  p.k0 = (uint32_t)opts->seed;
+  p.k1 = (uint32_t)(opts->seed >> 32);
+  p.stream = (uint32_t)image_stream;
+  p.step_index = opts->step_index;
+  p.step_index_dev = opts->step_index_dev;
+  p.env_id_offset = opts->env_id_offset;
+}
+
+template <bool kGrouped>
+int launch_render_discrete(mdpp_ctx* ctx, const RenderDParams& p,
+                           const mdpp_step_opts* opts, void* cuda_stream) {
+  const unsigned grid = (unsigned)((p.n_images + kImagesPerCta - 1) / kImagesPerCta);
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(grid);
+  cfg.blockDim = dim3(kRBlock);
+  cfg.stream = (cudaStream_t)cuda_stream;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = (opts->flags & MDPP_LAUNCH_OVERLAP_PREVIOUS) ? 1 : 0;
+  static const int variant = [] {  // experiment knob
+    const char* e = std::getenv("MDPP_RENDER_VARIANT");
+    return e ? std::atoi(e) : 0;
+  }();
+  switch (variant) {
+    case 1: MDPP_CUDA(ctx, cudaLaunchKernelEx(&cfg, render_discrete_kernel<1, kGrouped>, p)); break;
+    default: MDPP_CUDA(ctx, cudaLaunchKernelEx(&cfg, render_discrete_kernel<0, kGrouped>, p));
+  }
+  MDPP_CUDA(ctx, cudaGetLastError());
+  return MDPP_OK;
+}
+
+template <bool kGrouped>
+int launch_render_continuous(mdpp_ctx* ctx, const RenderCParams& p,
+                             int64_t n_images, void* cuda_stream) {
+  const unsigned grid = (unsigned)(n_images * p.cfg.n_sub_images);
+  if (p.cfg.is_f64)
+    render_continuous_kernel<double, kGrouped><<<grid, kRBlock, 0, (cudaStream_t)cuda_stream>>>(p);
+  else
+    render_continuous_kernel<float, kGrouped><<<grid, kRBlock, 0, (cudaStream_t)cuda_stream>>>(p);
+  MDPP_CUDA(ctx, cudaGetLastError());
+  return MDPP_OK;
+}
+
+// The checks every group set shares: the groups tile [0, N) in order, at most
+// 65 535 of them (the env -> group map is uint16).  Builds that map.
+template <typename G>
+int tile_groups(mdpp_ctx* ctx, const char* what, const G* groups, int32_t n,
+                std::vector<uint16_t>& env_group) {
+  if (!groups || n < 1)
+    return fail(ctx, MDPP_EINVAL, std::string(what) + ": need at least one group");
+  if (n > 65535)
+    return fail(ctx, MDPP_EINVAL, std::string(what) + ": at most 65535 groups");
+  int64_t next = 0;
+  for (int g = 0; g < n; ++g) {
+    if (groups[g].env_begin != next || groups[g].env_count < 0)
+      return fail(ctx, MDPP_EINVAL, std::string(what) + ": group " + std::to_string(g) +
+                  " does not continue the tiling of the env range (groups must tile "
+                  "[0, N) contiguously, in order)");
+    next += groups[g].env_count;
+  }
+  if (next < 1) return fail(ctx, MDPP_EINVAL, std::string(what) + ": no environments");
+  env_group.resize((size_t)next);
+  for (int g = 0; g < n; ++g)
+    std::fill(env_group.begin() + groups[g].env_begin,
+              env_group.begin() + groups[g].env_begin + groups[g].env_count, (uint16_t)g);
+  return MDPP_OK;
+}
+
+// Context-owned copies of the descriptors and of the env -> group map.
+template <typename G>
+int upload_groups(mdpp_ctx* ctx, const G* groups, int32_t n,
+                  const std::vector<uint16_t>& env_group, G** d_groups,
+                  uint16_t** d_env_group) {
+  MDPP_CUDA(ctx, cudaSetDevice(ctx->device));
+  MDPP_CUDA(ctx, cudaMalloc(d_groups, (size_t)n * sizeof(G)));
+  MDPP_CUDA(ctx, cudaMemcpy(*d_groups, groups, (size_t)n * sizeof(G),
+                            cudaMemcpyHostToDevice));
+  MDPP_CUDA(ctx, cudaMalloc(d_env_group, env_group.size() * sizeof(uint16_t)));
+  MDPP_CUDA(ctx, cudaMemcpy(*d_env_group, env_group.data(),
+                            env_group.size() * sizeof(uint16_t), cudaMemcpyHostToDevice));
+  return MDPP_OK;
+}
+
+void release_discrete_groups(mdpp_ctx* ctx) {
+  if (ctx->img_d_groups) cudaFree(ctx->img_d_groups);
+  if (ctx->img_d_env_group) cudaFree(ctx->img_d_env_group);
+  ctx->img_d_groups = nullptr;
+  ctx->img_d_env_group = nullptr;
+  ctx->img_d_n_groups = 0;
+  ctx->img_d_total_envs = 0;
+}
+
+void release_continuous_groups(mdpp_ctx* ctx) {
+  if (ctx->img_c_groups) cudaFree(ctx->img_c_groups);
+  if (ctx->img_c_env_group) cudaFree(ctx->img_c_env_group);
+  ctx->img_c_groups = nullptr;
+  ctx->img_c_env_group = nullptr;
+  ctx->img_c_n_groups = 0;
+  ctx->img_c_total_envs = 0;
+}
+
+inline int n_sub_of(const mdpp_image_discrete_tables& tb) {
+  return tb.n_sub_images < 1 ? 1 : tb.n_sub_images;
+}
+
+}  // namespace
+
+void mdpp::render_release(mdpp_ctx* ctx) {
+  release_discrete_groups(ctx);
+  release_continuous_groups(ctx);
+}
+
 extern "C" int mdpp_render_discrete(mdpp_ctx* ctx,
                                     const mdpp_image_discrete_tables* tb,
                                     const int64_t* states,
@@ -483,38 +663,11 @@ extern "C" int mdpp_render_discrete(mdpp_ctx* ctx,
   MDPP_CUDA(ctx, cudaSetDevice(ctx->device));
   RenderDParams p;
   p.tb = *tb;
-  p.states = states;
-  p.params_in = params_in;
-  p.params_out = params_out;
-  p.out = out;
-  p.n_images = n_images;
-  p.n_envs = n_envs;
-  p.k0 = (uint32_t)opts->seed;
-  p.k1 = (uint32_t)(opts->seed >> 32);
-  p.stream = (uint32_t)image_stream;
-  p.step_index = opts->step_index;
-  p.step_index_dev = opts->step_index_dev;
-  p.env_id_offset = opts->env_id_offset;
-  const unsigned grid = (unsigned)((n_images + kImagesPerCta - 1) / kImagesPerCta);
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(kRBlock);
-  cfg.stream = (cudaStream_t)cuda_stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = (opts->flags & MDPP_LAUNCH_OVERLAP_PREVIOUS) ? 1 : 0;
-  static const int variant = [] {  // experiment knob
-    const char* e = std::getenv("MDPP_RENDER_VARIANT");
-    return e ? std::atoi(e) : 0;
-  }();
-  switch (variant) {
-    case 1: MDPP_CUDA(ctx, cudaLaunchKernelEx(&cfg, render_discrete_kernel<1>, p)); break;
-    default: MDPP_CUDA(ctx, cudaLaunchKernelEx(&cfg, render_discrete_kernel<0>, p));
-  }
-  MDPP_CUDA(ctx, cudaGetLastError());
-  return MDPP_OK;
+  p.groups = nullptr;
+  p.env_group = nullptr;
+  fill_render_params(p, states, params_in, params_out, out, n_images, n_envs,
+                     image_stream, opts);
+  return launch_render_discrete<false>(ctx, p, opts, cuda_stream);
 }
 
 extern "C" int mdpp_render_continuous(mdpp_ctx* ctx,
@@ -532,13 +685,125 @@ extern "C" int mdpp_render_continuous(mdpp_ctx* ctx,
   MDPP_CUDA(ctx, cudaSetDevice(ctx->device));
   RenderCParams p;
   p.cfg = *cfg;
+  p.groups = nullptr;
+  p.env_group = nullptr;
+  p.n_envs = 0;
   p.states = states;
   p.out = out;
-  const unsigned grid = (unsigned)(n_images * cfg->n_sub_images);
-  if (cfg->is_f64)
-    render_continuous_kernel<double><<<grid, kRBlock, 0, (cudaStream_t)cuda_stream>>>(p);
-  else
-    render_continuous_kernel<float><<<grid, kRBlock, 0, (cudaStream_t)cuda_stream>>>(p);
-  MDPP_CUDA(ctx, cudaGetLastError());
+  return launch_render_continuous<false>(ctx, p, n_images, cuda_stream);
+}
+
+extern "C" int mdpp_set_image_discrete_groups(mdpp_ctx* ctx,
+                                              const mdpp_image_discrete_group* groups,
+                                              int32_t n_groups) {
+  if (!ctx) return MDPP_EINVAL;
+  std::vector<uint16_t> env_group;
+  int rc = tile_groups(ctx, "set_image_discrete_groups", groups, n_groups, env_group);
+  if (rc) return rc;
+  const mdpp_image_discrete_tables& t0 = groups[0].tb;
+  mdpp_image_discrete_tables first = t0;
+  for (int g = 0; g < n_groups; ++g) {
+    const mdpp_image_discrete_tables& t = groups[g].tb;
+    const std::string which = "set_image_discrete_groups: group " + std::to_string(g);
+    if (t.width != t0.width || t.height != t0.height || n_sub_of(t) != n_sub_of(t0))
+      return fail(ctx, MDPP_EINVAL, which + " differs from group 0 in width, height "
+                  "or n_sub_images");
+    if (t.width < 1 || t.height < 1 || t.n_states < 1 || t.n_radii < 1)
+      return fail(ctx, MDPP_EINVAL, which + ": bad sizes");
+    if (!t.mask_bits || !t.mask_index || !t.xvar || !t.yvar || !t.rot_coeff ||
+        (t.has_scale && t.n_radii > 1 && !t.r_thresholds))
+      return fail(ctx, MDPP_EINVAL, which + ": missing table pointer");
+    first.has_rotate |= t.has_rotate;  // (the kernel's zero-fill schedule)
+  }
+  release_discrete_groups(ctx);
+  rc = upload_groups(ctx, groups, n_groups, env_group, &ctx->img_d_groups,
+                     &ctx->img_d_env_group);
+  if (rc) { release_discrete_groups(ctx); return rc; }
+  ctx->img_d_first = first;
+  ctx->img_d_n_groups = n_groups;
+  ctx->img_d_total_envs = (int64_t)env_group.size();
   return MDPP_OK;
+}
+
+extern "C" int mdpp_render_discrete_groups(mdpp_ctx* ctx, const int64_t* states,
+                                           const int32_t* params_in,
+                                           int32_t* params_out, uint8_t* out,
+                                           int64_t n_images, int64_t n_envs,
+                                           int32_t image_stream,
+                                           const mdpp_step_opts* opts,
+                                           void* cuda_stream) {
+  if (!ctx) return MDPP_EINVAL;
+  if (!ctx->img_d_groups)
+    return fail(ctx, MDPP_EINVAL, "render_discrete_groups: no image groups set");
+  if (!states || !out || !opts || n_images < 1 || n_envs < 1)
+    return fail(ctx, MDPP_EINVAL, "render_discrete_groups: bad arguments");
+  if (n_envs != ctx->img_d_total_envs)
+    return fail(ctx, MDPP_EINVAL, "render_discrete_groups: n_envs = " +
+                std::to_string(n_envs) + " differs from the groups' total of " +
+                std::to_string(ctx->img_d_total_envs) + " envs");
+  if (n_images > 0x7fffffffLL)
+    return fail(ctx, MDPP_EINVAL, "render_discrete_groups: too many images per call");
+  MDPP_CUDA(ctx, cudaSetDevice(ctx->device));
+  RenderDParams p;
+  p.tb = ctx->img_d_first;
+  p.groups = ctx->img_d_groups;
+  p.env_group = ctx->img_d_env_group;
+  fill_render_params(p, states, params_in, params_out, out, n_images, n_envs,
+                     image_stream, opts);
+  return launch_render_discrete<true>(ctx, p, opts, cuda_stream);
+}
+
+extern "C" int mdpp_set_image_continuous_groups(mdpp_ctx* ctx,
+                                                const mdpp_image_continuous_group* groups,
+                                                int32_t n_groups) {
+  if (!ctx) return MDPP_EINVAL;
+  std::vector<uint16_t> env_group;
+  int rc = tile_groups(ctx, "set_image_continuous_groups", groups, n_groups, env_group);
+  if (rc) return rc;
+  const mdpp_image_continuous_config& c0 = groups[0].cfg;
+  for (int g = 0; g < n_groups; ++g) {
+    const mdpp_image_continuous_config& c = groups[g].cfg;
+    const std::string which = "set_image_continuous_groups: group " + std::to_string(g);
+    if (c.width != c0.width || c.height != c0.height || c.n_sub_images != c0.n_sub_images)
+      return fail(ctx, MDPP_EINVAL, which + " differs from group 0 in width, height "
+                  "or n_sub_images");
+    if (c.dim != c0.dim || c.is_f64 != c0.is_f64)
+      return fail(ctx, MDPP_EINVAL, which + " differs from group 0 in dim or is_f64");
+    if (c.width < 1 || c.height < 1 || c.n_sub_images < 1 || c.n_sub_images > 2 ||
+        c.stamp_rows > MDPP_MAX_STAMP_ROWS || c.n_rects > MDPP_MAX_TERM_BOXES)
+      return fail(ctx, MDPP_EINVAL, which + ": bad configuration");
+  }
+  release_continuous_groups(ctx);
+  rc = upload_groups(ctx, groups, n_groups, env_group, &ctx->img_c_groups,
+                     &ctx->img_c_env_group);
+  if (rc) { release_continuous_groups(ctx); return rc; }
+  ctx->img_c_first = c0;
+  ctx->img_c_n_groups = n_groups;
+  ctx->img_c_total_envs = (int64_t)env_group.size();
+  return MDPP_OK;
+}
+
+extern "C" int mdpp_render_continuous_groups(mdpp_ctx* ctx, const void* states,
+                                             uint8_t* out, int64_t n_images,
+                                             int64_t n_envs, void* cuda_stream) {
+  if (!ctx) return MDPP_EINVAL;
+  if (!ctx->img_c_groups)
+    return fail(ctx, MDPP_EINVAL, "render_continuous_groups: no image groups set");
+  if (!states || !out || n_images < 1 || n_envs < 1)
+    return fail(ctx, MDPP_EINVAL, "render_continuous_groups: bad arguments");
+  if (n_envs != ctx->img_c_total_envs)
+    return fail(ctx, MDPP_EINVAL, "render_continuous_groups: n_envs = " +
+                std::to_string(n_envs) + " differs from the groups' total of " +
+                std::to_string(ctx->img_c_total_envs) + " envs");
+  if (n_images * ctx->img_c_first.n_sub_images > 0x7fffffffLL)
+    return fail(ctx, MDPP_EINVAL, "render_continuous_groups: too many images per call");
+  MDPP_CUDA(ctx, cudaSetDevice(ctx->device));
+  RenderCParams p;
+  p.cfg = ctx->img_c_first;
+  p.groups = ctx->img_c_groups;
+  p.env_group = ctx->img_c_env_group;
+  p.n_envs = n_envs;
+  p.states = states;
+  p.out = out;
+  return launch_render_continuous<true>(ctx, p, n_images, cuda_stream);
 }

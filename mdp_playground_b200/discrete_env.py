@@ -305,9 +305,9 @@ class DiscreteEnv(VectorRLToyEnv):
         prm = torch.empty((M, 5), dtype=torch.int32, device=dev)
         ropts = self._opts(1)
         ropts.flags = _lib.MDPP_LAUNCH_OVERLAP_PREVIOUS
-        args = (C.byref(self._img_cfg), _ptr(state), None, _ptr(prm), _ptr(img),
-                M, self.num_envs, 3, C.byref(ropts))
-        return img, (self._lib.mdpp_render_discrete, ropts, args, prm)
+        args = self._render_tables() + (_ptr(state), None, _ptr(prm), _ptr(img),
+                                        M, self.num_envs, 3, C.byref(ropts))
+        return img, (self._render_fn(), ropts, args, prm)
 
     def rollout(self, n_steps, actions=None, replay=None, out=None,
                 want_final_obs=True):
@@ -337,7 +337,19 @@ class DiscreteEnv(VectorRLToyEnv):
     # ------------------------------------------------------------------
     # image observations
     # ------------------------------------------------------------------
+    @staticmethod
+    def _image_key(sp):
+        """What a discrete renderer table set depends on besides the state
+        count: the transforms and their parameters."""
+        tr = sp.image_transforms
+        flags = tuple(t in tr for t in ("scale", "shift", "rotate", "flip"))
+        return flags + (int(sp.image_sh_quant or 1), int(sp.image_ro_quant or 1),
+                        tuple(sp.image_scale_range) if flags[0] else None)
+
     def _init_images(self):
+        """Renderer tables: one set per distinct image configuration of the
+        config groups (a sweep whose cells do not vary the images builds one),
+        for the largest state count of the groups that share it."""
         from . import image_tables as it
         sp, dev = self.spec, self.device
         W, H = sp.image_width, sp.image_height
@@ -347,29 +359,48 @@ class DiscreteEnv(VectorRLToyEnv):
             t = torch.as_tensor(np.ascontiguousarray(a)).to(dtype).to(dev).contiguous()
             self._img_keep.append(t)
             return _ptr(t)
-        tb = it.build_discrete_image_tables(
-            max(self.tables.n_states, self.tables.n_states_irr), W, H,
-            sp.image_transforms,
-            sp.image_sh_quant, sp.image_ro_quant, sp.image_scale_range)
-        self.image_tables = tb
-        c = _lib.ImageDiscreteTables()
-        c.width, c.height, c.n_states = W, H, tb.n_states
-        c.r_min, c.n_radii = tb.r_min, tb.n_radii
-        c.n_xvar, c.n_yvar = tb.n_xvar, tb.n_yvar
-        c.has_scale, c.has_shift = int(tb.has_scale), int(tb.has_shift)
-        c.has_rotate, c.has_flip = int(tb.has_rotate), int(tb.has_flip)
-        c.sh_quant, c.ro_quant = tb.sh_quant, tb.ro_quant
-        c.mask_bits = up(tb.mask_bits.view(np.int64), torch.int64)
-        c.mask_index = up(tb.mask_index, torch.int32)
-        c.xvar, c.yvar = up(tb.xvar, torch.uint8), up(tb.yvar, torch.uint8)
-        c.rot_coeff = up(tb.rot_coeff, torch.int32)
-        c.r_thresholds = up(tb.r_thresholds if len(tb.r_thresholds)
-                            else np.zeros(1), torch.float64)
+        keys = [self._image_key(s_) for s_ in self._group_specs]
+        n_states = {}
+        for k, t_ in zip(keys, self.group_tables):
+            n_states[k] = max(n_states.get(k, 0), t_.n_states, t_.n_states_irr or 0)
         # irrelevant_features: one polygon image per sub-state, stacked
         # along x (image_multi_discrete.py:272-288)
         self._n_sub = 2 if self._irr else 1
-        c.n_sub_images = self._n_sub
-        self._img_cfg = c
+        self.image_table_sets = {}  # image key -> (host tables, struct)
+        for k, s_ in zip(keys, self._group_specs):
+            if k in self.image_table_sets:
+                continue
+            tb = it.build_discrete_image_tables(
+                n_states[k], W, H, s_.image_transforms,
+                s_.image_sh_quant, s_.image_ro_quant, s_.image_scale_range)
+            c = _lib.ImageDiscreteTables()
+            c.width, c.height, c.n_states = W, H, tb.n_states
+            c.r_min, c.n_radii = tb.r_min, tb.n_radii
+            c.n_xvar, c.n_yvar = tb.n_xvar, tb.n_yvar
+            c.has_scale, c.has_shift = int(tb.has_scale), int(tb.has_shift)
+            c.has_rotate, c.has_flip = int(tb.has_rotate), int(tb.has_flip)
+            c.sh_quant, c.ro_quant = tb.sh_quant, tb.ro_quant
+            c.mask_bits = up(tb.mask_bits.view(np.int64), torch.int64)
+            c.mask_index = up(tb.mask_index, torch.int32)
+            c.xvar, c.yvar = up(tb.xvar, torch.uint8), up(tb.yvar, torch.uint8)
+            c.rot_coeff = up(tb.rot_coeff, torch.int32)
+            c.r_thresholds = up(tb.r_thresholds if len(tb.r_thresholds)
+                                else np.zeros(1), torch.float64)
+            c.n_sub_images = self._n_sub
+            self.image_table_sets[k] = (tb, c)
+        self.image_tables, self._img_cfg = self.image_table_sets[keys[0]]
+        # (replay mode needs image_params when any group draws transforms)
+        self._img_random = any(tb.has_scale or tb.has_shift or tb.has_rotate
+                               or tb.has_flip
+                               for tb, _ in self.image_table_sets.values())
+        if self.n_groups > 1:
+            groups = (_lib.ImageDiscreteGroup * self.n_groups)()
+            for g, k, (begin, count, id_base) in zip(groups, keys,
+                                                     self._group_layout()):
+                g.tb = self.image_table_sets[k][1]
+                g.env_begin, g.env_count, g.global_id_base = begin, count, id_base
+            self._check(self._lib.mdpp_set_image_discrete_groups(
+                self._ctx, groups, self.n_groups))
         self.obs_shape = (W * self._n_sub, H, 1)
         if self.noise == "numpy":
             self._rng_I = self._numpy_lanes(self.seed_dict.get("image_representations"))
@@ -423,9 +454,7 @@ class DiscreteEnv(VectorRLToyEnv):
         if image_params is not None:
             image_params = torch.as_tensor(image_params, device=dev).to(
                 torch.int32).reshape(M, 5).contiguous()
-        elif self.noise == "replay" and not allow_philox and (
-                self.image_tables.has_scale or self.image_tables.has_shift
-                or self.image_tables.has_rotate or self.image_tables.has_flip):
+        elif self.noise == "replay" and not allow_philox and self._img_random:
             raise ValueError("replay mode: pass image_params [N, 5]")
         out = torch.empty(lead + self.obs_shape, dtype=torch.uint8, device=dev)
         self.last_image_params = torch.empty((M, 5), dtype=torch.int32,
@@ -433,11 +462,21 @@ class DiscreteEnv(VectorRLToyEnv):
         if self._overlap_render and st.data_ptr() == state.data_ptr():
             # (no cast / copy kernel sits between the step and this launch)
             opts.flags = _lib.MDPP_LAUNCH_OVERLAP_PREVIOUS
-        self._check(self._lib.mdpp_render_discrete(
-            self._ctx, C.byref(self._img_cfg), _ptr(st), _ptr(image_params),
+        self._check(self._render_fn()(
+            self._ctx, *self._render_tables(), _ptr(st), _ptr(image_params),
             _ptr(self.last_image_params), _ptr(out), M, N,
             6 if reset else 3, C.byref(opts), self._stream()))
         return out
+
+    def _render_fn(self):
+        """The renderer entry point: one table set, or each group's own."""
+        return self._lib.mdpp_render_discrete_groups if self.n_groups > 1 \
+            else self._lib.mdpp_render_discrete
+
+    def _render_tables(self):
+        """The entry point's table argument (none for the grouped one: the
+        context holds the groups' tables)."""
+        return () if self.n_groups > 1 else (C.byref(self._img_cfg),)
 
     # ------------------------------------------------------------------
     def get_augmented_state(self):

@@ -51,9 +51,9 @@ class GridEnv(VectorRLToyEnv):
             if any(len(s_.grid_shape) != nd for s_ in specs):
                 raise ValueError("config_groups of grid envs must agree on the "
                                  "number of grid dimensions (irrelevant_features)")
-            if sp.image_representations or self.noise == "numpy":
+            if self.noise == "numpy":
                 raise NotImplementedError(
-                    "config_groups of grid envs: no images, no noise='numpy'")
+                    "config_groups of grid envs: no noise='numpy'")
         self._set_configs([grid_cfg(s_) for s_ in specs], _lib.GridGroup,
                           self._lib.mdpp_set_grid_groups,
                           self._lib.mdpp_set_grid_config)
@@ -127,10 +127,14 @@ class GridEnv(VectorRLToyEnv):
 
     # ------------------------------------------------------------------
     def _init_images(self):
+        """One renderer configuration per config group (its own grid lines,
+        target and terminal cells)."""
+        self._set_image_groups([self._grid_image_cfg(s_) for s_ in self._group_specs])
+
+    def _grid_image_cfg(self, sp):
         # ImageContinuous with grid_shape (image_continuous.py:139-207):
         # white grid lines, black terminal cells, green target and blue
         # agent discs at the cell centres (+0.5), per sub-grid
-        sp = self.spec
         W, H = sp.image_width, sp.image_height
         nd, gs = self._nd, sp.grid_shape
         if W > 256 or H > 256:
@@ -140,7 +144,7 @@ class GridEnv(VectorRLToyEnv):
             raise NotImplementedError("at most 8 terminal cells in images")
         corners = [np.array(cell, dtype=np.float64).astype(np.int64) for cell in cells]
         # (image_continuous.py:248-277 over Box(0, shape))
-        c = self._box_image_cfg(nd, np.zeros(2, dtype=np.int64),
+        c = self._box_image_cfg(sp, nd, np.zeros(2, dtype=np.int64),
                                 np.array(gs[:2], dtype=np.int64),
                                 [(lo_, lo_ + 1.0) for lo_ in corners],
                                 np.array(sp.target_point, dtype=float) + 0.5, True)
@@ -154,7 +158,7 @@ class GridEnv(VectorRLToyEnv):
                 y = j * H // gs[off]             # divisor is the FIRST extent)
                 if 0 <= y < H:
                     c.hline[sub][y >> 6] |= 1 << (y & 63)
-        self._img_cfg = c
+        return c
 
     def _render_states(self, state):
         return (state.to(torch.float64) + 0.5).contiguous()  # cell centres

@@ -9,9 +9,12 @@ static `env_config["env_config"]` and hands each to a separate Ray trial
 configuration group of a single batched env, stepped by one kernel launch,
 and the per-cell episode statistics are written in the reference's CSV layout
 (config_processor.py:241-259, :340-373) so its analysis code can read them.
-Continuous and grid experiment files whose cells cannot share one launch
-(different state dimension / dtype) get one batched env per cell instead.  No
-agent is trained: the policy is uniform random (or supplied by the caller).
+Continuous and grid experiment files run the same way, image observations
+included: each cell renders with its own image settings (discrete transforms
+and their quantisation, continuous / grid targets, terminal regions and
+bounds).  Only cells that cannot share one launch (different state dimension
+/ dtype, image size) get one batched env per cell instead.  No agent is
+trained: the policy is uniform random (or supplied by the caller).
 """
 import copy
 import importlib.util
@@ -146,7 +149,8 @@ class Sweep:
         """Continuous cells that share dim / dtype / reward function, and grid
         cells that share the number of coordinates, run as config groups of
         one env: one launch per rollout for the whole grid
-        (e.g. experiments/sac_move_to_a_point_p_order_2.py:10-30)."""
+        (e.g. experiments/sac_move_to_a_point_p_order_2.py:10-30), and one
+        render launch per observation when the cells have images."""
         try:
             self.env = Env(
                 self.n_cells * self.envs_per_cell, device=device, autoreset=True,

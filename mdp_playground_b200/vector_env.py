@@ -174,6 +174,7 @@ class VectorRLToyEnv:
         self._history = None
         if self.noise == "numpy":
             self._rng_E = [None] * N  # seeded by the first reset
+        self._check_image_groups()
         self._init_kind()
         self._fast_step = (self.noise == "philox" and self._step_buffers > 0
                            and (self._renders_in_step
@@ -247,6 +248,34 @@ class VectorRLToyEnv:
             g.env_begin, g.env_count, g.global_id_base = begin, count, id_base
         self._check(set_groups(self._ctx, groups, len(cfgs)))
 
+    def _check_image_groups(self):
+        """Config groups share one observation tensor: they must agree on
+        whether observations are images and on the image size."""
+        sp = self.spec
+        for gi, s_ in enumerate(self._group_specs):
+            if s_.image_representations != sp.image_representations or (
+                    sp.image_representations
+                    and (s_.image_width, s_.image_height)
+                    != (sp.image_width, sp.image_height)):
+                raise ValueError(
+                    "config_groups must agree on image_representations, "
+                    f"image_width and image_height (group {gi} differs from "
+                    "group 0)")
+
+    def _set_image_groups(self, cfgs):
+        """Hand the image configs of a continuous or grid env (one per
+        group) to the library: a single one is passed to each render call,
+        config groups are set once for the grouped renderer."""
+        self._img_cfg = cfgs[0]
+        if len(cfgs) == 1:
+            return
+        groups = (_lib.ImageContinuousGroup * len(cfgs))()
+        for g, cfg, (begin, count, _) in zip(groups, cfgs, self._group_layout()):
+            g.cfg = cfg
+            g.env_begin, g.env_count = begin, count
+        self._check(self._lib.mdpp_set_image_continuous_groups(
+            self._ctx, groups, len(cfgs)))
+
     def _new_state(self, cls):
         """The kind's state struct, with the fields every kind has set."""
         st = cls()
@@ -255,15 +284,15 @@ class VectorRLToyEnv:
         st.stats, st.stats_slots = _ptr(self._stats), _lib.STATS_SLOTS
         return st
 
-    def _box_image_cfg(self, dim, lo, hi, rects, target, is_f64):
+    def _box_image_cfg(self, sp, dim, lo, hi, rects, target, is_f64):
         """ImageContinuousConfig of the renderer of the feature box [lo, hi]
-        (image_continuous.py): black `rects` given as (low, high) corners,
-        the green target disc at `target` and the agent discs of
-        circle_radius=5 (rl_toy_env.py:774).  Dimensions 0 and 1 are the
-        relevant ones (ImageContinuous' default; the env does not pass its
+        of parsed config `sp` (image_continuous.py): black `rects` given as
+        (low, high) corners, the green target disc at `target` and the agent
+        discs of circle_radius=5 (rl_toy_env.py:774).  Dimensions 0 and 1 are
+        the relevant ones (ImageContinuous' default; the env does not pass its
         own); with dim 4, 2 and 3 are drawn in a second sub-image."""
         from .image_tables import disc_stamp
-        W, H = self.spec.image_width, self.spec.image_height
+        W, H = sp.image_width, sp.image_height
 
         def to_pixel(vec):  # image_continuous.py:248-277
             frac = (np.asarray(vec) - lo) / (hi - lo)
@@ -417,9 +446,15 @@ class VectorRLToyEnv:
         st = self._render_states(state)
         out = torch.empty(tuple(st.shape[:-1]) + self.obs_shape,
                           dtype=torch.uint8, device=self.device)
-        self._check(self._lib.mdpp_render_continuous(
-            self._ctx, C.byref(self._img_cfg), _ptr(st), _ptr(out),
-            st.numel() // self._row[0], self._stream()))
+        n_images = st.numel() // self._row[0]
+        if self.n_groups > 1:  # each image with its config group's settings
+            self._check(self._lib.mdpp_render_continuous_groups(
+                self._ctx, _ptr(st), _ptr(out), n_images, self.num_envs,
+                self._stream()))
+        else:
+            self._check(self._lib.mdpp_render_continuous(
+                self._ctx, C.byref(self._img_cfg), _ptr(st), _ptr(out),
+                n_images, self._stream()))
         return out
 
     # ------------------------------------------------------------------

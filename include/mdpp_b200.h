@@ -235,6 +235,38 @@ int mdpp_discrete_rollout(mdpp_ctx* ctx, const mdpp_discrete_state* st,
                           const mdpp_step_opts* opts, void* cuda_stream);
 #endif
 
+/* Tabular Q-learning fused into the discrete rollout: T steps of epsilon-
+ * greedy Q-learning, one Q-table per env, in one launch.  At global step
+ * `step` env i (global Philox id g) in state s draws
+ * w = philox(g, step, STREAM_ACTION) -- the random policy's word --, explores
+ * iff (double)w.z < epsilon * 2^32 (then a = the random policy's action
+ * umulhi(w.x, A)), else a = argmax_a' q[i][s][a'] (ties: lowest index), steps
+ * like mdpp_discrete_rollout, and updates, with r the returned reward and nxt
+ * the state before any auto-reset,
+ *   target = terminated ? r : r + gamma * max_a' q[i][nxt][a']
+ *   q[i][s][a] += alpha * (target - q[i][s][a])
+ * in float64 with every operation rounded on its own (no FMA).  Truncation
+ * bootstraps.  The env state and statistics end as mdpp_discrete_rollout
+ * leaves them with the same actions.  `io->actions` must be NULL; the other
+ * outputs of `io` and `actions_taken` may be NULL (skipped).  Philox noise,
+ * no irrelevant features.                                                  */
+typedef struct mdpp_qlearn_params {
+  double alpha, gamma, epsilon;   /* each in [0, 1]                          */
+  double* q;                      /* [N][q_states][q_actions], env-major     */
+  int32_t q_states, q_actions;    /* >= every group's S / A                  */
+  double* ep_return;              /* [N] return of the running episode       */
+  double* ret_sum;                /* [N] sum of the returns of the episodes  */
+  int32_t* ret_count;             /* [N] ... that ended in an auto-reset     */
+  int32_t* actions_taken;         /* [T*N] or NULL                           */
+} mdpp_qlearn_params;
+
+#ifndef __CUDACC_RTC__ /* NVRTC sees the types only */
+int mdpp_discrete_qlearn(mdpp_ctx* ctx, const mdpp_discrete_state* st,
+                         const mdpp_discrete_io* io,
+                         const mdpp_qlearn_params* qp,
+                         const mdpp_step_opts* opts, void* cuda_stream);
+#endif
+
 /* K6: (masked) reset.  mask NULL = all envs.  The initial state comes from
  * `init_states` when given, else from the init cdf driven by `replay_reset_u`
  * (MDPP_NOISE_REPLAY) or Philox.  `obs` may be NULL.  With

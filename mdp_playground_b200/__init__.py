@@ -6,6 +6,7 @@ reset/step semantics and runs every step on hand-written sm_100a CUDA kernels
 """
 from .vector_env import VectorRLToyEnv  # noqa: F401
 from .wrapper_tail import VectorGymEnvTail  # noqa: F401
+from .qlearning import TabularQLearner  # noqa: F401
 
-__all__ = ["VectorRLToyEnv", "VectorGymEnvTail"]
+__all__ = ["VectorRLToyEnv", "VectorGymEnvTail", "TabularQLearner"]
 __version__ = "0.1.0"

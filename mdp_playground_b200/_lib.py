@@ -36,6 +36,7 @@ EXPORTED_SYMBOLS = (
     "mdpp_set_grid_groups",
     "mdpp_set_image_discrete_groups", "mdpp_render_discrete_groups",
     "mdpp_set_image_continuous_groups", "mdpp_render_continuous_groups",
+    "mdpp_discrete_qlearn",
 )
 MDPP_MAX_DIM, MDPP_MAX_ORDER, MDPP_MAX_TERM_BOXES = 16, 4, 8
 
@@ -97,6 +98,15 @@ class StepOpts(C.Structure):
         ("normal_mode", C.c_int32), ("flags", C.c_int32),
         ("seed", C.c_uint64), ("step_index", C.c_uint64),
         ("env_id_offset", C.c_int64), ("step_index_dev", C.c_void_p),
+    ]
+
+
+class QlearnParams(C.Structure):
+    _fields_ = [
+        ("alpha", C.c_double), ("gamma", C.c_double), ("epsilon", C.c_double),
+        ("q", C.c_void_p), ("q_states", C.c_int32), ("q_actions", C.c_int32),
+        ("ep_return", C.c_void_p), ("ret_sum", C.c_void_p),
+        ("ret_count", C.c_void_p), ("actions_taken", C.c_void_p),
     ]
 
 
@@ -278,6 +288,9 @@ def load():
     lib.mdpp_set_discrete_groups.argtypes = [P, C.POINTER(DiscreteGroup), C.c_int32]
     lib.mdpp_discrete_rollout.argtypes = [
         P, C.POINTER(DiscreteState), C.POINTER(DiscreteIO), C.POINTER(StepOpts), P]
+    lib.mdpp_discrete_qlearn.argtypes = [
+        P, C.POINTER(DiscreteState), C.POINTER(DiscreteIO), C.POINTER(QlearnParams),
+        C.POINTER(StepOpts), P]
     lib.mdpp_discrete_reset.argtypes = [
         P, C.POINTER(DiscreteState), P, P, P, P, C.POINTER(StepOpts), P]
     lib.mdpp_set_jit.argtypes = [P, C.c_int]

@@ -118,11 +118,11 @@ static int check_state(mdpp_ctx* ctx, const mdpp_discrete_state* st) {
   return MDPP_OK;
 }
 
-extern "C" int mdpp_discrete_rollout(mdpp_ctx* ctx,
-                                     const mdpp_discrete_state* st,
-                                     const mdpp_discrete_io* io,
-                                     const mdpp_step_opts* opts,
-                                     void* cuda_stream) {
+// Checks and kernel parameters shared by mdpp_discrete_rollout and
+// mdpp_discrete_qlearn (qlearn.cu).
+int mdpp::prepare_rollout(mdpp_ctx* ctx, const mdpp_discrete_state* st,
+                          const mdpp_discrete_io* io, const mdpp_step_opts* opts,
+                          RolloutParams& p) {
   int rc = check_state(ctx, st);
   if (rc) return rc;
   if (!io || !opts || opts->n_steps < 1)
@@ -147,7 +147,6 @@ extern "C" int mdpp_discrete_rollout(mdpp_ctx* ctx,
   MDPP_CUDA(ctx, cudaSetDevice(ctx->device));
   rc = ensure_cta_map(ctx);
   if (rc) return rc;
-  RolloutParams p;
   p.group0 = ctx->d_groups_host[0];
   p.groups = ctx->d_groups;
   p.blob = ctx->d_blob;
@@ -167,6 +166,17 @@ extern "C" int mdpp_discrete_rollout(mdpp_ctx* ctx,
   p.n_groups = (int32_t)ctx->d_groups_host.size();
   p.zig = ctx->d_zig;
   p.tab_smem_bytes = 0;
+  return MDPP_OK;
+}
+
+extern "C" int mdpp_discrete_rollout(mdpp_ctx* ctx,
+                                     const mdpp_discrete_state* st,
+                                     const mdpp_discrete_io* io,
+                                     const mdpp_step_opts* opts,
+                                     void* cuda_stream) {
+  RolloutParams p;
+  int rc = prepare_rollout(ctx, st, io, opts, p);
+  if (rc) return rc;
   cudaStream_t s = (cudaStream_t)cuda_stream;
   if (opts->noise_mode < MDPP_NOISE_OFF || opts->noise_mode > MDPP_NOISE_PHILOX)
     return fail(ctx, MDPP_EINVAL, "unknown noise_mode");

@@ -462,6 +462,29 @@ struct Cfg {
   static constexpr int CDF_LOG2 = CDF_LOG2_;
 };
 
+// ---- agents riding along the chain ------------------------------------------
+// rollout_body runs a policy-free rollout with NoAgent: every hook is empty and
+// inlines to nothing.  qlearn.cu plugs a learner in through the same hooks:
+// draw()   sees the STREAM_ACTION words of the random policy (phase A),
+// act()    picks the action of a step from the random one and the env state,
+// update() sees the step's outcome (StepOut) and the state after any reset,
+// begin() / end() load and store per-env agent state around the launch.
+struct StepOut {
+  double r;      // the returned reward
+  int32_t nxt;   // state before any auto-reset (final_obs)
+  bool done, trunc;
+};
+
+struct NoAgent {
+  static constexpr bool kStepOut = false;  // chain_step hands out no StepOut
+  __device__ __forceinline__ void begin(const GroupView&, int64_t, int32_t) {}
+  __device__ __forceinline__ void draw(int, const U4&) {}
+  __device__ __forceinline__ int32_t act(int, int32_t a_rand, int32_t) { return a_rand; }
+  __device__ __forceinline__ void update(const RolloutParams&, const GroupView&,
+                                         const StepOut&, int32_t, int64_t, int64_t) {}
+  __device__ __forceinline__ void end(int64_t) {}
+};
+
 // ---- phase A: loads and state-independent random draws -------------------
 // Everything a chunk of U steps needs that does not depend on the env state:
 // the actions, the transition uniforms, the (sigma-scaled) reward normals and
@@ -494,9 +517,10 @@ __device__ __forceinline__ void load_action(const RolloutParams& p, int64_t off,
 
 // `zs` (STAGED): this thread's column of staged ziggurat normals, sigma
 // applied, zs[j * kBlock] = step t0 + j (zig_fill); else drawn here.
-template <typename C, int U, bool PRELOADED = false, bool STAGED = false>
+template <typename C, int U, bool PRELOADED = false, bool STAGED = false,
+          typename AG = NoAgent>
 __device__ __forceinline__ void phase_a(const RolloutParams& p, const GroupView& v,
-                                        int64_t env, uint32_t gid,
+                                        AG& ag, int64_t env, uint32_t gid,
                                         uint64_t step_base, int t0,
                                         int n_valid, int32_t* act, double* u_tr,
                                         int32_t* k_tr, double* n_rw, int32_t* s0,
@@ -524,6 +548,7 @@ __device__ __forceinline__ void phase_a(const RolloutParams& p, const GroupView&
                            STREAM_ACTION, p.k0, p.k1);
       act[j] = (int32_t)__umulhi(w.x, (uint32_t)v.A);
       q.act[j] = irr ? (int32_t)__umulhi(w.y, (uint32_t)v.A1) : 0;
+      ag.draw(j, w);
     }
     u_tr[j] = 0.0; k_tr[j] = 0; n_rw[j] = 0.0; u_rs[j] = 0.0; s0[j] = 0;
     q.u_tr[j] = 0.0; q.k_tr[j] = 0; q.s0[j] = 0; u_rs_i[j] = 0.0;
@@ -707,7 +732,8 @@ __device__ __forceinline__ void chain_step(const RolloutParams& p, const GroupVi
                                            int32_t act, double u_tr, int32_t k_tr,
                                            double n_rw, int32_t s0,
                                            int32_t act_i, double u_tr_i,
-                                           int32_t k_tr_i, int32_t s0_i) {
+                                           int32_t k_tr_i, int32_t s0_i,
+                                           StepOut* so = nullptr) {
   constexpr int NOISE = C::NOISE;
   constexpr bool RING_SMEM = C::RING_SMEM;
   constexpr bool FAST = C::FAST;
@@ -790,6 +816,7 @@ __device__ __forceinline__ void chain_step(const RolloutParams& p, const GroupVi
   if (!kTermRewardIsZero)
     if (done) r = __dadd_rn(r, v.term_reward_scaled);
   const bool trunc = horizon > 0 && e.tl >= horizon;
+  if (so) { so->r = r; so->nxt = nxt; so->done = done; so->trunc = trunc; }
 #ifndef MDPP_EXP_NO_STATS
   e.n_terminated += done;
 #endif
@@ -813,9 +840,10 @@ __device__ __forceinline__ void chain_step(const RolloutParams& p, const GroupVi
   if (FAST || p.io.truncated) st_stream(p.io.truncated + off, (uint8_t)trunc);
 }
 
-template <typename C, int U, bool PARTIAL>
+template <typename C, int U, bool PARTIAL, typename AG>
 __device__ __forceinline__ void phase_b(const RolloutParams& p, const GroupView& v,
-                                        EnvRegs& e, double* ring_smem, int ring_stride,
+                                        AG& ag, EnvRegs& e, double* ring_smem,
+                                        int ring_stride,
                                         int64_t env, int t0, int n_valid,
                                         const int32_t* act, const double* u_tr,
                                         const int32_t* k_tr, const double* n_rw,
@@ -825,17 +853,21 @@ __device__ __forceinline__ void phase_b(const RolloutParams& p, const GroupView&
 #pragma unroll
   for (int j = 0; j < U; ++j) {
     if (PARTIAL && j >= n_valid) break;
-    chain_step<C>(p, v, e, ring_smem, ring_stride, env, off0 + (int64_t)j * N,
-                  act[j], u_tr[j], k_tr[j], n_rw[j], s0[j],
-                  q.act[j], q.u_tr[j], q.k_tr[j], q.s0[j]);
+    const int64_t off = off0 + (int64_t)j * N;
+    StepOut so;
+    chain_step<C>(p, v, e, ring_smem, ring_stride, env, off,
+                  ag.act(j, act[j], e.s), u_tr[j], k_tr[j], n_rw[j], s0[j],
+                  q.act[j], q.u_tr[j], q.k_tr[j], q.s0[j],
+                  AG::kStepOut ? &so : nullptr);
+    ag.update(p, v, so, e.s, env, off);
   }
   e.n_steps += PARTIAL ? n_valid : U;
 }
 
 // A full chunk whose actions were prefetched into act[] (and act_i[]).
-template <typename C, int U, bool STAGED = false>
+template <typename C, int U, bool STAGED, typename AG>
 __device__ __forceinline__ void run_chunk_preloaded(
-    const RolloutParams& p, const GroupView& v, EnvRegs& e, double* ring_smem,
+    const RolloutParams& p, const GroupView& v, AG& ag, EnvRegs& e, double* ring_smem,
     int64_t env, uint32_t gid, uint64_t step_base, int t0, int32_t* act,
     const int32_t* act_i, const double* zs = nullptr) {
   int32_t s0[U], k_tr[U];
@@ -843,15 +875,15 @@ __device__ __forceinline__ void run_chunk_preloaded(
   IrrDraws<U> q;
 #pragma unroll
   for (int j = 0; j < U; ++j) q.act[j] = act_i[j];
-  phase_a<C, U, true, STAGED>(p, v, env, gid, step_base, t0, U, act, u_tr, k_tr,
-                              n_rw, s0, q, zs);
-  phase_b<C, U, false>(p, v, e, ring_smem, kBlock, env, t0, U, act, u_tr, k_tr,
+  phase_a<C, U, true, STAGED>(p, v, ag, env, gid, step_base, t0, U, act, u_tr,
+                              k_tr, n_rw, s0, q, zs);
+  phase_b<C, U, false>(p, v, ag, e, ring_smem, kBlock, env, t0, U, act, u_tr, k_tr,
                        n_rw, s0, q);
 }
 
-template <typename C, int U, bool STAGED = false>
+template <typename C, int U, bool STAGED, typename AG>
 __device__ __forceinline__ void run_chunk(const RolloutParams& p,
-                                          const GroupView& v, EnvRegs& e,
+                                          const GroupView& v, AG& ag, EnvRegs& e,
                                           double* ring_smem, int64_t env,
                                           uint32_t gid, uint64_t step_base, int t0,
                                           const double* zs = nullptr) {
@@ -859,9 +891,9 @@ __device__ __forceinline__ void run_chunk(const RolloutParams& p,
   int32_t k_tr[U];
   double u_tr[U], n_rw[U];
   IrrDraws<U> q;
-  phase_a<C, U, false, STAGED>(p, v, env, gid, step_base, t0, U, act, u_tr, k_tr,
-                               n_rw, s0, q, zs);
-  phase_b<C, U, false>(p, v, e, ring_smem, kBlock, env, t0, U, act, u_tr, k_tr,
+  phase_a<C, U, false, STAGED>(p, v, ag, env, gid, step_base, t0, U, act, u_tr,
+                               k_tr, n_rw, s0, q, zs);
+  phase_b<C, U, false>(p, v, ag, e, ring_smem, kBlock, env, t0, U, act, u_tr, k_tr,
                        n_rw, s0, q);
 }
 
@@ -961,8 +993,8 @@ __device__ __forceinline__ double warp_sum(double x) {
   return x;
 }
 
-template <typename C>
-__device__ __forceinline__ void rollout_body(const RolloutParams& p) {
+template <typename C, typename AG>
+__device__ __forceinline__ void rollout_body(const RolloutParams& p, AG& ag) {
   // A kernel launched behind this one with programmatic stream serialisation
   // (the renderer, MDPP_LAUNCH_OVERLAP_PREVIOUS) may start its independent
   // prologue now; it still waits for this grid to finish before it reads the
@@ -1054,6 +1086,7 @@ __device__ __forceinline__ void rollout_body(const RolloutParams& p) {
   e.n_noisy = e.n_episodes = e.n_terminated = e.n_steps = 0;
 
   if (active) {
+    ag.begin(v, env, e.s);
     // the value written j steps ago sits in ring slot (pos - j) mod d
     if (C::RING_REGS > 0) {
 #pragma unroll
@@ -1069,14 +1102,14 @@ __device__ __forceinline__ void rollout_body(const RolloutParams& p) {
     // chunks of kChunk steps start on a multiple-of-4 global step (the Philox
     // draws come in groups of 4 steps); peel single steps until aligned
     while (t0 < p.T && ((step_base + (uint64_t)t0) & 3)) {
-      run_chunk<C, 1>(p, v, e, ring_smem, env, gid, step_base, t0);
+      run_chunk<C, 1, false>(p, v, ag, e, ring_smem, env, gid, step_base, t0);
       ++t0;
     }
 #ifdef MDPP_STAGGER
     // de-synchronise the warps of an SM: odd warps run a half chunk first
     if (kChunk > 4 && ((blockIdx.x * (kBlock / 32) + (threadIdx.x >> 5)) & 1) &&
         t0 + 4 <= p.T) {
-      run_chunk<C, 4>(p, v, e, ring_smem, env, gid, step_base, t0);
+      run_chunk<C, 4, false>(p, v, ag, e, ring_smem, env, gid, step_base, t0);
       t0 += 4;
     }
 #endif
@@ -1111,11 +1144,11 @@ __device__ __forceinline__ void rollout_body(const RolloutParams& p) {
           load_action<C>(p, (int64_t)(tn + j) * N + env, act_next[j], act_next_i[j]);
         }
         if (stage_path)
-          run_chunk_preloaded<C, kChunk, ZIG && SMEM>(p, v, e, ring_smem, env, gid,
+          run_chunk_preloaded<C, kChunk, ZIG && SMEM>(p, v, ag, e, ring_smem, env, gid,
                                                       step_base, t0, act, act_i,
                                                       zst.zs + (t0 - zs_t0) * kBlock);
         else
-          run_chunk_preloaded<C, kChunk, false>(p, v, e, ring_smem, env, gid,
+          run_chunk_preloaded<C, kChunk, false>(p, v, ag, e, ring_smem, env, gid,
                                                 step_base, t0, act, act_i);
       }
     } else {
@@ -1126,24 +1159,25 @@ __device__ __forceinline__ void rollout_body(const RolloutParams& p) {
                    (p.T - t0) / kChunk * kChunk);
         }
         if (stage_path)
-          run_chunk<C, kChunk, ZIG && SMEM>(p, v, e, ring_smem, env, gid, step_base, t0,
+          run_chunk<C, kChunk, ZIG && SMEM>(p, v, ag, e, ring_smem, env, gid, step_base, t0,
                                             zst.zs + (t0 - zs_t0) * kBlock);
         else
-          run_chunk<C, kChunk, false>(p, v, e, ring_smem, env, gid, step_base, t0);
+          run_chunk<C, kChunk, false>(p, v, ag, e, ring_smem, env, gid, step_base, t0);
       }
     }
     // remainder: a half chunk first (t0 is still quad-aligned here; single
     // steps pay a whole Philox quad each), then single steps
     if (kChunk > 4)
       for (; t0 + 4 <= p.T; t0 += 4)
-        run_chunk<C, 4>(p, v, e, ring_smem, env, gid, step_base, t0);
+        run_chunk<C, 4, false>(p, v, ag, e, ring_smem, env, gid, step_base, t0);
     for (; t0 < p.T; ++t0)
-      run_chunk<C, 1>(p, v, e, ring_smem, env, gid, step_base, t0);
+      run_chunk<C, 1, false>(p, v, ag, e, ring_smem, env, gid, step_base, t0);
     p.st.cur_state[env] = e.s;
     if (irr) p.st.cur_state_irr[env] = e.s_irr;
     p.st.seq_key[env] = e.key;
     p.st.t_episode[env] = e.tl;
     p.st.episode[env] = e.ep + e.n_episodes;
+    ag.end(env);
     if (C::RING_REGS > 0) {
       const int pos_end = (int)((step_base + (uint64_t)p.T) % (uint64_t)C::RING_REGS);
 #pragma unroll
@@ -1177,6 +1211,12 @@ __device__ __forceinline__ void rollout_body(const RolloutParams& p) {
       if ((threadIdx.x & 31) == 0 && s != 0.0) atomicAdd(row + k, s);
     }
   }
+}
+
+template <typename C>
+__device__ __forceinline__ void rollout_body(const RolloutParams& p) {
+  NoAgent ag;
+  rollout_body<C>(p, ag);
 }
 
 template <typename C>

@@ -8,10 +8,12 @@ namespace mdpp {
 // Ring of delayed rewards lives in shared memory when it is small enough.
 constexpr int kRingSmemMaxDelay = 16;
 
-template <typename C>
-inline int launch_one(mdpp_ctx* ctx, RolloutParams& p, int smem_tab,
-                      cudaStream_t stream) {
-  auto kern = discrete_rollout_kernel<C>;
+// Launch `kern` with argument `kp` for configuration C.  `p` is the rollout
+// part of `kp` (kp itself for the rollout kernels): its shared-memory sizes
+// are set here, before the launch copies `kp`.
+template <typename C, typename KP>
+inline int launch_kernel(mdpp_ctx* ctx, RolloutParams& p, int smem_tab,
+                         cudaStream_t stream, void (*kern)(KP), const KP& kp) {
   p.ring_smem_bytes = C::RING_SMEM ? ctx->max_delay * kBlock * 8 : 0;
   p.tab_smem_bytes = C::SMEM ? smem_tab : 0;
   const bool zig = C::NORMAL == MDPP_NORMAL_ZIGGURAT && C::NOISE == MDPP_NOISE_PHILOX;
@@ -34,9 +36,25 @@ inline int launch_one(mdpp_ctx* ctx, RolloutParams& p, int smem_tab,
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = p.T < kChunk ? 1 : 0;
-  MDPP_CUDA(ctx, cudaLaunchKernelEx(&cfg, kern, p));
+  MDPP_CUDA(ctx, cudaLaunchKernelEx(&cfg, kern, kp));
   MDPP_CUDA(ctx, cudaGetLastError());
   return MDPP_OK;
+}
+
+template <typename C>
+inline int launch_one(mdpp_ctx* ctx, RolloutParams& p, int smem_tab,
+                      cudaStream_t stream) {
+  return launch_kernel<C>(ctx, p, smem_tab, stream, discrete_rollout_kernel<C>, p);
+}
+
+// Whether the group tables (and the delay ring) of a launch go to shared
+// memory: `ring_ok` the ring, the return value the tables.
+inline bool tables_in_smem(const mdpp_ctx* ctx, const RolloutParams& p, bool* ring_ok) {
+  *ring_ok = ctx->max_delay <= kRingSmemMaxDelay;
+  const int ring_bytes = *ring_ok ? ctx->max_delay * kBlock * 8 : 0;
+  return p.T >= smem_min_steps() &&
+         ctx->max_group_blob + ring_bytes + kZigBytes + zig_stage_bytes(kBlock) <=
+             ctx->max_smem_optin - 1024;
 }
 
 // Kernel variants.  The FAST ones (standard signature, tables + ring in
@@ -47,11 +65,8 @@ inline int launch_one(mdpp_ctx* ctx, RolloutParams& p, int smem_tab,
 template <int NOISE, int NORMAL>
 inline int launch_rollout(mdpp_ctx* ctx, RolloutParams& p, cudaStream_t stream) {
   const int smem_tab = ctx->max_group_blob;
-  const bool ring_ok = ctx->max_delay <= kRingSmemMaxDelay;
-  const int ring_bytes = ring_ok ? ctx->max_delay * kBlock * 8 : 0;
-  const bool smem_ok =
-      p.T >= smem_min_steps() && smem_tab + ring_bytes + kZigBytes + zig_stage_bytes(kBlock) <=
-                           ctx->max_smem_optin - 1024;
+  bool ring_ok;
+  const bool smem_ok = tables_in_smem(ctx, p, &ring_ok);
   const bool fast_io = p.io.actions && p.io.obs && p.io.reward &&
                        p.io.terminated && p.io.truncated && !p.io.final_obs &&
                        !p.st.history && !p.irr;  // (FAST kernels: no sub-MDP)

@@ -86,6 +86,10 @@ void jit_release(mdpp_ctx* ctx);
 void render_release(mdpp_ctx* ctx);  // render.cu: the per-group image descriptors
 int smem_min_steps();  // MDPP_SMEM_MIN_T (default 1): shorter launches skip the smem staging
 int fail(mdpp_ctx* ctx, int code, const std::string& msg);
+// discrete.cu: validate a discrete launch and fill its parameters
+int prepare_rollout(mdpp_ctx* ctx, const mdpp_discrete_state* st,
+                    const mdpp_discrete_io* io, const mdpp_step_opts* opts,
+                    RolloutParams& p);
 int cuda_fail(mdpp_ctx* ctx, cudaError_t e, const char* what);
 }  // namespace mdpp
 

@@ -13,8 +13,11 @@ Continuous and grid experiment files run the same way, image observations
 included: each cell renders with its own image settings (discrete transforms
 and their quantisation, continuous / grid targets, terminal regions and
 bounds).  Only cells that cannot share one launch (different state dimension
-/ dtype, image size) get one batched env per cell instead.  No agent is
-trained: the policy is uniform random (or supplied by the caller).
+/ dtype, image size) get one batched env per cell instead.  `run` steps a
+uniform random policy (or one supplied by the caller); `train` trains a
+tabular Q-learning agent per env of a discrete grid inside the step kernel
+(qlearning.py) and writes a learning curve per cell, one CSV row per
+(training iteration, cell) like the reference's stats files.
 """
 import copy
 import importlib.util
@@ -144,6 +147,8 @@ class Sweep:
             self.env = self.envs[0]
         self.timesteps = 0
         self._returned = np.zeros(self.n_cells)
+        self.agent = None
+        self.train_results = []  # one dict per training iteration
 
     def _try_grouped(self, Env, device, horizon, shard, env_kwargs):
         """Continuous cells that share dim / dtype / reward function, and grid
@@ -194,6 +199,43 @@ class Sweep:
             done += T
         self.timesteps += steps_per_env
         return self.results()
+
+    def train(self, iterations, steps_per_iteration, alpha=0.1, gamma=0.99,
+              epsilon=0.1, chunk=256):
+        """Tabular Q-learning (one agent per env; envs_per_cell seeds per
+        cell), `iterations` times `steps_per_iteration` steps per env.  Each
+        iteration appends to `train_results`, per cell: the cumulative
+        timesteps_total, episode_reward_mean (mean return of the episodes
+        completed in the iteration; NaN if none) and episode_len_mean (from
+        the episode counters' change over the iteration).  Discrete grids
+        only.  Calling train again continues with the same Q-tables."""
+        if self.kind != "discrete":
+            raise NotImplementedError(
+                "Sweep.train: tabular Q-learning runs on discrete grids only")
+        from .qlearning import TabularQLearner
+        if self.agent is None:
+            self.agent = TabularQLearner(self.env, alpha=alpha, gamma=gamma,
+                                         epsilon=epsilon)
+        env = self.env
+        self.agent.episode_returns(clear=True)
+        for _ in range(int(iterations)):
+            before = env.episode_stats()
+            done = 0
+            while done < steps_per_iteration:
+                T = min(chunk, steps_per_iteration - done)
+                self.agent.learn(T, alpha=alpha, gamma=gamma, epsilon=epsilon)
+                done += T
+            self.timesteps += steps_per_iteration
+            after = env.episode_stats()
+            ret = self.agent.episode_returns(clear=True)
+            d_ep = after["episodes"] - before["episodes"]
+            d_tr = after["transitions"] - before["transitions"]
+            self.train_results.append({
+                "training_iteration": len(self.train_results) + 1,
+                "timesteps_total": after["transitions"],
+                "episode_reward_mean": ret["episode_reward_mean"],
+                "episode_len_mean": d_tr / np.maximum(d_ep, 1)})
+        return self.train_results
 
     def _random_actions(self, env, T, t0):
         """Uniform random policy for the per-cell envs (continuous: uniform
@@ -252,21 +294,32 @@ class Sweep:
                 "episode_len_mean": st["transitions"] / ep,
                 "noisy_transitions": st["noisy_transitions"]}
 
-    def write_csv(self, path, algorithm="RandomPolicy"):
-        """One row per grid cell in the reference's stats-file layout."""
-        res = self.results()
+    def write_csv(self, path, algorithm=None):
+        """The reference's stats-file layout: one row per grid cell, or, once
+        `train` has run, one row per (training iteration, cell).  algorithm
+        defaults to "RandomPolicy", or "TabularQLearning" after `train`."""
+        if self.train_results:
+            iters = self.train_results
+            algorithm = algorithm or "TabularQLearning"
+        else:
+            res = self.results()
+            iters = [{"training_iteration": 1, "timesteps_total": res["transitions"],
+                      "episode_reward_mean": res["episode_reward_mean"],
+                      "episode_len_mean": res["episode_len_mean"]}]
+            algorithm = algorithm or "RandomPolicy"
         with open(path, "w") as f:
             f.write("# training_iteration, algorithm, "
                     + "".join(k + ", " for k in self.env_keys)
                     + "timesteps_total, episode_reward_mean, episode_len_mean\n")
-            for i, cfg in enumerate(self.cell_configs):
-                row = ["1", algorithm]
-                for k in self.env_keys:
-                    v = cfg[k]
-                    row.append("%.2e" % v if isinstance(v, float)
-                               else str(v).replace(" ", ""))
-                row += [str(int(res["transitions"][i])),
-                        "%.2e" % res["episode_reward_mean"][i],
-                        "%.2e" % res["episode_len_mean"][i]]
-                f.write(" ".join(row) + "\n")
+            for it in iters:
+                for i, cfg in enumerate(self.cell_configs):
+                    row = [str(it["training_iteration"]), algorithm]
+                    for k in self.env_keys:
+                        v = cfg[k]
+                        row.append("%.2e" % v if isinstance(v, float)
+                                   else str(v).replace(" ", ""))
+                    row += [str(int(it["timesteps_total"][i])),
+                            "%.2e" % it["episode_reward_mean"][i],
+                            "%.2e" % it["episode_len_mean"][i]]
+                    f.write(" ".join(row) + "\n")
         return path

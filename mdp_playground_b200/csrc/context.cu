@@ -4,6 +4,7 @@
 #include <cstdlib>
 #include <cstring>
 
+#include "discrete_kernels.cuh"  // kBlock: the rollout's CTA size
 #include "internal.h"
 #include "ziggurat.cuh"
 #include "ziggurat_tables.h"
@@ -80,28 +81,15 @@ extern "C" int mdpp_create(int device, mdpp_ctx** out_ctx) {
   return MDPP_OK;
 }
 
-static void free_discrete(mdpp_ctx* ctx) {
-  if (ctx->d_groups) cudaFree(ctx->d_groups);
-  if (ctx->d_blob) cudaFree(ctx->d_blob);
-  if (ctx->d_cta_map) cudaFree(ctx->d_cta_map);
-  ctx->d_groups = nullptr;
-  ctx->d_blob = nullptr;
-  ctx->d_cta_map = nullptr;
-  ctx->cta_map_block = 0;
-  ctx->d_groups_host.clear();
-}
-
 extern "C" void mdpp_destroy(mdpp_ctx* ctx) {
   if (!ctx) return;
   cudaSetDevice(ctx->device);
   jit_release(ctx);
-  free_discrete(ctx);
+  if (ctx->d_blob) cudaFree(ctx->d_blob);
   if (ctx->d_zig) cudaFree(ctx->d_zig);
-  if (ctx->c_groups) cudaFree(ctx->c_groups);
-  if (ctx->c_cta_map) cudaFree(ctx->c_cta_map);
-  if (ctx->g_groups) cudaFree(ctx->g_groups);
-  if (ctx->g_cta_map) cudaFree(ctx->g_cta_map);
-  render_release(ctx);
+  for (GroupSet* set : {&ctx->d_set, &ctx->c_set, &ctx->g_set, &ctx->img_d_set,
+                        &ctx->img_c_set})
+    release_groups(*set);
   delete ctx;
 }
 
@@ -125,17 +113,12 @@ extern "C" int mdpp_set_discrete_groups(mdpp_ctx* ctx,
                                         const mdpp_discrete_group* groups,
                                         int32_t n_groups) {
   if (!ctx) return MDPP_EINVAL;
-  if (!groups || n_groups <= 0)
-    return fail(ctx, MDPP_EINVAL, "need at least one discrete group");
-  MDPP_CUDA(ctx, cudaSetDevice(ctx->device));
-  free_discrete(ctx);
-
+  int rc = validate_groups(ctx, __func__, groups, n_groups, /*env_map=*/false);
+  if (rc) return rc;
   std::vector<DiscreteGroupDev> dev(n_groups);
   std::vector<uint8_t> blob;
-  int64_t next_env = 0;
-  ctx->max_group_blob = 0;
-  ctx->max_delay = 0;
-  ctx->d_irr = groups[0].n_states_irr > 0;
+  int max_group_blob = 0, max_delay = 0;
+  const int irr = groups[0].n_states_irr > 0;
   for (int g = 0; g < n_groups; ++g) {
     const mdpp_discrete_group& in = groups[g];
     DiscreteGroupDev& d = dev[g];
@@ -148,17 +131,13 @@ extern "C" int mdpp_set_discrete_groups(mdpp_ctx* ctx,
       return fail(ctx, MDPP_EINVAL, "discrete group: missing table");
     if (in.has_transition_noise && !in.noise_cdf)
       return fail(ctx, MDPP_EINVAL, "transition noise needs noise_cdf");
-    if ((in.n_states_irr > 0) != (ctx->d_irr != 0))
+    if ((in.n_states_irr > 0) != (irr != 0))
       return fail(ctx, MDPP_EINVAL,
                   "all groups must agree on having an irrelevant sub-MDP");
     if (in.n_states_irr > 0 &&
         (in.n_states_irr > 65535 || in.n_actions_irr < 1 || !in.transition_irr ||
          !in.init_cdf_irr || (in.has_transition_noise && !in.noise_cdf_irr)))
       return fail(ctx, MDPP_EINVAL, "discrete group: bad irrelevant sub-MDP");
-    if (in.env_begin != next_env || in.env_count < 0)
-      return fail(ctx, MDPP_EINVAL,
-                  "groups must tile the env range contiguously, in order");
-    next_env += in.env_count;
     const int b = bits_for(S);
     if ((int64_t)b * L > 63)
       return fail(ctx, MDPP_EINVAL,
@@ -180,7 +159,7 @@ extern "C" int mdpp_set_discrete_groups(mdpp_ctx* ctx,
     d.env_begin = in.env_begin;
     d.gid_base = in.global_id_base;
     d.env_count = in.env_count;
-    if (in.delay > ctx->max_delay) ctx->max_delay = in.delay;
+    if (in.delay > max_delay) max_delay = in.delay;
 
     // ---- pack the blob -------------------------------------------------
     std::vector<uint8_t> gb;
@@ -382,18 +361,26 @@ extern "C" int mdpp_set_discrete_groups(mdpp_ctx* ctx,
     gb.resize(d.blob_bytes, 0);
     d.blob_offset = (int64_t)blob.size();
     blob.insert(blob.end(), gb.begin(), gb.end());
-    if (d.blob_bytes > ctx->max_group_blob) ctx->max_group_blob = d.blob_bytes;
+    if (d.blob_bytes > max_group_blob) max_group_blob = d.blob_bytes;
   }
-  ctx->d_total_envs = next_env;
+  MDPP_CUDA(ctx, cudaSetDevice(ctx->device));
+  uint8_t* d_blob = nullptr;
+  cudaError_t e = cudaMalloc(&d_blob, blob.size());
+  if (e == cudaSuccess)
+    e = cudaMemcpy(d_blob, blob.data(), blob.size(), cudaMemcpyHostToDevice);
+  rc = e == cudaSuccess ? install_groups(ctx, ctx->d_set, dev.data(), n_groups, kBlock)
+                        : cuda_fail(ctx, e, "discrete table upload");
+  if (rc) {
+    if (d_blob) cudaFree(d_blob);
+    return rc;
+  }
+  if (ctx->d_blob) cudaFree(ctx->d_blob);
+  ctx->d_blob = d_blob;
   ctx->d_blob_bytes = blob.size();
-  MDPP_CUDA(ctx, cudaMalloc(&ctx->d_blob, blob.size()));
-  MDPP_CUDA(ctx, cudaMemcpy(ctx->d_blob, blob.data(), blob.size(),
-                            cudaMemcpyHostToDevice));
-  MDPP_CUDA(ctx, cudaMalloc(&ctx->d_groups, sizeof(DiscreteGroupDev) * n_groups));
-  MDPP_CUDA(ctx, cudaMemcpy(ctx->d_groups, dev.data(),
-                            sizeof(DiscreteGroupDev) * n_groups,
-                            cudaMemcpyHostToDevice));
   ctx->d_groups_host = dev;
+  ctx->max_group_blob = max_group_blob;
+  ctx->max_delay = max_delay;
+  ctx->d_irr = irr;
   ctx->d_groups_version += 1;
   return MDPP_OK;
 }

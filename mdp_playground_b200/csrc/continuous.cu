@@ -11,16 +11,6 @@
 
 using namespace mdpp;
 
-static void free_groups(mdpp_ctx* ctx) {
-  if (ctx->c_groups) cudaFree(ctx->c_groups);
-  if (ctx->c_cta_map) cudaFree(ctx->c_cta_map);
-  ctx->c_groups = nullptr;
-  ctx->c_cta_map = nullptr;
-  ctx->c_n_groups = 0;
-  ctx->c_n_ctas = 0;
-  ctx->c_total_envs = 0;
-}
-
 static int check_config(mdpp_ctx* ctx, const mdpp_continuous_config* cfg) {
   if (!cfg) return fail(ctx, MDPP_EINVAL, "cfg is NULL");
   if (cfg->dim < 1 || cfg->dim > MDPP_MAX_DIM)
@@ -53,7 +43,7 @@ extern "C" int mdpp_set_continuous_config(mdpp_ctx* ctx,
   if (!ctx) return MDPP_EINVAL;
   int rc = check_config(ctx, cfg);
   if (rc) return rc;
-  free_groups(ctx);
+  release_groups(ctx->c_set);
   ctx->c_cfg = *cfg;
   ctx->have_continuous = true;
   return MDPP_OK;
@@ -63,15 +53,15 @@ extern "C" int mdpp_set_continuous_groups(mdpp_ctx* ctx,
                                           const mdpp_continuous_group* groups,
                                           int32_t n_groups) {
   if (!ctx) return MDPP_EINVAL;
-  if (!groups || n_groups < 1)
-    return fail(ctx, MDPP_EINVAL, "need at least one continuous group");
+  int rc = validate_groups(ctx, __func__, groups, n_groups, /*env_map=*/false);
+  if (rc) return rc;
   std::vector<ContinuousGroupDev> dev(n_groups);
-  std::vector<CtaMapEntry> map;
-  int64_t next_env = 0;
   const mdpp_continuous_config& c0 = groups[0].cfg;
+  // the launch-wide view: flags any group has (replay arrays, ring depth)
+  mdpp_continuous_config view = c0;
   for (int g = 0; g < n_groups; ++g) {
     const mdpp_continuous_config& c = groups[g].cfg;
-    int rc = check_config(ctx, &c);
+    rc = check_config(ctx, &c);
     if (rc) return rc;
     // the groups share everything that shapes the state arrays and the I/O rows
     // (the order may differ: derivative planes are addressed independently of it)
@@ -83,39 +73,19 @@ extern "C" int mdpp_set_continuous_groups(mdpp_ctx* ctx,
       return fail(ctx, MDPP_EINVAL,
                   "continuous groups must agree on dim, relevant_indices, dtype, "
                   "reward function (and its sequence_length) and image mode");
-    if (groups[g].env_begin != next_env || groups[g].env_count < 0)
-      return fail(ctx, MDPP_EINVAL,
-                  "groups must tile the env range contiguously, in order");
-    next_env += groups[g].env_count;
     std::memset(&dev[g], 0, sizeof dev[g]);
     dev[g].cfg = c;
     for (int j = 0; j < MDPP_MAX_ORDER; ++j) dev[g].tu_pow[j] = std::pow(c.time_unit, j + 1);
     dev[g].env_begin = groups[g].env_begin;
     dev[g].env_count = groups[g].env_count;
     dev[g].gid_base = groups[g].global_id_base;
-    const int64_t chunks = (groups[g].env_count + kCBlock - 1) / kCBlock;
-    for (int64_t k = 0; k < chunks; ++k) map.push_back(CtaMapEntry{g, (int32_t)k});
+    view.has_transition_noise |= c.has_transition_noise;
+    view.has_reward_noise |= c.has_reward_noise;
+    if (c.delay > view.delay) view.delay = c.delay;
   }
-  if (map.empty()) return fail(ctx, MDPP_EINVAL, "no environments");
-  MDPP_CUDA(ctx, cudaSetDevice(ctx->device));
-  free_groups(ctx);
-  MDPP_CUDA(ctx, cudaMalloc(&ctx->c_groups, dev.size() * sizeof(ContinuousGroupDev)));
-  MDPP_CUDA(ctx, cudaMemcpy(ctx->c_groups, dev.data(), dev.size() * sizeof(ContinuousGroupDev),
-                            cudaMemcpyHostToDevice));
-  MDPP_CUDA(ctx, cudaMalloc(&ctx->c_cta_map, map.size() * sizeof(CtaMapEntry)));
-  MDPP_CUDA(ctx, cudaMemcpy(ctx->c_cta_map, map.data(), map.size() * sizeof(CtaMapEntry),
-                            cudaMemcpyHostToDevice));
-  ctx->c_n_groups = n_groups;
-  ctx->c_n_ctas = (int64_t)map.size();
-  ctx->c_total_envs = next_env;
-  // the launch-wide view: flags any group has (replay arrays, ring depth)
-  ctx->c_cfg = c0;
-  for (int g = 1; g < n_groups; ++g) {
-    const mdpp_continuous_config& c = groups[g].cfg;
-    ctx->c_cfg.has_transition_noise |= c.has_transition_noise;
-    ctx->c_cfg.has_reward_noise |= c.has_reward_noise;
-    if (c.delay > ctx->c_cfg.delay) ctx->c_cfg.delay = c.delay;
-  }
+  rc = install_groups(ctx, ctx->c_set, dev.data(), n_groups, kCBlock);
+  if (rc) return rc;
+  ctx->c_cfg = view;
   ctx->have_continuous = true;
   return MDPP_OK;
 }
@@ -150,19 +120,19 @@ static int fill_params(mdpp_ctx* ctx, const mdpp_continuous_state* st,
   p->step_index = opts->step_index;
   p->step_index_dev = opts->step_index_dev;
   p->env_id_offset = opts->env_id_offset;
-  if (ctx->c_n_groups > 0) {
-    if (st->n_envs != ctx->c_total_envs)
-      return fail(ctx, MDPP_EINVAL, "state.n_envs != sum of group env counts");
-    p->groups = reinterpret_cast<const ContinuousGroupDev*>(ctx->c_groups);
-    p->cta_map = reinterpret_cast<const CtaMapEntry*>(ctx->c_cta_map);
-    p->n_groups = ctx->c_n_groups;
+  if (ctx->c_set.n_groups > 0) {
+    int rc = bind_groups(ctx, ctx->c_set, "continuous launch", st->n_envs);
+    if (rc) return rc;
+    p->groups = static_cast<const ContinuousGroupDev*>(ctx->c_set.groups);
+    p->cta_map = ctx->c_set.cta_map;
+    p->n_groups = ctx->c_set.n_groups;
   }
   return MDPP_OK;
 }
 
 template <typename R>
 static int launch_groups(mdpp_ctx* ctx, const ContinuousParams& p, cudaStream_t s) {
-  const unsigned grid = (unsigned)ctx->c_n_ctas;
+  const unsigned grid = (unsigned)ctx->c_set.n_ctas;
   switch (p.noise_mode) {
     case MDPP_NOISE_OFF:
       continuous_rollout_kernel<R, MDPP_NOISE_OFF, true><<<grid, kCBlock, 0, s>>>(p);
@@ -242,7 +212,7 @@ extern "C" int mdpp_continuous_reset(mdpp_ctx* ctx,
   p.init_states = init_states;
   p.reset_obs = obs;
   MDPP_CUDA(ctx, cudaSetDevice(ctx->device));
-  const unsigned grid = p.groups ? (unsigned)ctx->c_n_ctas
+  const unsigned grid = p.groups ? (unsigned)ctx->c_set.n_ctas
                                  : (unsigned)((p.st.n_envs + kCBlock - 1) / kCBlock);
   cudaStream_t s = (cudaStream_t)cuda_stream;
   if (p.groups && ctx->c_cfg.is_f64)

@@ -1,7 +1,7 @@
-// C entry points of the discrete step path (include/mdpp_b200.h), the reset
-// kernel (K6) and the CTA -> (group, chunk) map.  The rollout kernels live in
-// discrete_kernels.cuh and are instantiated per noise mode in
-// discrete_{off,replay,philox_f64,philox_fast}.cu so they compile in parallel.
+// C entry points of the discrete step path (include/mdpp_b200.h) and the reset
+// kernel (K6).  The rollout kernels live in discrete_kernels.cuh and are
+// instantiated per noise mode in discrete_{off,replay,philox_f64,philox_fast}.cu
+// so they compile in parallel.
 #include "discrete_kernels.cuh"
 #include "internal.h"
 
@@ -77,38 +77,19 @@ discrete_reset_kernel(const __grid_constant__ ResetParams p) {
   }
 }
 
-static int ensure_cta_map(mdpp_ctx* ctx) {
-  if (ctx->d_cta_map && ctx->cta_map_block == kBlock) return MDPP_OK;
-  std::vector<CtaMapEntry> map;
-  for (size_t g = 0; g < ctx->d_groups_host.size(); ++g) {
-    int64_t chunks = (ctx->d_groups_host[g].env_count + kBlock - 1) / kBlock;
-    for (int64_t c = 0; c < chunks; ++c)
-      map.push_back(CtaMapEntry{(int32_t)g, (int32_t)c});
-  }
-  if (ctx->d_cta_map) cudaFree(ctx->d_cta_map);
-  ctx->d_cta_map = nullptr;
-  if (map.empty()) return fail(ctx, MDPP_EINVAL, "no environments");
-  MDPP_CUDA(ctx, cudaMalloc(&ctx->d_cta_map, map.size() * sizeof(CtaMapEntry)));
-  MDPP_CUDA(ctx, cudaMemcpy(ctx->d_cta_map, map.data(),
-                            map.size() * sizeof(CtaMapEntry),
-                            cudaMemcpyHostToDevice));
-  ctx->cta_map_block = kBlock;
-  ctx->n_ctas = (int64_t)map.size();
-  return MDPP_OK;
-}
-
 }  // namespace mdpp
 
 using namespace mdpp;
 
-static int check_state(mdpp_ctx* ctx, const mdpp_discrete_state* st) {
+static int check_state(mdpp_ctx* ctx, const mdpp_discrete_state* st,
+                       const char* entry) {
   if (!ctx) return MDPP_EINVAL;
   if (ctx->d_groups_host.empty())
     return fail(ctx, MDPP_EINVAL, "mdpp_set_discrete_groups was not called");
   if (!st || !st->cur_state || !st->seq_key || !st->t_episode || !st->episode)
     return fail(ctx, MDPP_EINVAL, "discrete state has NULL arrays");
-  if (st->n_envs != ctx->d_total_envs)
-    return fail(ctx, MDPP_EINVAL, "state.n_envs != sum of group env counts");
+  int rc = bind_groups(ctx, ctx->d_set, entry, st->n_envs);
+  if (rc) return rc;
   if (ctx->max_delay > 0 && (!st->ring || st->ring_depth < ctx->max_delay))
     return fail(ctx, MDPP_EINVAL, "delay ring missing or too shallow");
   if (st->history && st->history_depth < 1)
@@ -123,7 +104,7 @@ static int check_state(mdpp_ctx* ctx, const mdpp_discrete_state* st) {
 int mdpp::prepare_rollout(mdpp_ctx* ctx, const mdpp_discrete_state* st,
                           const mdpp_discrete_io* io, const mdpp_step_opts* opts,
                           RolloutParams& p) {
-  int rc = check_state(ctx, st);
+  int rc = check_state(ctx, st, "discrete rollout");
   if (rc) return rc;
   if (!io || !opts || opts->n_steps < 1)
     return fail(ctx, MDPP_EINVAL, "bad io/opts");
@@ -145,12 +126,10 @@ int mdpp::prepare_rollout(mdpp_ctx* ctx, const mdpp_discrete_state* st,
       return fail(ctx, MDPP_EINVAL, "replay mode: missing replay array");
   }
   MDPP_CUDA(ctx, cudaSetDevice(ctx->device));
-  rc = ensure_cta_map(ctx);
-  if (rc) return rc;
   p.group0 = ctx->d_groups_host[0];
-  p.groups = ctx->d_groups;
+  p.groups = static_cast<const DiscreteGroupDev*>(ctx->d_set.groups);
   p.blob = ctx->d_blob;
-  p.cta_map = ctx->d_cta_map;
+  p.cta_map = ctx->d_set.cta_map;
   p.st = *st;
   p.io = *io;
   p.T = opts->n_steps;
@@ -163,7 +142,7 @@ int mdpp::prepare_rollout(mdpp_ctx* ctx, const mdpp_discrete_state* st,
   p.step_index_dev = opts->step_index_dev;
   p.env_id_offset = opts->env_id_offset;
   p.irr = ctx->d_irr;
-  p.n_groups = (int32_t)ctx->d_groups_host.size();
+  p.n_groups = ctx->d_set.n_groups;
   p.zig = ctx->d_zig;
   p.tab_smem_bytes = 0;
   return MDPP_OK;
@@ -202,18 +181,16 @@ extern "C" int mdpp_discrete_reset(mdpp_ctx* ctx, const mdpp_discrete_state* st,
                                    const double* replay_reset_u, int64_t* obs,
                                    const mdpp_step_opts* opts,
                                    void* cuda_stream) {
-  int rc = check_state(ctx, st);
+  int rc = check_state(ctx, st, "discrete reset");
   if (rc) return rc;
   if (!opts) return fail(ctx, MDPP_EINVAL, "opts is NULL");
   if (!init_states && opts->noise_mode == MDPP_NOISE_REPLAY && !replay_reset_u)
     return fail(ctx, MDPP_EINVAL, "replay reset needs replay_reset_u");
   MDPP_CUDA(ctx, cudaSetDevice(ctx->device));
-  rc = ensure_cta_map(ctx);
-  if (rc) return rc;
   ResetParams p;
-  p.groups = ctx->d_groups;
+  p.groups = static_cast<const DiscreteGroupDev*>(ctx->d_set.groups);
   p.blob = ctx->d_blob;
-  p.cta_map = ctx->d_cta_map;
+  p.cta_map = ctx->d_set.cta_map;
   p.st = *st;
   p.mask = mask;
   p.init_states = init_states;
@@ -225,8 +202,8 @@ extern "C" int mdpp_discrete_reset(mdpp_ctx* ctx, const mdpp_discrete_state* st,
   p.step_index = opts->step_index;
   p.env_id_offset = opts->env_id_offset;
   p.irr = ctx->d_irr;
-  p.n_groups = (int32_t)ctx->d_groups_host.size();
-  discrete_reset_kernel<<<(unsigned)ctx->n_ctas, kBlock, 0,
+  p.n_groups = ctx->d_set.n_groups;
+  discrete_reset_kernel<<<(unsigned)ctx->d_set.n_ctas, kBlock, 0,
                           (cudaStream_t)cuda_stream>>>(p);
   MDPP_CUDA(ctx, cudaGetLastError());
   return MDPP_OK;

@@ -27,7 +27,7 @@ inline int launch_kernel(mdpp_ctx* ctx, RolloutParams& p, int smem_tab,
   // (rollout_body waits with griddepcontrol.wait before it touches anything
   // mutable).  Long rollouts gain nothing and measured 2-3 % slower with it.
   cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)ctx->n_ctas);
+  cfg.gridDim = dim3((unsigned)ctx->d_set.n_ctas);
   cfg.blockDim = dim3(kBlock);
   cfg.dynamicSmemBytes = smem;
   cfg.stream = stream;

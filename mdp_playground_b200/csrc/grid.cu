@@ -455,16 +455,6 @@ grid_reset_kernel(const __grid_constant__ GridParams p) {
 
 using namespace mdpp;
 
-static void free_grid_groups(mdpp_ctx* ctx) {
-  if (ctx->g_groups) cudaFree(ctx->g_groups);
-  if (ctx->g_cta_map) cudaFree(ctx->g_cta_map);
-  ctx->g_groups = nullptr;
-  ctx->g_cta_map = nullptr;
-  ctx->g_n_groups = 0;
-  ctx->g_n_ctas = 0;
-  ctx->g_total_envs = 0;
-}
-
 static int check_grid_config(mdpp_ctx* ctx, const mdpp_grid_config* cfg) {
   if (!cfg) return fail(ctx, MDPP_EINVAL, "cfg is NULL");
   if (cfg->n_dims != 2 && cfg->n_dims != 4)
@@ -484,7 +474,7 @@ extern "C" int mdpp_set_grid_config(mdpp_ctx* ctx, const mdpp_grid_config* cfg) 
   if (!ctx) return MDPP_EINVAL;
   int rc = check_grid_config(ctx, cfg);
   if (rc) return rc;
-  free_grid_groups(ctx);
+  release_groups(ctx->g_set);
   ctx->g_cfg = *cfg;
   ctx->have_grid = true;
   return MDPP_OK;
@@ -493,47 +483,28 @@ extern "C" int mdpp_set_grid_config(mdpp_ctx* ctx, const mdpp_grid_config* cfg) 
 extern "C" int mdpp_set_grid_groups(mdpp_ctx* ctx, const mdpp_grid_group* groups,
                                     int32_t n_groups) {
   if (!ctx) return MDPP_EINVAL;
-  if (!groups || n_groups < 1)
-    return fail(ctx, MDPP_EINVAL, "need at least one grid group");
+  int rc = validate_groups(ctx, __func__, groups, n_groups, /*env_map=*/false);
+  if (rc) return rc;
   std::vector<GridGroupDev> dev(n_groups);
-  std::vector<CtaMapEntry> map;
-  int64_t next_env = 0;
+  // the launch-wide view: flags any group has (which replay arrays are needed)
+  mdpp_grid_config view = groups[0].cfg;
   for (int g = 0; g < n_groups; ++g) {
     const mdpp_grid_config& c = groups[g].cfg;
-    int rc = check_grid_config(ctx, &c);
+    rc = check_grid_config(ctx, &c);
     if (rc) return rc;
     if (c.n_dims != groups[0].cfg.n_dims)  // the row layout of state and I/O
       return fail(ctx, MDPP_EINVAL, "grid groups must agree on n_dims");
-    if (groups[g].env_begin != next_env || groups[g].env_count < 0)
-      return fail(ctx, MDPP_EINVAL,
-                  "groups must tile the env range contiguously, in order");
-    next_env += groups[g].env_count;
     std::memset(&dev[g], 0, sizeof dev[g]);
     dev[g].cfg = c;
     dev[g].env_begin = groups[g].env_begin;
     dev[g].env_count = groups[g].env_count;
     dev[g].gid_base = groups[g].global_id_base;
-    const int64_t chunks = (groups[g].env_count + kGBlock - 1) / kGBlock;
-    for (int64_t k = 0; k < chunks; ++k) map.push_back(CtaMapEntry{g, (int32_t)k});
+    view.has_transition_noise |= c.has_transition_noise;
+    view.has_reward_noise |= c.has_reward_noise;
   }
-  if (map.empty()) return fail(ctx, MDPP_EINVAL, "no environments");
-  MDPP_CUDA(ctx, cudaSetDevice(ctx->device));
-  free_grid_groups(ctx);
-  MDPP_CUDA(ctx, cudaMalloc(&ctx->g_groups, dev.size() * sizeof(GridGroupDev)));
-  MDPP_CUDA(ctx, cudaMemcpy(ctx->g_groups, dev.data(), dev.size() * sizeof(GridGroupDev),
-                            cudaMemcpyHostToDevice));
-  MDPP_CUDA(ctx, cudaMalloc(&ctx->g_cta_map, map.size() * sizeof(CtaMapEntry)));
-  MDPP_CUDA(ctx, cudaMemcpy(ctx->g_cta_map, map.data(), map.size() * sizeof(CtaMapEntry),
-                            cudaMemcpyHostToDevice));
-  ctx->g_n_groups = n_groups;
-  ctx->g_n_ctas = (int64_t)map.size();
-  ctx->g_total_envs = next_env;
-  // the launch-wide view: flags any group has (which replay arrays are needed)
-  ctx->g_cfg = groups[0].cfg;
-  for (int g = 1; g < n_groups; ++g) {
-    ctx->g_cfg.has_transition_noise |= groups[g].cfg.has_transition_noise;
-    ctx->g_cfg.has_reward_noise |= groups[g].cfg.has_reward_noise;
-  }
+  rc = install_groups(ctx, ctx->g_set, dev.data(), n_groups, kGBlock);
+  if (rc) return rc;
+  ctx->g_cfg = view;
   ctx->have_grid = true;
   return MDPP_OK;
 }
@@ -562,19 +533,19 @@ static int fill_grid(mdpp_ctx* ctx, const mdpp_grid_state* st,
   p->env_id_offset = opts->env_id_offset;
   philox_round_keys(p->k0, p->k1, p->rk);
   p->zig = ctx->d_zig;
-  if (ctx->g_n_groups > 0) {
-    if (st->n_envs != ctx->g_total_envs)
-      return fail(ctx, MDPP_EINVAL, "state arrays do not match the grid groups");
-    p->groups = reinterpret_cast<const GridGroupDev*>(ctx->g_groups);
-    p->cta_map = reinterpret_cast<const CtaMapEntry*>(ctx->g_cta_map);
-    p->n_groups = ctx->g_n_groups;
+  if (ctx->g_set.n_groups > 0) {
+    int rc = bind_groups(ctx, ctx->g_set, "grid launch", st->n_envs);
+    if (rc) return rc;
+    p->groups = static_cast<const GridGroupDev*>(ctx->g_set.groups);
+    p->cta_map = ctx->g_set.cta_map;
+    p->n_groups = ctx->g_set.n_groups;
   }
   return MDPP_OK;
 }
 
 template <int ND, bool FAST, bool GROUPS>
 static int launch_grid(mdpp_ctx* ctx, const GridParams& p, cudaStream_t s) {
-  const unsigned grid = GROUPS ? (unsigned)ctx->g_n_ctas
+  const unsigned grid = GROUPS ? (unsigned)ctx->g_set.n_ctas
                                : (unsigned)((p.st.n_envs + kGBlock - 1) / kGBlock);
   switch (p.noise_mode) {
     case MDPP_NOISE_OFF:
@@ -650,7 +621,7 @@ extern "C" int mdpp_grid_reset(mdpp_ctx* ctx, const mdpp_grid_state* st,
   p.init_states = init_states;
   p.reset_obs = obs;
   MDPP_CUDA(ctx, cudaSetDevice(ctx->device));
-  const unsigned grid = p.groups ? (unsigned)ctx->g_n_ctas
+  const unsigned grid = p.groups ? (unsigned)ctx->g_set.n_ctas
                                  : (unsigned)((p.st.n_envs + kGBlock - 1) / kGBlock);
   cudaStream_t s = (cudaStream_t)cuda_stream;
   if (p.groups && ctx->g_cfg.n_dims == 4) grid_reset_kernel<4, true><<<grid, kGBlock, 0, s>>>(p);

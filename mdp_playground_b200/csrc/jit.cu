@@ -463,7 +463,7 @@ int jit_try_rollout(mdpp_ctx* ctx, RolloutParams& p, int noise_mode,
   if (!fn) return 0;
   p.ring_smem_bytes = ring_bytes;
   p.tab_smem_bytes = smem ? ctx->max_group_blob : 0;
-  return launch(ctx, fn, (unsigned)ctx->n_ctas, kBlock,
+  return launch(ctx, fn, (unsigned)ctx->d_set.n_ctas, kBlock,
                 ring_bytes + (smem ? ctx->max_group_blob + zig_bytes : 0), stream, &p,
                 /*pdl=*/p.T < kChunk);
 }

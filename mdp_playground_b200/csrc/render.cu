@@ -12,10 +12,8 @@
 // streaming stores first; the shape is then assembled as column bitmaps of the
 // FINAL image in shared memory and only its non-empty 4-byte words are stored
 // again.  K5: one CTA per (sub-)image, 16 output bytes per thread and store.
-#include <algorithm>
 #include <cstdlib>
 #include <string>
-#include <vector>
 
 #include "internal.h"
 #include "philox.cuh"
@@ -572,74 +570,11 @@ int launch_render_continuous(mdpp_ctx* ctx, const RenderCParams& p,
   return MDPP_OK;
 }
 
-// The checks every group set shares: the groups tile [0, N) in order, at most
-// 65 535 of them (the env -> group map is uint16).  Builds that map.
-template <typename G>
-int tile_groups(mdpp_ctx* ctx, const char* what, const G* groups, int32_t n,
-                std::vector<uint16_t>& env_group) {
-  if (!groups || n < 1)
-    return fail(ctx, MDPP_EINVAL, std::string(what) + ": need at least one group");
-  if (n > 65535)
-    return fail(ctx, MDPP_EINVAL, std::string(what) + ": at most 65535 groups");
-  int64_t next = 0;
-  for (int g = 0; g < n; ++g) {
-    if (groups[g].env_begin != next || groups[g].env_count < 0)
-      return fail(ctx, MDPP_EINVAL, std::string(what) + ": group " + std::to_string(g) +
-                  " does not continue the tiling of the env range (groups must tile "
-                  "[0, N) contiguously, in order)");
-    next += groups[g].env_count;
-  }
-  if (next < 1) return fail(ctx, MDPP_EINVAL, std::string(what) + ": no environments");
-  env_group.resize((size_t)next);
-  for (int g = 0; g < n; ++g)
-    std::fill(env_group.begin() + groups[g].env_begin,
-              env_group.begin() + groups[g].env_begin + groups[g].env_count, (uint16_t)g);
-  return MDPP_OK;
-}
-
-// Context-owned copies of the descriptors and of the env -> group map.
-template <typename G>
-int upload_groups(mdpp_ctx* ctx, const G* groups, int32_t n,
-                  const std::vector<uint16_t>& env_group, G** d_groups,
-                  uint16_t** d_env_group) {
-  MDPP_CUDA(ctx, cudaSetDevice(ctx->device));
-  MDPP_CUDA(ctx, cudaMalloc(d_groups, (size_t)n * sizeof(G)));
-  MDPP_CUDA(ctx, cudaMemcpy(*d_groups, groups, (size_t)n * sizeof(G),
-                            cudaMemcpyHostToDevice));
-  MDPP_CUDA(ctx, cudaMalloc(d_env_group, env_group.size() * sizeof(uint16_t)));
-  MDPP_CUDA(ctx, cudaMemcpy(*d_env_group, env_group.data(),
-                            env_group.size() * sizeof(uint16_t), cudaMemcpyHostToDevice));
-  return MDPP_OK;
-}
-
-void release_discrete_groups(mdpp_ctx* ctx) {
-  if (ctx->img_d_groups) cudaFree(ctx->img_d_groups);
-  if (ctx->img_d_env_group) cudaFree(ctx->img_d_env_group);
-  ctx->img_d_groups = nullptr;
-  ctx->img_d_env_group = nullptr;
-  ctx->img_d_n_groups = 0;
-  ctx->img_d_total_envs = 0;
-}
-
-void release_continuous_groups(mdpp_ctx* ctx) {
-  if (ctx->img_c_groups) cudaFree(ctx->img_c_groups);
-  if (ctx->img_c_env_group) cudaFree(ctx->img_c_env_group);
-  ctx->img_c_groups = nullptr;
-  ctx->img_c_env_group = nullptr;
-  ctx->img_c_n_groups = 0;
-  ctx->img_c_total_envs = 0;
-}
-
 inline int n_sub_of(const mdpp_image_discrete_tables& tb) {
   return tb.n_sub_images < 1 ? 1 : tb.n_sub_images;
 }
 
 }  // namespace
-
-void mdpp::render_release(mdpp_ctx* ctx) {
-  release_discrete_groups(ctx);
-  release_continuous_groups(ctx);
-}
 
 extern "C" int mdpp_render_discrete(mdpp_ctx* ctx,
                                     const mdpp_image_discrete_tables* tb,
@@ -697,8 +632,7 @@ extern "C" int mdpp_set_image_discrete_groups(mdpp_ctx* ctx,
                                               const mdpp_image_discrete_group* groups,
                                               int32_t n_groups) {
   if (!ctx) return MDPP_EINVAL;
-  std::vector<uint16_t> env_group;
-  int rc = tile_groups(ctx, "set_image_discrete_groups", groups, n_groups, env_group);
+  int rc = validate_groups(ctx, __func__, groups, n_groups, /*env_map=*/true);
   if (rc) return rc;
   const mdpp_image_discrete_tables& t0 = groups[0].tb;
   mdpp_image_discrete_tables first = t0;
@@ -715,13 +649,9 @@ extern "C" int mdpp_set_image_discrete_groups(mdpp_ctx* ctx,
       return fail(ctx, MDPP_EINVAL, which + ": missing table pointer");
     first.has_rotate |= t.has_rotate;  // (the kernel's zero-fill schedule)
   }
-  release_discrete_groups(ctx);
-  rc = upload_groups(ctx, groups, n_groups, env_group, &ctx->img_d_groups,
-                     &ctx->img_d_env_group);
-  if (rc) { release_discrete_groups(ctx); return rc; }
+  rc = install_groups(ctx, ctx->img_d_set, groups, n_groups, /*block=*/0);
+  if (rc) return rc;
   ctx->img_d_first = first;
-  ctx->img_d_n_groups = n_groups;
-  ctx->img_d_total_envs = (int64_t)env_group.size();
   return MDPP_OK;
 }
 
@@ -733,21 +663,19 @@ extern "C" int mdpp_render_discrete_groups(mdpp_ctx* ctx, const int64_t* states,
                                            const mdpp_step_opts* opts,
                                            void* cuda_stream) {
   if (!ctx) return MDPP_EINVAL;
-  if (!ctx->img_d_groups)
+  if (!ctx->img_d_set.groups)
     return fail(ctx, MDPP_EINVAL, "render_discrete_groups: no image groups set");
   if (!states || !out || !opts || n_images < 1 || n_envs < 1)
     return fail(ctx, MDPP_EINVAL, "render_discrete_groups: bad arguments");
-  if (n_envs != ctx->img_d_total_envs)
-    return fail(ctx, MDPP_EINVAL, "render_discrete_groups: n_envs = " +
-                std::to_string(n_envs) + " differs from the groups' total of " +
-                std::to_string(ctx->img_d_total_envs) + " envs");
+  int rc = bind_groups(ctx, ctx->img_d_set, "render_discrete_groups", n_envs);
+  if (rc) return rc;
   if (n_images > 0x7fffffffLL)
     return fail(ctx, MDPP_EINVAL, "render_discrete_groups: too many images per call");
   MDPP_CUDA(ctx, cudaSetDevice(ctx->device));
   RenderDParams p;
   p.tb = ctx->img_d_first;
-  p.groups = ctx->img_d_groups;
-  p.env_group = ctx->img_d_env_group;
+  p.groups = static_cast<const mdpp_image_discrete_group*>(ctx->img_d_set.groups);
+  p.env_group = ctx->img_d_set.env_group;
   fill_render_params(p, states, params_in, params_out, out, n_images, n_envs,
                      image_stream, opts);
   return launch_render_discrete<true>(ctx, p, opts, cuda_stream);
@@ -757,8 +685,7 @@ extern "C" int mdpp_set_image_continuous_groups(mdpp_ctx* ctx,
                                                 const mdpp_image_continuous_group* groups,
                                                 int32_t n_groups) {
   if (!ctx) return MDPP_EINVAL;
-  std::vector<uint16_t> env_group;
-  int rc = tile_groups(ctx, "set_image_continuous_groups", groups, n_groups, env_group);
+  int rc = validate_groups(ctx, __func__, groups, n_groups, /*env_map=*/true);
   if (rc) return rc;
   const mdpp_image_continuous_config& c0 = groups[0].cfg;
   for (int g = 0; g < n_groups; ++g) {
@@ -773,13 +700,9 @@ extern "C" int mdpp_set_image_continuous_groups(mdpp_ctx* ctx,
         c.stamp_rows > MDPP_MAX_STAMP_ROWS || c.n_rects > MDPP_MAX_TERM_BOXES)
       return fail(ctx, MDPP_EINVAL, which + ": bad configuration");
   }
-  release_continuous_groups(ctx);
-  rc = upload_groups(ctx, groups, n_groups, env_group, &ctx->img_c_groups,
-                     &ctx->img_c_env_group);
-  if (rc) { release_continuous_groups(ctx); return rc; }
+  rc = install_groups(ctx, ctx->img_c_set, groups, n_groups, /*block=*/0);
+  if (rc) return rc;
   ctx->img_c_first = c0;
-  ctx->img_c_n_groups = n_groups;
-  ctx->img_c_total_envs = (int64_t)env_group.size();
   return MDPP_OK;
 }
 
@@ -787,21 +710,19 @@ extern "C" int mdpp_render_continuous_groups(mdpp_ctx* ctx, const void* states,
                                              uint8_t* out, int64_t n_images,
                                              int64_t n_envs, void* cuda_stream) {
   if (!ctx) return MDPP_EINVAL;
-  if (!ctx->img_c_groups)
+  if (!ctx->img_c_set.groups)
     return fail(ctx, MDPP_EINVAL, "render_continuous_groups: no image groups set");
   if (!states || !out || n_images < 1 || n_envs < 1)
     return fail(ctx, MDPP_EINVAL, "render_continuous_groups: bad arguments");
-  if (n_envs != ctx->img_c_total_envs)
-    return fail(ctx, MDPP_EINVAL, "render_continuous_groups: n_envs = " +
-                std::to_string(n_envs) + " differs from the groups' total of " +
-                std::to_string(ctx->img_c_total_envs) + " envs");
+  int rc = bind_groups(ctx, ctx->img_c_set, "render_continuous_groups", n_envs);
+  if (rc) return rc;
   if (n_images * ctx->img_c_first.n_sub_images > 0x7fffffffLL)
     return fail(ctx, MDPP_EINVAL, "render_continuous_groups: too many images per call");
   MDPP_CUDA(ctx, cudaSetDevice(ctx->device));
   RenderCParams p;
   p.cfg = ctx->img_c_first;
-  p.groups = ctx->img_c_groups;
-  p.env_group = ctx->img_c_env_group;
+  p.groups = static_cast<const mdpp_image_continuous_group*>(ctx->img_c_set.groups);
+  p.env_group = ctx->img_c_set.env_group;
   p.n_envs = n_envs;
   p.states = states;
   p.out = out;

@@ -69,11 +69,9 @@ class DiscreteEnv(VectorRLToyEnv):
         self._adt = torch.int32
         self._obs_dtype_override = None  # set_obs_dtype()
         self._io_cache = None            # rollout()'s last marshalled launch
-        groups = (_lib.DiscreteGroup * G)()
+        groups = self._group_array(_lib.DiscreteGroup)
         self._host_keep = []
-        for gi, (s_, t_, (begin, count, id_base)) in enumerate(
-                zip(specs, self.group_tables, self._group_layout())):
-            g = groups[gi]
+        for g, s_, t_ in zip(groups, specs, self.group_tables):
             g.n_states, g.n_actions = t_.n_states, t_.n_actions
             g.sequence_length, g.delay = s_.sequence_length, s_.delay
             g.reward_every_n_steps = s_.reward_every_n_steps
@@ -96,7 +94,6 @@ class DiscreteEnv(VectorRLToyEnv):
                 keep.extend(keep_irr)
                 (g.transition_irr, g.init_cdf_irr,
                  g.noise_cdf_irr) = _host_ptrs(keep_irr)
-            g.env_begin, g.env_count, g.global_id_base = begin, count, id_base
         self._check(self._lib.mdpp_set_discrete_groups(self._ctx, groups, G))
         max_delay = max(s_.delay for s_ in specs)
 
@@ -394,11 +391,9 @@ class DiscreteEnv(VectorRLToyEnv):
                                or tb.has_flip
                                for tb, _ in self.image_table_sets.values())
         if self.n_groups > 1:
-            groups = (_lib.ImageDiscreteGroup * self.n_groups)()
-            for g, k, (begin, count, id_base) in zip(groups, keys,
-                                                     self._group_layout()):
+            groups = self._group_array(_lib.ImageDiscreteGroup)
+            for g, k in zip(groups, keys):
                 g.tb = self.image_table_sets[k][1]
-                g.env_begin, g.env_count, g.global_id_base = begin, count, id_base
             self._check(self._lib.mdpp_set_image_discrete_groups(
                 self._ctx, groups, self.n_groups))
         self.obs_shape = (W * self._n_sub, H, 1)

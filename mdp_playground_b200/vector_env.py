@@ -229,6 +229,18 @@ class VectorRLToyEnv:
         return [(s.start, s.stop - s.start, base) for s, base in zip(
             self.group_slices, group_id_bases(self._group_sizes, *self._shard))]
 
+    def _group_array(self, group_cls):
+        """A ctypes array of `group_cls`, one per config group, with env_begin,
+        env_count and (where the struct has it) global_id_base filled in from
+        _group_layout()."""
+        groups = (group_cls * self.n_groups)()
+        has_base = any(f[0] == "global_id_base" for f in group_cls._fields_)
+        for g, (begin, count, id_base) in zip(groups, self._group_layout()):
+            g.env_begin, g.env_count = begin, count
+            if has_base:
+                g.global_id_base = id_base
+        return groups
+
     def _set_configs(self, cfgs, group_cls, set_groups, set_config):
         """Hand the config structs of a continuous or grid env (one per
         group) to the library.  A single configuration keeps its own entry
@@ -240,12 +252,9 @@ class VectorRLToyEnv:
                 self.env_id_offset += self._shard[0] * self.num_envs
             self._check(set_config(self._ctx, C.byref(cfgs[0])))
             return
-        groups = (group_cls * len(cfgs))()
-        for gi, (cfg, (begin, count, id_base)) in enumerate(
-                zip(cfgs, self._group_layout())):
-            g = groups[gi]
+        groups = self._group_array(group_cls)
+        for g, cfg in zip(groups, cfgs):
             g.cfg = cfg
-            g.env_begin, g.env_count, g.global_id_base = begin, count, id_base
         self._check(set_groups(self._ctx, groups, len(cfgs)))
 
     def _check_image_groups(self):
@@ -269,10 +278,9 @@ class VectorRLToyEnv:
         self._img_cfg = cfgs[0]
         if len(cfgs) == 1:
             return
-        groups = (_lib.ImageContinuousGroup * len(cfgs))()
-        for g, cfg, (begin, count, _) in zip(groups, cfgs, self._group_layout()):
+        groups = self._group_array(_lib.ImageContinuousGroup)
+        for g, cfg in zip(groups, cfgs):
             g.cfg = cfg
-            g.env_begin, g.env_count = begin, count
         self._check(self._lib.mdpp_set_image_continuous_groups(
             self._ctx, groups, len(cfgs)))
 

@@ -481,6 +481,36 @@ int mdpp_grid_reset(mdpp_ctx* ctx, const mdpp_grid_state* st,
                     int64_t* obs, const mdpp_step_opts* opts, void* cuda_stream);
 #endif
 
+/* Tabular Q-learning fused into the grid rollout (like mdpp_discrete_qlearn):
+ * T steps of epsilon-greedy Q-learning, one Q-table per env, in one launch.
+ * The state of env i is its cell pos[0..n_dims), every coordinate in
+ * [0, shape_k] (the cell one past the grid included; the caller keeps the
+ * cells in that range), indexed row-major:
+ *   s = sum_k pos[k] * prod_{j>k} (shape_j + 1),  S = prod_k (shape_k + 1).
+ * Action index a in [0, A), A = 2 n_dims + 1: 0 = the no-op, 1 + 2k = -1 on
+ * dim k, 2 + 2k = +1 on dim k (the distinct GridActionSpace members).  At
+ * global step `step` env i (global Philox id g) draws
+ * w = philox(g, step >> 1, STREAM_GRID_ACTION = 45); words (x, y) belong to
+ * the even step, (z, w) to the odd one.  It explores iff the first word
+ * < ceil(epsilon * 2^32) (then a = umulhi(second word, A)), else
+ * a = argmax_a' q[i][s][a'] (ties: lowest index), steps like
+ * mdpp_grid_rollout with that action row (transition noise may substitute
+ * the move; the update is still made for a), and updates, with r the
+ * returned reward and nxt the cell before any auto-reset,
+ *   target = terminated ? r : r + gamma * max_a' q[i][nxt][a']
+ *   q[i][s][a] += alpha * (target - q[i][s][a])
+ * in float64 with every operation rounded on its own (no FMA).  Truncation
+ * bootstraps.  The env state and statistics end as mdpp_grid_rollout leaves
+ * them with the same action rows.  q is [N][q_states][q_actions] with
+ * q_states >= every group's S and q_actions >= A; `actions_taken` receives
+ * the action index.  `io->actions` must be NULL; the other outputs of `io`
+ * and `actions_taken` may be NULL (skipped).  Philox noise only.            */
+#ifndef __CUDACC_RTC__ /* NVRTC sees the types only */
+int mdpp_grid_qlearn(mdpp_ctx* ctx, const mdpp_grid_state* st,
+                     const mdpp_grid_io* io, const mdpp_qlearn_params* qp,
+                     const mdpp_step_opts* opts, void* cuda_stream);
+#endif
+
 /* ------------------------------------------------------------------------
  * Image observations (replaces ImageMultiDiscrete.generate_image,
  * spaces/image_multi_discrete.py:129-270, and ImageContinuous.generate_image

@@ -36,7 +36,7 @@ EXPORTED_SYMBOLS = (
     "mdpp_set_grid_groups",
     "mdpp_set_image_discrete_groups", "mdpp_render_discrete_groups",
     "mdpp_set_image_continuous_groups", "mdpp_render_continuous_groups",
-    "mdpp_discrete_qlearn",
+    "mdpp_discrete_qlearn", "mdpp_grid_qlearn",
 )
 MDPP_MAX_DIM, MDPP_MAX_ORDER, MDPP_MAX_TERM_BOXES = 16, 4, 8
 
@@ -324,6 +324,9 @@ def load():
     lib.mdpp_set_grid_groups.argtypes = [P, C.POINTER(GridGroup), C.c_int32]
     lib.mdpp_grid_rollout.argtypes = [
         P, C.POINTER(GridState), C.POINTER(GridIO), C.POINTER(StepOpts), P]
+    lib.mdpp_grid_qlearn.argtypes = [
+        P, C.POINTER(GridState), C.POINTER(GridIO), C.POINTER(QlearnParams),
+        C.POINTER(StepOpts), P]
     lib.mdpp_grid_reset.argtypes = [
         P, C.POINTER(GridState), P, P, P, C.POINTER(StepOpts), P]
     lib.mdpp_tail_actions.argtypes = [

@@ -79,6 +79,26 @@ struct RolloutParams {
   const uint8_t* zig;  // ziggurat tables (ziggurat.cuh), MDPP_NORMAL_ZIGGURAT
 };
 
+// What a learner riding along a rollout kernel sees of one step
+// (discrete_kernels.cuh rollout_body, grid.cu grid_rollout_kernel).
+struct StepOut {
+  double r;      // the returned reward
+  int32_t nxt;   // state (grid: cell index) before any auto-reset (final_obs)
+  bool done, trunc;
+};
+
+// Device view of mdpp_qlearn_params (qlearn.cu check_qlearn_params).
+struct QlearnDev {
+  double* q;
+  int32_t q_states, q_actions;
+  double alpha, gamma;
+  uint64_t explore_below;  // explore iff the exploring word < ceil(epsilon * 2^32)
+  double* ep_return;
+  double* ret_sum;
+  int32_t* ret_count;
+  int32_t* actions_taken;
+};
+
 struct ResetParams {
   const DiscreteGroupDev* groups;
   const uint8_t* blob;

@@ -469,12 +469,6 @@ struct Cfg {
 // act()    picks the action of a step from the random one and the env state,
 // update() sees the step's outcome (StepOut) and the state after any reset,
 // begin() / end() load and store per-env agent state around the launch.
-struct StepOut {
-  double r;      // the returned reward
-  int32_t nxt;   // state before any auto-reset (final_obs)
-  bool done, trunc;
-};
-
 struct NoAgent {
   static constexpr bool kStepOut = false;  // chain_step hands out no StepOut
   __device__ __forceinline__ void begin(const GroupView&, int64_t, int32_t) {}

@@ -12,6 +12,9 @@
 // is time-major with one 16- / 32-byte row per env and step (action rows are
 // prefetched a step ahead).  Integer arithmetic and fp64 rewards in the
 // reference's operation order: bit-exact.
+// The second half of the file is mdpp_grid_qlearn: the same rollout kernel with
+// a tabular Q-learner choosing the actions instead of the action rows.
+#include <algorithm>
 #include <cstring>
 #include <vector>
 
@@ -121,6 +124,16 @@ __device__ __forceinline__ uint32_t pack_action(const Row<ND>& r) {
   return (valid && moves <= 1) ? code : 0x80000000u;
 }
 
+// Q-table row of a cell: row-major over [0, shape_k] (reset draws the cell one
+// past the grid too)
+template <int ND>
+__device__ __forceinline__ int32_t cell_index(const mdpp_grid_config& c, const int32_t* pos) {
+  int32_t s = pos[0];
+#pragma unroll
+  for (int k = 1; k < ND; ++k) s = s * (c.shape[k] + 1) + pos[k];
+  return s;
+}
+
 template <int ND>
 __device__ __forceinline__ void st_row(int64_t* p, const int32_t* c) {
 #pragma unroll
@@ -186,11 +199,13 @@ struct GridEnv {
 // terminated, truncated written, no final_obs), so no per-step NULL tests.
 // NORMAL: generator of the reward normals (MDPP_NORMAL_*), a template
 // parameter so that each kernel carries one generator's registers only.
+// `so` (a learner's launch only): the step's outcome before any auto-reset.
 template <int ND, int NOISE, bool FAST, int NORMAL>
 __device__ __forceinline__ void grid_step(const GridParams& p, const mdpp_grid_config& c,
                                           GridEnv<ND>& g,
                                           uint32_t code, int64_t off, uint64_t step,
-                                          uint32_t gid, uint32_t pn_T, double term_add) {
+                                          uint32_t gid, uint32_t pn_T, double term_add,
+                                          StepOut* so = nullptr) {
   // GridActionSpace.contains: entries in {-1, 0, 1}, at most one move
   const bool valid = (code >> 31) == 0;
   int32_t a[ND];
@@ -299,6 +314,7 @@ __device__ __forceinline__ void grid_step(const GridParams& p, const mdpp_grid_c
   if (done) r = __dadd_rn(r, term_add);
   const bool trunc = p.horizon > 0 && g.tl >= p.horizon;
   g.n_term += done;
+  if (so) *so = StepOut{r, cell_index<ND>(c, g.pos), done, trunc};
   if (!FAST && p.io.final_obs) st_row<ND>(p.io.final_obs + off * ND, g.pos);
   if (p.autoreset && (done || trunc)) {
     if (NOISE == MDPP_NOISE_REPLAY) {
@@ -322,9 +338,23 @@ __device__ __forceinline__ void grid_step(const GridParams& p, const mdpp_grid_c
   if (FAST || p.io.truncated) __stcs(p.io.truncated + off, (uint8_t)trunc);
 }
 
-template <int ND, int NOISE, bool FAST, bool GROUPS = false, int NORMAL = MDPP_NORMAL_F64>
-__global__ void __launch_bounds__(kGBlock, ND == 2 ? 5 : 4)
-grid_rollout_kernel(const __grid_constant__ GridParams p) {
+// The rollout takes its actions from the action rows (NoGridAgent) or from a
+// learner (GridQAgent below), which acts, sees each step's StepOut and the
+// cell after any auto-reset, and loads / stores its per-env state around the
+// launch (begin / end).  The agent also names the kernel's parameter struct
+// and its occupancy target (kMinBlocks; 0: the rollout's own).
+struct NoGridAgent {
+  static constexpr bool kActs = false;
+  static constexpr int kMinBlocks = 0;
+  using Params = GridParams;
+  __device__ __forceinline__ explicit NoGridAgent(const GridParams&) {}
+};
+
+template <int ND, int NOISE, bool FAST, bool GROUPS = false, int NORMAL = MDPP_NORMAL_F64,
+          typename AG = NoGridAgent>
+__global__ void __launch_bounds__(kGBlock, AG::kMinBlocks ? AG::kMinBlocks : ND == 2 ? 5 : 4)
+grid_rollout_kernel(const __grid_constant__ typename AG::Params p) {
+  AG ag(p);
   __shared__ double red[kGBlock / 32];
   __shared__ GridGroupSmem<GROUPS> gsm;
   const GridSel sel = select_group<GROUPS>(p, gsm);
@@ -351,7 +381,20 @@ grid_rollout_kernel(const __grid_constant__ GridParams p) {
   const uint32_t pn_T = (uint32_t)fmin(
       floor(c.transition_noise * 4294967296.0 + 0.5), 4294967295.0);
   const double term_add = c.term_state_reward * c.reward_scale;
-  if (active) {
+  if constexpr (AG::kActs) {
+    if (active) {
+      ag.begin(c, e, g.pos);
+      for (int t = 0; t < p.T; ++t) {
+        const int64_t off = (int64_t)t * N + e;
+        const uint64_t step = step_base + (uint64_t)t;
+        StepOut so;
+        grid_step<ND, NOISE, FAST, NORMAL>(p, c, g, ag.act(p, gid, step), off, step, gid,
+                                           pn_T, term_add, &so);
+        ag.update(p, c, so, g.pos, e, off);
+      }
+      ag.end(e);
+    }
+  } else if (active) {
     // Action rows run 4 steps ahead of their use (a DRAM read under the
     // write-heavy stream takes longer than one step's arithmetic).  The ring
     // holds the RAW rows: touching a row before its turn would stall on the
@@ -386,6 +429,8 @@ grid_rollout_kernel(const __grid_constant__ GridParams p) {
         grid_step<ND, NOISE, FAST, NORMAL>(p, c, g, pack_action<ND>(ring[j]),
                                    (int64_t)(t0 + j) * N + e,
                                    step_base + (uint64_t)(t0 + j), gid, pn_T, term_add);
+  }
+  if (active) {
 #pragma unroll
     for (int k = 0; k < ND; ++k) p.st.pos[(int64_t)k * N + e] = g.pos[k];
     p.st.t_episode[e] = g.tl;
@@ -451,9 +496,128 @@ grid_reset_kernel(const __grid_constant__ GridParams p) {
   if (p.st.prev) p.st.prev[env] = p.st.prev[N + env] = -1;
 }
 
+// ---- tabular Q-learning (mdpp_grid_qlearn) ----------------------------------
+// Per env and step (global step `step`, Philox id g, cell index s):
+//   w = philox(g, step >> 1, STREAM_GRID_ACTION), (x, y) / (z, w) = even / odd step
+//   a = first word < ceil(epsilon * 2^32) ? umulhi(second word, A) : argmax Q[s]
+//   step -> r, nxt (before any auto-reset), terminated
+//   target = terminated ? r : r + gamma * max_a' Q[nxt][a']
+//   Q[s][a] = q + alpha * (target - q)
+// in float64 with every operation rounded on its own, like QAgent (qlearn.cu).
+// Action index a: 0 = no-op, 1 + 2k = -1 on dim k, 2 + 2k = +1 on dim k.
+// Q is float64 [N][q_states][q_actions], env-major; the host passes q_actions
+// = 8 for 2-D grids, so a row is one 64-byte line.
+struct GridQlearnParams : GridParams {
+  QlearnDev q;
+};
+
+template <int ND>
+struct GridQAgent {
+  static constexpr bool kActs = true;
+  // 65 536 envs are 512 CTAs of 128, 4 per SM on 148 SMs: at most 128
+  // registers a thread keep them resident (one wave)
+  static constexpr int kMinBlocks = 4;
+  using Params = GridQlearnParams;
+  static constexpr int A = 2 * ND + 1;
+  const QlearnDev& d;
+  double* tab;      // this env's Q-table
+  int32_t greedy;   // argmax of the current cell's row
+  int32_t s, a;     // the step's cell index and action
+  double ep_ret;    // return of the running episode
+  uint64_t cached;  // step >> 1 of w
+  U4 w;
+
+  __device__ __forceinline__ explicit GridQAgent(const GridQlearnParams& p) : d(p.q) {}
+
+  // (max, lowest argmax) of row st; numpy.argmax order
+  __device__ __forceinline__ int32_t row_argmax(int32_t st, double& m) const {
+    const double* row = tab + (int64_t)st * d.q_actions;
+    m = row[0];
+    int32_t am = 0;
+#pragma unroll
+    for (int k = 1; k < A; ++k) {
+      const double x = row[k];
+      if (x > m) { m = x; am = k; }
+    }
+    return am;
+  }
+
+  __device__ __forceinline__ void begin(const mdpp_grid_config& c, int64_t env,
+                                        const int32_t* pos) {
+    tab = d.q + env * (int64_t)d.q_states * d.q_actions;
+    s = cell_index<ND>(c, pos);
+    double m;
+    greedy = row_argmax(s, m);
+    ep_ret = d.ep_return[env];
+    cached = ~0ull;
+  }
+
+  // the step's action, packed like pack_action
+  __device__ __forceinline__ uint32_t act(const GridParams& p, uint32_t gid, uint64_t step) {
+    if ((step >> 1) != cached) {  // uniform over the launch
+      cached = step >> 1;
+      w = philox4x32_10(gid, (uint32_t)cached, (uint32_t)(cached >> 32), STREAM_GRID_ACTION,
+                        p.k0, p.k1);
+    }
+    const uint32_t w_explore = (step & 1) ? w.z : w.x;
+    const uint32_t w_action = (step & 1) ? w.w : w.y;
+    a = (uint64_t)w_explore < d.explore_below ? (int32_t)__umulhi(w_action, (uint32_t)A)
+                                              : greedy;
+    constexpr uint32_t noop = ND == 2 ? 0x5u : 0x55u;  // every entry 0 (code 1)
+    const uint32_t one = 1u << (2 * ((a - 1) >> 1));
+    return a == 0 ? noop : (a & 1) ? noop - one : noop + one;
+  }
+
+  __device__ __forceinline__ void update(const GridParams& p, const mdpp_grid_config& c,
+                                         const StepOut& o, const int32_t* pos_after,
+                                         int64_t env, int64_t off) {
+    double* q_at = tab + (int64_t)s * d.q_actions + a;
+    const double q = *q_at;  // (loaded beside the row of nxt)
+    double m;
+    const int32_t am = row_argmax(o.nxt, m);
+    const double target = o.done ? o.r : __dadd_rn(o.r, __dmul_rn(d.gamma, m));
+    const double qn = __dadd_rn(q, __dmul_rn(d.alpha, __dsub_rn(target, q)));
+    *q_at = qn;
+    const bool reset = p.autoreset && (o.done || o.trunc);
+    if (reset) {
+      const int32_t s_after = cell_index<ND>(c, pos_after);
+      greedy = row_argmax(s_after, m);
+      s = s_after;
+    } else {
+      if (o.nxt != s) {
+        greedy = am;
+      } else if (a != am) {  // the row just loaded changed in entry a only
+        greedy = (qn > m || (qn == m && a < am)) ? a : am;
+      } else {  // the maximum itself changed: rescan unless it only grew
+        greedy = qn >= m ? am : row_argmax(s, m);
+      }
+      s = o.nxt;
+    }
+    ep_ret = __dadd_rn(ep_ret, o.r);
+    if (reset) {
+      d.ret_sum[env] = __dadd_rn(d.ret_sum[env], ep_ret);
+      d.ret_count[env] += 1;
+      ep_ret = 0.0;
+    }
+    if (d.actions_taken) __stcs(d.actions_taken + off, a);
+  }
+
+  __device__ __forceinline__ void end(int64_t env) { d.ep_return[env] = ep_ret; }
+};
+
+
 }  // namespace mdpp
 
 using namespace mdpp;
+
+// prod_k (shape_k + 1), the cells of a grid (one past the grid included),
+// capped at 2^31
+static int64_t grid_states(const mdpp_grid_config& c) {
+  int64_t n = 1;
+  for (int k = 0; k < c.n_dims; ++k)
+    n = std::min<int64_t>(n * ((int64_t)c.shape[k] + 1), (int64_t)1 << 31);
+  return n;
+}
 
 static int check_grid_config(mdpp_ctx* ctx, const mdpp_grid_config* cfg) {
   if (!cfg) return fail(ctx, MDPP_EINVAL, "cfg is NULL");
@@ -476,6 +640,7 @@ extern "C" int mdpp_set_grid_config(mdpp_ctx* ctx, const mdpp_grid_config* cfg) 
   if (rc) return rc;
   release_groups(ctx->g_set);
   ctx->g_cfg = *cfg;
+  ctx->g_states = grid_states(*cfg);
   ctx->have_grid = true;
   return MDPP_OK;
 }
@@ -488,6 +653,7 @@ extern "C" int mdpp_set_grid_groups(mdpp_ctx* ctx, const mdpp_grid_group* groups
   std::vector<GridGroupDev> dev(n_groups);
   // the launch-wide view: flags any group has (which replay arrays are needed)
   mdpp_grid_config view = groups[0].cfg;
+  int64_t states = 0;
   for (int g = 0; g < n_groups; ++g) {
     const mdpp_grid_config& c = groups[g].cfg;
     rc = check_grid_config(ctx, &c);
@@ -501,10 +667,12 @@ extern "C" int mdpp_set_grid_groups(mdpp_ctx* ctx, const mdpp_grid_group* groups
     dev[g].gid_base = groups[g].global_id_base;
     view.has_transition_noise |= c.has_transition_noise;
     view.has_reward_noise |= c.has_reward_noise;
+    states = std::max(states, grid_states(c));
   }
   rc = install_groups(ctx, ctx->g_set, dev.data(), n_groups, kGBlock);
   if (rc) return rc;
   ctx->g_cfg = view;
+  ctx->g_states = states;
   ctx->have_grid = true;
   return MDPP_OK;
 }
@@ -630,4 +798,49 @@ extern "C" int mdpp_grid_reset(mdpp_ctx* ctx, const mdpp_grid_state* st,
   else grid_reset_kernel<2><<<grid, kGBlock, 0, s>>>(p);
   MDPP_CUDA(ctx, cudaGetLastError());
   return MDPP_OK;
+}
+
+template <int ND, bool GROUPS>
+static int launch_grid_qlearn(mdpp_ctx* ctx, const GridQlearnParams& qp, int normal_mode,
+                              cudaStream_t s) {
+  const unsigned grid = GROUPS ? (unsigned)ctx->g_set.n_ctas
+                               : (unsigned)((qp.st.n_envs + kGBlock - 1) / kGBlock);
+  if (normal_mode == MDPP_NORMAL_ZIGGURAT)
+    grid_rollout_kernel<ND, MDPP_NOISE_PHILOX, false, GROUPS, MDPP_NORMAL_ZIGGURAT, GridQAgent<ND>><<<grid, kGBlock, 0, s>>>(qp);
+  else if (normal_mode == MDPP_NORMAL_FAST)
+    grid_rollout_kernel<ND, MDPP_NOISE_PHILOX, false, GROUPS, MDPP_NORMAL_FAST, GridQAgent<ND>><<<grid, kGBlock, 0, s>>>(qp);
+  else
+    grid_rollout_kernel<ND, MDPP_NOISE_PHILOX, false, GROUPS, MDPP_NORMAL_F64, GridQAgent<ND>><<<grid, kGBlock, 0, s>>>(qp);
+  MDPP_CUDA(ctx, cudaGetLastError());
+  return MDPP_OK;
+}
+
+extern "C" int mdpp_grid_qlearn(mdpp_ctx* ctx, const mdpp_grid_state* st,
+                                const mdpp_grid_io* io, const mdpp_qlearn_params* qp,
+                                const mdpp_step_opts* opts, void* cuda_stream) {
+  GridQlearnParams k;
+  int rc = fill_grid(ctx, st, opts, &k);
+  if (rc) return rc;
+  if (!io) return fail(ctx, MDPP_EINVAL, "grid qlearn: io is NULL");
+  if (io->actions)
+    return fail(ctx, MDPP_EINVAL, "grid qlearn: io->actions must be NULL (the agent acts)");
+  if (opts->noise_mode != MDPP_NOISE_PHILOX)
+    return fail(ctx, MDPP_EINVAL, "grid qlearn: Philox noise only");
+  if (opts->n_steps < 1) return fail(ctx, MDPP_EINVAL, "grid qlearn: T must be >= 1");
+  if (ctx->g_states > INT32_MAX)
+    return fail(ctx, MDPP_EINVAL, "grid qlearn: a group has more than 2^31 - 1 cells");
+  const int nd = ctx->g_cfg.n_dims;
+  rc = check_qlearn_params(ctx, qp, ctx->g_states, 2 * nd + 1, &k.q);
+  if (rc) return rc;
+  if (((uintptr_t)io->obs | (uintptr_t)io->final_obs) & 15)
+    return fail(ctx, MDPP_EINVAL, "grid rows must be 16-byte aligned");
+  k.io = *io;
+  MDPP_CUDA(ctx, cudaSetDevice(ctx->device));
+  cudaStream_t s = (cudaStream_t)cuda_stream;
+  const int normal = opts->normal_mode;
+  if (k.groups)
+    return nd == 4 ? launch_grid_qlearn<4, true>(ctx, k, normal, s)
+                   : launch_grid_qlearn<2, true>(ctx, k, normal, s);
+  return nd == 4 ? launch_grid_qlearn<4, false>(ctx, k, normal, s)
+                 : launch_grid_qlearn<2, false>(ctx, k, normal, s);
 }

@@ -42,6 +42,7 @@ struct mdpp_ctx {
   bool have_grid = false;
   mdpp_grid_config g_cfg;
   GroupSet g_set;  // GridGroupDev
+  int64_t g_states = 0;  // most cells prod_k (shape_k + 1) of a grid group (capped at 2^31)
   // per-group image renderers: the ABI descriptors as given, with an
   // env -> group map (one load per image); the first-group views hold what
   // the groups share
@@ -81,6 +82,11 @@ int prepare_rollout(mdpp_ctx* ctx, const mdpp_discrete_state* st,
                     const mdpp_discrete_io* io, const mdpp_step_opts* opts,
                     RolloutParams& p);
 int cuda_fail(mdpp_ctx* ctx, cudaError_t e, const char* what);
+// qlearn.cu: the checks of mdpp_qlearn_params that every learner shares (NULL
+// arrays, a table smaller than n_states x n_actions, alpha / gamma / epsilon
+// outside [0, 1]), then its device view
+int check_qlearn_params(mdpp_ctx* ctx, const mdpp_qlearn_params* qp, int64_t n_states,
+                        int64_t n_actions, QlearnDev* d);
 
 // Checks that groups[0..n) cover [0, N) contiguously, in order, with N >= 1, and
 // that a set with an env -> group map has at most 65 535 groups (uint16).

@@ -30,6 +30,9 @@ enum PhiloxStream : uint32_t {
   STREAM_GRID_AUTORESET = 41,
   STREAM_GRID_RESET = 42,
   STREAM_GRID_NORMAL = 43,
+  // grid Q-learning (mdpp_grid_qlearn), counter = (env, step >> 1): (w0, w1) /
+  // (w2, w3) = explore decision + exploring action of the even / odd step
+  STREAM_GRID_ACTION = 45,
   STREAM_RESET_BOX = 64,   // + attempt*16 + dim/4 (continuous reset sampling)
   STREAM_ZIG_RETRY = 0x100,  // + c, counter = step: ziggurat words after a
                              // rejected first attempt (ziggurat.cuh)

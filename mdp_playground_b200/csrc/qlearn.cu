@@ -19,22 +19,12 @@
 // stays resident in the 126 MB L2).  One row load per step sits on the
 // dependent chain: Q[nxt] gives both the target's max and, when no
 // auto-reset follows, the next step's greedy action.
+#include <algorithm>
 #include <cmath>
 
 #include "discrete_launch.h"
 
 namespace mdpp {
-
-struct QlearnDev {
-  double* q;
-  int32_t q_states, q_actions;
-  double alpha, gamma;
-  uint64_t explore_below;  // explore iff w.z < ceil(epsilon * 2^32)
-  double* ep_return;
-  double* ret_sum;
-  int32_t* ret_count;
-  int32_t* actions_taken;
-};
 
 struct QlearnParams {
   RolloutParams base;
@@ -140,6 +130,30 @@ static int launch_qlearn(mdpp_ctx* ctx, QlearnParams& qp, cudaStream_t stream) {
   return launch_kernel<Cg>(ctx, p, smem_tab, stream, discrete_qlearn_kernel<Cg>, qp);
 }
 
+int check_qlearn_params(mdpp_ctx* ctx, const mdpp_qlearn_params* qp, int64_t n_states,
+                        int64_t n_actions, QlearnDev* d) {
+  if (!qp || !qp->q || !qp->ep_return || !qp->ret_sum || !qp->ret_count)
+    return fail(ctx, MDPP_EINVAL, "qlearn: q, ep_return, ret_sum or ret_count is NULL");
+  if (qp->q_states < n_states || qp->q_actions < n_actions)
+    return fail(ctx, MDPP_EINVAL, "qlearn: q_states / q_actions smaller than a group's S / A");
+  // (written so that NaN fails too)
+  if (!(qp->alpha >= 0.0 && qp->alpha <= 1.0) || !(qp->gamma >= 0.0 && qp->gamma <= 1.0) ||
+      !(qp->epsilon >= 0.0 && qp->epsilon <= 1.0))
+    return fail(ctx, MDPP_EINVAL, "qlearn: alpha, gamma and epsilon must lie in [0, 1]");
+  d->q = qp->q;
+  d->q_states = qp->q_states;
+  d->q_actions = qp->q_actions;
+  d->alpha = qp->alpha;
+  d->gamma = qp->gamma;
+  // w < x for an integer w <=> w < ceil(x); x = epsilon * 2^32 is exact
+  d->explore_below = (uint64_t)std::ceil(qp->epsilon * 4294967296.0);
+  d->ep_return = qp->ep_return;
+  d->ret_sum = qp->ret_sum;
+  d->ret_count = qp->ret_count;
+  d->actions_taken = qp->actions_taken;
+  return MDPP_OK;
+}
+
 }  // namespace mdpp
 
 using namespace mdpp;
@@ -157,26 +171,13 @@ extern "C" int mdpp_discrete_qlearn(mdpp_ctx* ctx, const mdpp_discrete_state* st
     return fail(ctx, MDPP_EINVAL, "qlearn: Philox noise only");
   if (ctx->d_irr)
     return fail(ctx, MDPP_EINVAL, "qlearn: irrelevant features are not supported");
-  if (!qp || !qp->q || !qp->ep_return || !qp->ret_sum || !qp->ret_count)
-    return fail(ctx, MDPP_EINVAL, "qlearn: q, ep_return, ret_sum or ret_count is NULL");
-  for (auto& g : ctx->d_groups_host)
-    if (qp->q_states < g.S || qp->q_actions < g.A)
-      return fail(ctx, MDPP_EINVAL, "qlearn: q_states / q_actions smaller than a group's S / A");
-  // (written so that NaN fails too)
-  if (!(qp->alpha >= 0.0 && qp->alpha <= 1.0) || !(qp->gamma >= 0.0 && qp->gamma <= 1.0) ||
-      !(qp->epsilon >= 0.0 && qp->epsilon <= 1.0))
-    return fail(ctx, MDPP_EINVAL, "qlearn: alpha, gamma and epsilon must lie in [0, 1]");
-  k.q.q = qp->q;
-  k.q.q_states = qp->q_states;
-  k.q.q_actions = qp->q_actions;
-  k.q.alpha = qp->alpha;
-  k.q.gamma = qp->gamma;
-  // w.z < x for an integer w.z <=> w.z < ceil(x); x = epsilon * 2^32 is exact
-  k.q.explore_below = (uint64_t)std::ceil(qp->epsilon * 4294967296.0);
-  k.q.ep_return = qp->ep_return;
-  k.q.ret_sum = qp->ret_sum;
-  k.q.ret_count = qp->ret_count;
-  k.q.actions_taken = qp->actions_taken;
+  int64_t S = 0, A = 0;
+  for (auto& g : ctx->d_groups_host) {
+    S = std::max<int64_t>(S, g.S);
+    A = std::max<int64_t>(A, g.A);
+  }
+  rc = check_qlearn_params(ctx, qp, S, A, &k.q);
+  if (rc) return rc;
   cudaStream_t s = (cudaStream_t)cuda_stream;
   switch (opts->normal_mode) {
     case MDPP_NORMAL_FAST: return launch_qlearn<MDPP_NORMAL_FAST>(ctx, k, s);

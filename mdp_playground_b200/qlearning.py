@@ -1,18 +1,22 @@
-"""Tabular Q-learning inside the discrete rollout kernel.
+"""Tabular Q-learning inside the discrete and grid rollout kernels.
 
 `TabularQLearner(env)` gives every env of a discrete VectorRLToyEnv its own
 Q-table, float64 [N, S_max, A_max] on the device, and trains all of them in
 one fused launch per `learn(T)` call (mdpp_discrete_qlearn,
 include/mdpp_b200.h): epsilon-greedy action selection, the env step and the
-one-step Q-learning update, T steps per launch.  Each env is one independent
+one-step Q-learning update, T steps per launch.  `GridQLearner(env)` does the
+same for a grid env (mdpp_grid_qlearn).  Each env is one independent
 training run (one seed); in a grouped env each config group is one cell of an
 experiment grid.
 
-The exploring action is the random policy's own draw (`rollout(actions=None)`
-at the same global step), so with epsilon = 1 `learn` takes exactly the
-actions a random rollout would take.  The env's step counter advances by T,
-like rollout(), so later rollout / step / reseed calls behave as they would
-after a rollout of T steps.
+Discrete envs explore with the random policy's own draw (`rollout(actions=
+None)` at the same global step), so with epsilon = 1 `learn` takes exactly
+the actions a random rollout would take.  Grid envs explore with a stream of
+their own; a grid state is the cell's row-major index over [0, shape_k] (the
+cell one past the grid that reset draws included), an action the index of a
+GridActionSpace member (grid_action_rows).  The env's step counter advances
+by T, like rollout(), so later rollout / step / reseed calls behave as they
+would after a rollout of T steps.
 """
 import ctypes as C
 
@@ -21,6 +25,20 @@ import torch
 
 from . import _lib
 from ._lib import _ptr
+
+
+def grid_action_rows(nd):
+    """The kernel's grid action indices as rows: 0 = no-op, 1 + 2k = -1 on
+    dim k, 2 + 2k = +1 on dim k.  int64 [2 nd + 1, nd]."""
+    rows = np.zeros((2 * nd + 1, nd), dtype=np.int64)
+    for k in range(nd):
+        rows[1 + 2 * k, k], rows[2 + 2 * k, k] = -1, 1
+    return rows
+
+
+def grid_cells(shape):
+    """Q-table rows of a grid: prod_k (shape_k + 1)."""
+    return int(np.prod([int(n) + 1 for n in shape]))
 
 
 def _unit(name, x):
@@ -32,30 +50,26 @@ def _unit(name, x):
 
 class TabularQLearner:
     """Per-env tabular Q-learning on a discrete env (Philox noise, no
-    irrelevant features, no image observations).
+    irrelevant features, no image observations).  Grid envs train with
+    GridQLearner.
 
     q: float64 [N, S_max, A_max] device tensor (S_max / A_max over the config
     groups; entries beyond an env's own S or A stay at q_init)."""
 
     def __init__(self, env, alpha=0.1, gamma=0.99, epsilon=0.1, q_init=0.0):
-        from .discrete_env import DiscreteEnv
-        if not isinstance(env, DiscreteEnv):
-            raise ValueError("TabularQLearner needs a discrete env "
-                             f"(got {type(env).__name__})")
+        self._check_env(env)
         if env.noise != "philox":
-            raise ValueError("TabularQLearner needs noise='philox' "
+            raise ValueError(f"{type(self).__name__} needs noise='philox' "
                              f"(got {env.noise!r})")
-        if env._irr:
-            raise ValueError("TabularQLearner does not support irrelevant_features")
         if any(s_.image_representations for s_ in env._group_specs):
-            raise ValueError("TabularQLearner does not support image_representations")
+            raise ValueError(f"{type(self).__name__} does not support "
+                             "image_representations")
         self.env = env
         self.alpha = _unit("alpha", alpha)
         self.gamma = _unit("gamma", gamma)
         self.epsilon = _unit("epsilon", epsilon)
         N, dev = env.num_envs, env.device
-        S = max(t.n_states for t in env.group_tables)
-        A = max(t.n_actions for t in env.group_tables)
+        S, A = self._table_shape()
         self.q = torch.full((N, S, A), float(q_init), dtype=torch.float64, device=dev)
         # return of each env's running episode, and sum / count of the returns
         # of the episodes that ended in an auto-reset
@@ -63,15 +77,39 @@ class TabularQLearner:
         self.ret_sum = torch.zeros(N, dtype=torch.float64, device=dev)
         self.ret_count = torch.zeros(N, dtype=torch.int32, device=dev)
 
+    # -- what differs between the env kinds -----------------------------------
+    def _check_env(self, env):
+        from .discrete_env import DiscreteEnv
+        if not isinstance(env, DiscreteEnv):
+            raise ValueError("TabularQLearner needs a discrete env (got "
+                             f"{type(env).__name__}; grid envs train with GridQLearner)")
+        if env._irr:
+            raise ValueError("TabularQLearner does not support irrelevant_features")
+
+    def _table_shape(self):
+        tables = self.env.group_tables
+        return max(t.n_states for t in tables), max(t.n_actions for t in tables)
+
+    def _launch(self, *args):
+        return self.env._lib.mdpp_discrete_qlearn(*args)
+
+    def _before_launch(self):
+        pass
+
+    def _actions_out(self, idx):
+        return idx
+
     def learn(self, n_steps, record=False, alpha=None, gamma=None, epsilon=None):
         """T steps of acting, stepping and learning in one launch.  Returns
         None, or with record=True a dict of time-major [T, N] tensors: obs
         (state after the step and any auto-reset), reward, terminated,
-        truncated and the actions taken.  alpha / gamma / epsilon override
-        the constructor's values for this call (e.g. epsilon=0, alpha=0 for a
-        greedy evaluation that leaves q unchanged)."""
+        truncated and the actions taken (GridQLearner: int64 [T, N, n_dims]
+        action rows, which env.rollout(actions=...) accepts).  alpha / gamma
+        / epsilon override the constructor's values for this call (e.g.
+        epsilon=0, alpha=0 for a greedy evaluation that leaves q unchanged)."""
         env = self.env
         T = int(n_steps)
+        self._before_launch()
         qp = _lib.QlearnParams()
         qp.alpha = self.alpha if alpha is None else _unit("alpha", alpha)
         qp.gamma = self.gamma if gamma is None else _unit("gamma", gamma)
@@ -88,10 +126,12 @@ class TabularQLearner:
             qp.actions_taken = _ptr(out["actions"])
         io = env._io(None, out)
         opts = env._opts(T)
-        env._check(env._lib.mdpp_discrete_qlearn(
+        env._check(self._launch(
             env._ctx, C.byref(env._state), C.byref(io), C.byref(qp),
             C.byref(opts), env._stream()))
         env._step_index += T
+        if record:
+            out["actions"] = self._actions_out(out["actions"])
         return out if record else None
 
     def episode_returns(self, clear=False):
@@ -113,3 +153,47 @@ class TabularQLearner:
             self.ret_sum.zero_()
             self.ret_count.zero_()
         return {"episodes": ep, "episode_reward_mean": mean}
+
+
+class GridQLearner(TabularQLearner):
+    """Per-env tabular Q-learning on a grid env (Philox noise, no image
+    observations; 2-D grids and irrelevant_features), one fused launch of
+    mdpp_grid_qlearn per learn(T).  The state is the cell's row-major index
+    over [0, shape_k], one past the grid included (grid_cells), the action
+    the index of a GridActionSpace member (grid_action_rows).
+
+    q: float64 [N, S_max, A], S_max = prod_k (shape_k + 1) over the config
+    groups, A = 8 for 2-D grids (one 64-byte row; 5 actions are used) and 9
+    for 4-D ones.  learn() raises ValueError when a cell lies outside
+    [0, shape_k] (e.g. one set by set_augmented_state): it has no table row."""
+
+    def _check_env(self, env):
+        from .grid_env import GridEnv
+        if not isinstance(env, GridEnv):
+            raise ValueError(f"GridQLearner needs a grid env (got {type(env).__name__})")
+        dev = env.device
+        self._action_rows = torch.as_tensor(grid_action_rows(env._nd), device=dev)
+        # [nd, N] largest coordinate of each env's cells
+        self._cell_max = torch.repeat_interleave(
+            torch.tensor([list(s_.grid_shape) for s_ in env._group_specs],
+                         dtype=torch.int32), torch.tensor(env._group_sizes),
+            dim=0).t().contiguous().to(dev)
+
+    def _table_shape(self):
+        env = self.env
+        return (max(grid_cells(s_.grid_shape) for s_ in env._group_specs),
+                8 if env._nd == 2 else 9)
+
+    def _launch(self, *args):
+        return self.env._lib.mdpp_grid_qlearn(*args)
+
+    def _before_launch(self):
+        pos = self.env._pos
+        if bool(((pos < 0) | (pos > self._cell_max)).any()):
+            raise ValueError("GridQLearner: a grid cell lies outside [0, grid_shape] "
+                             "(set_augmented_state / reset(init_state=...))")
+
+    def _actions_out(self, idx):
+        T, N = idx.shape
+        return torch.index_select(self._action_rows, 0,
+                                  idx.reshape(-1)).reshape(T, N, -1)

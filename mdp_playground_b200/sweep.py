@@ -14,10 +14,11 @@ included: each cell renders with its own image settings (discrete transforms
 and their quantisation, continuous / grid targets, terminal regions and
 bounds).  Only cells that cannot share one launch (different state dimension
 / dtype, image size) get one batched env per cell instead.  `run` steps a
-uniform random policy (or one supplied by the caller); `train` trains a
-tabular Q-learning agent per env of a discrete grid inside the step kernel
-(qlearning.py) and writes a learning curve per cell, one CSV row per
-(training iteration, cell) like the reference's stats files.
+uniform random policy (or one supplied by the caller); `train` (discrete
+experiments) and `train_grid` (grid-world experiments) train a tabular
+Q-learning agent per env inside the step kernel (qlearning.py) and write a
+learning curve per cell, one CSV row per (training iteration, cell) like the
+reference's stats files.
 """
 import copy
 import importlib.util
@@ -147,7 +148,7 @@ class Sweep:
             self.env = self.envs[0]
         self.timesteps = 0
         self._returned = np.zeros(self.n_cells)
-        self.agent = None
+        self.agents = None  # one learner per env of self.envs
         self.train_results = []  # one dict per training iteration
 
     def _try_grouped(self, Env, device, horizon, shard, env_kwargs):
@@ -208,32 +209,55 @@ class Sweep:
         timesteps_total, episode_reward_mean (mean return of the episodes
         completed in the iteration; NaN if none) and episode_len_mean (from
         the episode counters' change over the iteration).  Discrete grids
-        only.  Calling train again continues with the same Q-tables."""
+        only (grid-world experiments: train_grid).  Calling train again
+        continues with the same Q-tables."""
         if self.kind != "discrete":
             raise NotImplementedError(
-                "Sweep.train: tabular Q-learning runs on discrete grids only")
+                "Sweep.train: tabular Q-learning runs on discrete grids only "
+                "(grid-world experiments: Sweep.train_grid)")
         from .qlearning import TabularQLearner
-        if self.agent is None:
-            self.agent = TabularQLearner(self.env, alpha=alpha, gamma=gamma,
-                                         epsilon=epsilon)
-        env = self.env
-        self.agent.episode_returns(clear=True)
+        return self._train(TabularQLearner, iterations, steps_per_iteration,
+                           alpha, gamma, epsilon, chunk)
+
+    def train_grid(self, iterations, steps_per_iteration, alpha=0.1, gamma=0.99,
+                   epsilon=0.1, chunk=256):
+        """train() for grid-world experiments (GridQLearner): one learner on
+        the grouped env, or one per cell when the cells differ in
+        irrelevant_features; results in cell order either way."""
+        if self.kind != "grid":
+            raise NotImplementedError(
+                "Sweep.train_grid: runs grid-world experiments only")
+        from .qlearning import GridQLearner
+        return self._train(GridQLearner, iterations, steps_per_iteration,
+                           alpha, gamma, epsilon, chunk)
+
+    def _train(self, learner, iterations, steps_per_iteration, alpha, gamma,
+               epsilon, chunk):
+        if self.agents is None:
+            self.agents = [learner(e, alpha=alpha, gamma=gamma, epsilon=epsilon)
+                           for e in self.envs]
+
+        def per_cell(dicts, key):  # one value per group of each env, in cell order
+            return np.concatenate([np.asarray(d[key]).reshape(-1) for d in dicts])
+        for ag in self.agents:
+            ag.episode_returns(clear=True)
         for _ in range(int(iterations)):
-            before = env.episode_stats()
+            before = [e.episode_stats() for e in self.envs]
             done = 0
             while done < steps_per_iteration:
                 T = min(chunk, steps_per_iteration - done)
-                self.agent.learn(T, alpha=alpha, gamma=gamma, epsilon=epsilon)
+                for ag in self.agents:
+                    ag.learn(T, alpha=alpha, gamma=gamma, epsilon=epsilon)
                 done += T
             self.timesteps += steps_per_iteration
-            after = env.episode_stats()
-            ret = self.agent.episode_returns(clear=True)
-            d_ep = after["episodes"] - before["episodes"]
-            d_tr = after["transitions"] - before["transitions"]
+            after = [e.episode_stats() for e in self.envs]
+            ret = [ag.episode_returns(clear=True) for ag in self.agents]
+            d_ep = per_cell(after, "episodes") - per_cell(before, "episodes")
+            d_tr = per_cell(after, "transitions") - per_cell(before, "transitions")
             self.train_results.append({
                 "training_iteration": len(self.train_results) + 1,
-                "timesteps_total": after["transitions"],
-                "episode_reward_mean": ret["episode_reward_mean"],
+                "timesteps_total": per_cell(after, "transitions"),
+                "episode_reward_mean": per_cell(ret, "episode_reward_mean"),
                 "episode_len_mean": d_tr / np.maximum(d_ep, 1)})
         return self.train_results
 

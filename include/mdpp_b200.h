@@ -395,6 +395,64 @@ int mdpp_continuous_reset(mdpp_ctx* ctx, const mdpp_continuous_state* st,
                           void* cuda_stream);
 #endif
 
+/* Augmented random search (Mania, Guy & Recht 2018, Algorithm 1, V1 / V1-t)
+ * fused into the continuous rollout: every config group (or the single
+ * configuration) is one ARS run whose envs are the perturbation population.
+ * D = dim, P = D (D + 1); the policy of group g is a = W [obs; 1] with
+ * theta[g] float64 [D][D+1] row-major.  Group sizes are even; local env 2p is
+ * the + member and 2p + 1 the - member of pair p.
+ *   delta_p: word c < ceil(P / 4) = philox(g+ = global id of the + member,
+ *     iteration lo, iteration hi, STREAM_ARS_DELTA = 0x20000 + c); Box-Muller
+ *     (fp64) of (w0, w1) -> entries 4c, 4c + 1, of (w2, w3) -> 4c + 2, 4c + 3
+ *   w = theta + (s noise_std) delta_p, s = +1 / -1, rounded per entry
+ *   a_d = sum_{k=0..D} w[d][k] phi_k, phi = (obs as fp64, 1), every product
+ *     and sum rounded on its own, cast to real, clipped to
+ *     [-(real)action_space_max, (real)action_space_max] when finite
+ * where obs is the state the env last emitted (after any auto-reset).
+ * mdpp_continuous_ars runs T fused steps and adds each returned reward
+ * (as fp64) to fitness[i]; ep_return / ret_sum / ret_count are those of
+ * mdpp_qlearn_params.  mdpp_continuous_ars_update, per group: keeps the
+ * top_directions pairs by max(F+, F-) (ties: lower p), m / sigma_R = mean /
+ * population std of the kept returns (sequential fp64 sums, ascending p, F+
+ * before F-), and, when sigma_R is finite and > 0,
+ *   theta[j] += (step_size / (b sigma_R)) * sum_{kept p} (F+ - F-) delta_p[j]
+ * (sequential, ascending p); then zeroes fitness and increments `iteration`.
+ * `io->actions` must be NULL; the outputs of `io`, `actions_taken`,
+ * `delta_out` and `group_stats` may be NULL.  Philox noise, no image
+ * observations.  The group layout is the context's (mdpp_set_continuous_
+ * groups), or one group of all envs.                                        */
+typedef struct mdpp_ars_params {
+  double step_size;               /* alpha > 0                               */
+  double noise_std;               /* nu >= 0 (0: every env acts with theta)  */
+  double* theta;                  /* [G][D][D+1] float64 master weights      */
+  double* fitness;                /* [N] reward sum since the last update    */
+  double* ep_return;              /* [N] return of the running episode       */
+  double* ret_sum;                /* [N] sum of the returns of the episodes  */
+  int32_t* ret_count;             /* [N] ... that ended in an auto-reset     */
+  void* actions_taken;            /* real [T][N][D] or NULL                  */
+  int32_t top_directions;         /* b in [1, smallest group's pairs]        */
+  int32_t reserved0;
+  uint64_t iteration;             /* counter word of delta; update adds 1    */
+  uint64_t seed;                  /* update / perturbations: the Philox seed */
+  int64_t env_id_offset;          /* and env_id_offset of the learn launches
+                                     (mdpp_continuous_ars takes opts')       */
+  double* delta_out;             /* [N/2][D][D+1] float64 or NULL           */
+  double* group_stats;            /* update: [G][3] (m, sigma_R, updated 0/1)
+                                     or NULL                                 */
+} mdpp_ars_params;
+
+#ifndef __CUDACC_RTC__ /* NVRTC sees the types only */
+int mdpp_continuous_ars(mdpp_ctx* ctx, const mdpp_continuous_state* st,
+                        const mdpp_continuous_io* io, const mdpp_ars_params* ap,
+                        const mdpp_step_opts* opts, void* cuda_stream);
+/* the update above; writes the iteration's delta to delta_out when given    */
+int mdpp_continuous_ars_update(mdpp_ctx* ctx, int64_t n_envs, mdpp_ars_params* ap,
+                               void* cuda_stream);
+/* writes the current iteration's delta to delta_out only (no update)        */
+int mdpp_continuous_ars_perturbations(mdpp_ctx* ctx, int64_t n_envs,
+                                      const mdpp_ars_params* ap, void* cuda_stream);
+#endif
+
 /* ------------------------------------------------------------------------
  * Grid environments, reward_function "move_to_a_point" (replaces
  * RLToyEnv.transition_function :1727-1778, reward_function :1947-1965 + tail

@@ -7,6 +7,8 @@ reset/step semantics and runs every step on hand-written sm_100a CUDA kernels
 from .vector_env import VectorRLToyEnv  # noqa: F401
 from .wrapper_tail import VectorGymEnvTail  # noqa: F401
 from .qlearning import GridQLearner, TabularQLearner  # noqa: F401
+from .ars import LinearARS  # noqa: F401
 
-__all__ = ["VectorRLToyEnv", "VectorGymEnvTail", "TabularQLearner", "GridQLearner"]
+__all__ = ["VectorRLToyEnv", "VectorGymEnvTail", "TabularQLearner", "GridQLearner",
+           "LinearARS"]
 __version__ = "0.1.0"

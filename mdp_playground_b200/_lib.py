@@ -37,6 +37,8 @@ EXPORTED_SYMBOLS = (
     "mdpp_set_image_discrete_groups", "mdpp_render_discrete_groups",
     "mdpp_set_image_continuous_groups", "mdpp_render_continuous_groups",
     "mdpp_discrete_qlearn", "mdpp_grid_qlearn",
+    "mdpp_continuous_ars", "mdpp_continuous_ars_update",
+    "mdpp_continuous_ars_perturbations",
 )
 MDPP_MAX_DIM, MDPP_MAX_ORDER, MDPP_MAX_TERM_BOXES = 16, 4, 8
 
@@ -107,6 +109,19 @@ class QlearnParams(C.Structure):
         ("q", C.c_void_p), ("q_states", C.c_int32), ("q_actions", C.c_int32),
         ("ep_return", C.c_void_p), ("ret_sum", C.c_void_p),
         ("ret_count", C.c_void_p), ("actions_taken", C.c_void_p),
+    ]
+
+
+class ArsParams(C.Structure):
+    _fields_ = [
+        ("step_size", C.c_double), ("noise_std", C.c_double),
+        ("theta", C.c_void_p), ("fitness", C.c_void_p),
+        ("ep_return", C.c_void_p), ("ret_sum", C.c_void_p),
+        ("ret_count", C.c_void_p), ("actions_taken", C.c_void_p),
+        ("top_directions", C.c_int32), ("reserved0", C.c_int32),
+        ("iteration", C.c_uint64), ("seed", C.c_uint64),
+        ("env_id_offset", C.c_int64), ("delta_out", C.c_void_p),
+        ("group_stats", C.c_void_p),
     ]
 
 
@@ -306,6 +321,12 @@ def load():
     lib.mdpp_continuous_rollout.argtypes = [
         P, C.POINTER(ContinuousState), C.POINTER(ContinuousIO),
         C.POINTER(StepOpts), P]
+    lib.mdpp_continuous_ars.argtypes = [
+        P, C.POINTER(ContinuousState), C.POINTER(ContinuousIO), C.POINTER(ArsParams),
+        C.POINTER(StepOpts), P]
+    lib.mdpp_continuous_ars_update.argtypes = [P, C.c_int64, C.POINTER(ArsParams), P]
+    lib.mdpp_continuous_ars_perturbations.argtypes = [
+        P, C.c_int64, C.POINTER(ArsParams), P]
     lib.mdpp_continuous_reset.argtypes = [
         P, C.POINTER(ContinuousState), P, P, P, C.POINTER(StepOpts), P]
     lib.mdpp_render_discrete.argtypes = [

@@ -15,7 +15,7 @@ SOURCES = ["context.cu", "discrete.cu", "discrete_off.cu", "discrete_replay.cu",
            "discrete_philox_f64.cu", "discrete_philox_fast.cu",
            "discrete_philox_zig.cu", "continuous.cu",
            "render.cu", "grid.cu", "wrapper_tail.cu",
-           "jit.cu", "qlearn.cu"]
+           "jit.cu", "qlearn.cu", "ars.cu"]
 HEADERS = ["internal.h", "device_types.h", "philox.cuh", "discrete_kernels.cuh",
            "continuous_kernels.cuh", "ziggurat.cuh", "ziggurat_tables.h",
            "discrete_launch.h", "../../include/mdpp_b200.h"]

@@ -44,6 +44,7 @@ extern "C" int mdpp_set_continuous_config(mdpp_ctx* ctx,
   int rc = check_config(ctx, cfg);
   if (rc) return rc;
   release_groups(ctx->c_set);
+  ctx->c_group_ranges.clear();
   ctx->c_cfg = *cfg;
   ctx->have_continuous = true;
   return MDPP_OK;
@@ -85,13 +86,18 @@ extern "C" int mdpp_set_continuous_groups(mdpp_ctx* ctx,
   }
   rc = install_groups(ctx, ctx->c_set, dev.data(), n_groups, kCBlock);
   if (rc) return rc;
+  ctx->c_group_ranges.clear();
+  for (int g = 0; g < n_groups; ++g)
+    ctx->c_group_ranges.insert(ctx->c_group_ranges.end(),
+                               {groups[g].env_begin, groups[g].env_count,
+                                groups[g].global_id_base});
   ctx->c_cfg = view;
   ctx->have_continuous = true;
   return MDPP_OK;
 }
 
-static int fill_params(mdpp_ctx* ctx, const mdpp_continuous_state* st,
-                       const mdpp_step_opts* opts, ContinuousParams* p) {
+int mdpp::fill_continuous_params(mdpp_ctx* ctx, const mdpp_continuous_state* st,
+                                   const mdpp_step_opts* opts, ContinuousParams* p) {
   if (!ctx) return MDPP_EINVAL;
   if (!ctx->have_continuous)
     return fail(ctx, MDPP_EINVAL, "mdpp_set_continuous_config was not called");
@@ -170,7 +176,7 @@ extern "C" int mdpp_continuous_rollout(mdpp_ctx* ctx,
                                        const mdpp_step_opts* opts,
                                        void* cuda_stream) {
   ContinuousParams p;
-  int rc = fill_params(ctx, st, opts, &p);
+  int rc = fill_continuous_params(ctx, st, opts, &p);
   if (rc) return rc;
   if (!io || !io->actions || opts->n_steps < 1)
     return fail(ctx, MDPP_EINVAL, "continuous rollout needs actions and T >= 1");
@@ -204,7 +210,7 @@ extern "C" int mdpp_continuous_reset(mdpp_ctx* ctx,
                                      const mdpp_step_opts* opts,
                                      void* cuda_stream) {
   ContinuousParams p;
-  int rc = fill_params(ctx, st, opts, &p);
+  int rc = fill_continuous_params(ctx, st, opts, &p);
   if (rc) return rc;
   if (!init_states && opts->noise_mode == MDPP_NOISE_REPLAY)
     return fail(ctx, MDPP_EINVAL, "replay reset needs init_states");

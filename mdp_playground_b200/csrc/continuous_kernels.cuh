@@ -445,9 +445,22 @@ __device__ __forceinline__ ContinuousGroupSel select_group(
   return s;
 }
 
-template <typename R, int NOISE, bool GROUPS = false>
-__device__ __forceinline__ void continuous_body(const ContinuousParams& p) {
+// The rollout takes its actions from the action rows (NoContinuousAgent) or
+// from an agent (ArsAgent, ars.cu), which loads its per-env state at launch
+// begin (every thread of the CTA takes part), provides each step's action
+// from the state the env last emitted, sees each step's returned reward,
+// termination and truncation, and stores its state at launch end.  The agent
+// also names the kernel's parameter struct.
+struct NoContinuousAgent {
+  static constexpr bool kActs = false;
+  using Params = ContinuousParams;
+  __device__ __forceinline__ explicit NoContinuousAgent(const ContinuousParams&) {}
+};
+
+template <typename R, int NOISE, bool GROUPS = false, typename AG = NoContinuousAgent>
+__device__ __forceinline__ void continuous_body(const typename AG::Params& p) {
   using O = RealOps<R>;
+  AG ag(p);
   __shared__ GroupSmem<GROUPS> gsm_store;
   ContinuousGroupDev* gsm = group_ptr(gsm_store);
   const int64_t N = MDPP_C_CONST(N_ENVS, p.st.n_envs);
@@ -525,6 +538,7 @@ __device__ __forceinline__ void continuous_body(const ContinuousParams& p) {
 
   double sum_reward = 0, sum_abs_rnoise = 0, sum_abs_pnoise = 0;
   uint32_t n_episodes = 0, n_terminated = 0;
+  if constexpr (AG::kActs) ag.begin(sel, cfg, D);
   if (active) {
 
   // distance of a state's relevant part to the target, in the dtype numpy
@@ -559,7 +573,7 @@ __device__ __forceinline__ void continuous_body(const ContinuousParams& p) {
   R abuf[PF][MDPP_MAX_DIM];
 #pragma unroll
   for (int u = 0; u < PF; ++u)
-    if (u < p.T)
+    if (!AG::kActs && u < p.T)
       load_row<R>(reinterpret_cast<const R*>(p.io.actions) + ((int64_t)u * N + env) * D,
                   D, abuf[u]);
   auto one_step = [&](const int t, R* a_slot) {
@@ -567,13 +581,14 @@ __device__ __forceinline__ void continuous_body(const ContinuousParams& p) {
     const int64_t row = ((int64_t)t * N + env);
     R a[MDPP_MAX_DIM], nxt[MDPP_MAX_DIM];
     bool in_range = true;
+    if constexpr (AG::kActs) ag.act(em, D, amax, row, a_slot);
 #pragma unroll
     for (int d = 0; d < MDPP_MAX_DIM; ++d)
       if (d < D) {
         a[d] = a_slot[d];
         in_range = in_range && a[d] >= -amax && a[d] <= amax;  // Box.contains
       }
-    if (t + PF < p.T)
+    if (!AG::kActs && t + PF < p.T)
       load_row<R>(reinterpret_cast<const R*>(p.io.actions) + (row + (int64_t)PF * N) * D,
                   D, a_slot);
     const double dist_old = dist_prev;
@@ -816,6 +831,7 @@ __device__ __forceinline__ void continuous_body(const ContinuousParams& p) {
     }
     const bool trunc = HORIZON > 0 && tl >= HORIZON;
     n_terminated += done;
+    if constexpr (AG::kActs) ag.step(out_r, AUTORESET && (done || trunc));
 #pragma unroll
     for (int d = 0; d < MDPP_MAX_DIM; ++d)
       if (d < D) em[d] = nxt[d];
@@ -873,6 +889,7 @@ __device__ __forceinline__ void continuous_body(const ContinuousParams& p) {
   p.st.t_episode[env] = tl;
   p.st.episode[env] = ep;
   p.st.reached[env] = (uint8_t)reached;
+  if constexpr (AG::kActs) ag.end(env);
   }  // active
   if (p.st.stats) {  // block-reduced: one atomic per CTA and counter (the
     // counters are single addresses; at T = 1 a per-warp atomic was the
@@ -957,10 +974,10 @@ __device__ __forceinline__ void continuous_reset_body(const ContinuousParams& p)
   p.st.reached[env] = 0;
 }
 
-template <typename R, int NOISE, bool GROUPS = false>
+template <typename R, int NOISE, bool GROUPS = false, typename AG = NoContinuousAgent>
 __global__ void __launch_bounds__(kCBlock)
-continuous_rollout_kernel(const __grid_constant__ ContinuousParams p) {
-  continuous_body<R, NOISE, GROUPS>(p);
+continuous_rollout_kernel(const __grid_constant__ typename AG::Params p) {
+  continuous_body<R, NOISE, GROUPS, AG>(p);
 }
 
 template <typename R, bool GROUPS = false>

@@ -39,6 +39,9 @@ struct mdpp_ctx {
   bool have_continuous = false;
   mdpp_continuous_config c_cfg;
   GroupSet c_set;
+  // (env_begin, env_count, global_id_base) of each group of c_set: the host
+  // side of the ARS update (ars.cu); empty for a single configuration
+  std::vector<int64_t> c_group_ranges;
   bool have_grid = false;
   mdpp_grid_config g_cfg;
   GroupSet g_set;  // GridGroupDev
@@ -85,6 +88,11 @@ int cuda_fail(mdpp_ctx* ctx, cudaError_t e, const char* what);
 // qlearn.cu: the checks of mdpp_qlearn_params that every learner shares (NULL
 // arrays, a table smaller than n_states x n_actions, alpha / gamma / epsilon
 // outside [0, 1]), then its device view
+// continuous.cu: the checks and launch parameters every continuous step
+// launch shares (state arrays, configuration, options, group binding)
+struct ContinuousParams;
+int fill_continuous_params(mdpp_ctx* ctx, const mdpp_continuous_state* st,
+                           const mdpp_step_opts* opts, ContinuousParams* p);
 int check_qlearn_params(mdpp_ctx* ctx, const mdpp_qlearn_params* qp, int64_t n_states,
                         int64_t n_actions, QlearnDev* d);
 

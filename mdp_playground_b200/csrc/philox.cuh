@@ -44,6 +44,11 @@ enum PhiloxStream : uint32_t {
   // dimension, 16 = continuous reward, 17 = grid reward): + 64 j + c
   STREAM_GRID_ZIG = 44,
   STREAM_ZIG_DRAW_RETRY = 0x1000,
+  // ARS perturbations (ars.cu), counter = (global id of the pair's + member,
+  // iteration lo, iteration hi): word c of delta is STREAM_ARS_DELTA + c, c <
+  // 68.  No other stream range reaches it: 0x1000 + 64 j + c tops out near
+  // 0x1450, and the wrapper tail's 0x10000 + pair stays below 0x16000.
+  STREAM_ARS_DELTA = 0x20000,
 };
 
 struct U4 { uint32_t x, y, z, w; };

@@ -48,7 +48,34 @@ def _unit(name, x):
     return x
 
 
-class TabularQLearner:
+class EpisodeReturns:
+    """The per-env return bookkeeping every in-kernel learner keeps
+    (TabularQLearner, GridQLearner, ars.LinearARS): ep_return (the running
+    episode's), ret_sum / ret_count (the episodes that ended in an
+    auto-reset), all [N] on the device next to self.env."""
+
+    def episode_returns(self, clear=False):
+        """Per config group: "episodes" completed by an auto-reset since the
+        last clear, and their mean return "episode_reward_mean" (NaN when
+        none completed).  clear=True starts the next count (the running
+        episodes carry on)."""
+        env, dev = self.env, self.ret_sum.device
+        group = torch.repeat_interleave(
+            torch.arange(env.n_groups, device=dev),
+            torch.tensor(env._group_sizes, device=dev))
+        per_group = torch.zeros((2, env.n_groups), dtype=torch.float64, device=dev)
+        per_group[0].index_add_(0, group, self.ret_count.to(torch.float64))
+        per_group[1].index_add_(0, group, self.ret_sum)
+        ep, tot = per_group.cpu().numpy()
+        with np.errstate(invalid="ignore", divide="ignore"):
+            mean = np.where(ep > 0, tot / np.maximum(ep, 1), np.nan)
+        if clear:
+            self.ret_sum.zero_()
+            self.ret_count.zero_()
+        return {"episodes": ep, "episode_reward_mean": mean}
+
+
+class TabularQLearner(EpisodeReturns):
     """Per-env tabular Q-learning on a discrete env (Philox noise, no
     irrelevant features, no image observations).  Grid envs train with
     GridQLearner.
@@ -133,26 +160,6 @@ class TabularQLearner:
         if record:
             out["actions"] = self._actions_out(out["actions"])
         return out if record else None
-
-    def episode_returns(self, clear=False):
-        """Per config group: "episodes" completed by an auto-reset since the
-        last clear, and their mean return "episode_reward_mean" (NaN when
-        none completed).  clear=True starts the next count (the running
-        episodes carry on)."""
-        env, dev = self.env, self.q.device
-        group = torch.repeat_interleave(
-            torch.arange(env.n_groups, device=dev),
-            torch.tensor(env._group_sizes, device=dev))
-        per_group = torch.zeros((2, env.n_groups), dtype=torch.float64, device=dev)
-        per_group[0].index_add_(0, group, self.ret_count.to(torch.float64))
-        per_group[1].index_add_(0, group, self.ret_sum)
-        ep, tot = per_group.cpu().numpy()
-        with np.errstate(invalid="ignore", divide="ignore"):
-            mean = np.where(ep > 0, tot / np.maximum(ep, 1), np.nan)
-        if clear:
-            self.ret_sum.zero_()
-            self.ret_count.zero_()
-        return {"episodes": ep, "episode_reward_mean": mean}
 
 
 class GridQLearner(TabularQLearner):

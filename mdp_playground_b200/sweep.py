@@ -16,9 +16,10 @@ bounds).  Only cells that cannot share one launch (different state dimension
 / dtype, image size) get one batched env per cell instead.  `run` steps a
 uniform random policy (or one supplied by the caller); `train` (discrete
 experiments) and `train_grid` (grid-world experiments) train a tabular
-Q-learning agent per env inside the step kernel (qlearning.py) and write a
-learning curve per cell, one CSV row per (training iteration, cell) like the
-reference's stats files.
+Q-learning agent per env inside the step kernel (qlearning.py), and
+`train_continuous` (continuous experiments) one linear ARS policy per cell
+(ars.py); each writes a learning curve per cell, one CSV row per (training
+iteration, cell) like the reference's stats files.
 """
 import copy
 import importlib.util
@@ -119,6 +120,7 @@ class Sweep:
         if horizon is None:
             horizon = int(self.module.env_config.get("horizon", 100))
         self.envs_per_cell = int(envs_per_cell)
+        self.world = int(shard[1])
         kinds = {str(c.get("state_space_type", "")).lower()
                  for c in self.cell_configs}
         assert len(kinds) == 1, "one state_space_type per experiment file"
@@ -149,6 +151,7 @@ class Sweep:
         self.timesteps = 0
         self._returned = np.zeros(self.n_cells)
         self.agents = None  # one learner per env of self.envs
+        self.algorithm = None  # the learner's name in write_csv once one has trained
         self.train_results = []  # one dict per training iteration
 
     def _try_grouped(self, Env, device, horizon, shard, env_kwargs):
@@ -216,8 +219,10 @@ class Sweep:
                 "Sweep.train: tabular Q-learning runs on discrete grids only "
                 "(grid-world experiments: Sweep.train_grid)")
         from .qlearning import TabularQLearner
-        return self._train(TabularQLearner, iterations, steps_per_iteration,
-                           alpha, gamma, epsilon, chunk)
+        return self._train(
+            lambda e: TabularQLearner(e, alpha=alpha, gamma=gamma, epsilon=epsilon),
+            iterations, steps_per_iteration, chunk,
+            dict(alpha=alpha, gamma=gamma, epsilon=epsilon), "TabularQLearning")
 
     def train_grid(self, iterations, steps_per_iteration, alpha=0.1, gamma=0.99,
                    epsilon=0.1, chunk=256):
@@ -228,14 +233,39 @@ class Sweep:
             raise NotImplementedError(
                 "Sweep.train_grid: runs grid-world experiments only")
         from .qlearning import GridQLearner
-        return self._train(GridQLearner, iterations, steps_per_iteration,
-                           alpha, gamma, epsilon, chunk)
+        return self._train(
+            lambda e: GridQLearner(e, alpha=alpha, gamma=gamma, epsilon=epsilon),
+            iterations, steps_per_iteration, chunk,
+            dict(alpha=alpha, gamma=gamma, epsilon=epsilon), "TabularQLearning")
 
-    def _train(self, learner, iterations, steps_per_iteration, alpha, gamma,
-               epsilon, chunk):
+    def train_continuous(self, iterations, steps_per_iteration, step_size=0.02,
+                         noise_std=0.03, top_directions=None, chunk=256):
+        """train() for continuous experiments: augmented random search
+        (ars.LinearARS), one linear policy per cell whose envs_per_cell envs
+        (an even number) are the perturbation population.  One learner on the
+        grouped env, or one per cell when the cells differ in dimension or
+        dtype.  Each iteration runs `steps_per_iteration` steps per env (the
+        learn chunks), then one ARS update per cell, and appends the same
+        per-cell results as train().  Calling it again continues with the
+        same policies.  Not for sharded sweeps (the update is per rank)."""
+        if self.kind != "continuous":
+            raise NotImplementedError(
+                "Sweep.train_continuous: runs continuous experiments only")
+        if self.world > 1:
+            raise NotImplementedError(
+                "Sweep.train_continuous: a sharded sweep would need a cross-rank "
+                "ARS update")
+        from .ars import LinearARS
+        return self._train(
+            lambda e: LinearARS(e, step_size=step_size, noise_std=noise_std,
+                                top_directions=top_directions),
+            iterations, steps_per_iteration, chunk, {}, "ARS", update=True)
+
+    def _train(self, make, iterations, steps_per_iteration, chunk, learn_kw,
+               algorithm, update=False):
         if self.agents is None:
-            self.agents = [learner(e, alpha=alpha, gamma=gamma, epsilon=epsilon)
-                           for e in self.envs]
+            self.agents = [make(e) for e in self.envs]
+        self.algorithm = algorithm
 
         def per_cell(dicts, key):  # one value per group of each env, in cell order
             return np.concatenate([np.asarray(d[key]).reshape(-1) for d in dicts])
@@ -247,8 +277,11 @@ class Sweep:
             while done < steps_per_iteration:
                 T = min(chunk, steps_per_iteration - done)
                 for ag in self.agents:
-                    ag.learn(T, alpha=alpha, gamma=gamma, epsilon=epsilon)
+                    ag.learn(T, **learn_kw)
                 done += T
+            if update:
+                for ag in self.agents:
+                    ag.update()
             self.timesteps += steps_per_iteration
             after = [e.episode_stats() for e in self.envs]
             ret = [ag.episode_returns(clear=True) for ag in self.agents]
@@ -321,10 +354,11 @@ class Sweep:
     def write_csv(self, path, algorithm=None):
         """The reference's stats-file layout: one row per grid cell, or, once
         `train` has run, one row per (training iteration, cell).  algorithm
-        defaults to "RandomPolicy", or "TabularQLearning" after `train`."""
+        defaults to "RandomPolicy", or after training to the learner's name
+        ("TabularQLearning", or "ARS" after `train_continuous`)."""
         if self.train_results:
             iters = self.train_results
-            algorithm = algorithm or "TabularQLearning"
+            algorithm = algorithm or self.algorithm
         else:
             res = self.results()
             iters = [{"training_iteration": 1, "timesteps_total": res["transitions"],

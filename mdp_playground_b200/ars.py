@@ -46,15 +46,11 @@ class LinearARS(EpisodeReturns):
         from .continuous_env import ContinuousEnv
         if not isinstance(env, ContinuousEnv):
             raise ValueError(f"LinearARS needs a continuous env (got {type(env).__name__})")
-        if env.noise != "philox":
-            raise ValueError(f"LinearARS needs noise='philox' (got {env.noise!r})")
-        if any(s_.image_representations for s_ in env._group_specs):
-            raise ValueError("LinearARS does not support image_representations")
+        super().__init__(env)
         sizes = list(env._group_sizes)
         if any(n % 2 or n < 2 for n in sizes):
             raise ValueError("LinearARS needs an even number (>= 2) of envs per "
                              f"config group (got {sizes})")
-        self.env = env
         self.step_size = _positive("step_size", step_size)
         self.noise_std = _positive("noise_std", noise_std, allow_zero=True)
         pairs = min(sizes) // 2
@@ -68,20 +64,15 @@ class LinearARS(EpisodeReturns):
         self.theta = torch.empty((env.n_groups, D, D + 1), dtype=torch.float64, device=dev)
         self.theta[:] = torch.as_tensor(theta_init, dtype=torch.float64)
         self.fitness = torch.zeros(N, dtype=torch.float64, device=dev)
-        self.ep_return = torch.zeros(N, dtype=torch.float64, device=dev)
-        self.ret_sum = torch.zeros(N, dtype=torch.float64, device=dev)
-        self.ret_count = torch.zeros(N, dtype=torch.int32, device=dev)
         self.iteration = 0
 
     def _params(self, noise_std=None):
         env = self.env
-        ap = _lib.ArsParams()
+        ap = self._new_params(_lib.ArsParams)
         ap.step_size = self.step_size
         ap.noise_std = self.noise_std if noise_std is None else \
             _positive("noise_std", noise_std, allow_zero=True)
         ap.theta, ap.fitness = _ptr(self.theta), _ptr(self.fitness)
-        ap.ep_return, ap.ret_sum = _ptr(self.ep_return), _ptr(self.ret_sum)
-        ap.ret_count = _ptr(self.ret_count)
         ap.top_directions = self.top_directions
         ap.iteration = self.iteration
         ap.seed = env.philox_seed
@@ -97,20 +88,8 @@ class LinearARS(EpisodeReturns):
         constructor's for this call (0: every env acts with theta)."""
         env = self.env
         T = int(n_steps)
-        ap = self._params(noise_std)
-        out = {}
-        if record:
-            out = env._alloc_out(T, env._obs_torch_dtype(), final_obs=False)
-            out["actions"] = torch.empty((T, env.num_envs, self.D), dtype=env._real,
-                                         device=env.device)
-            ap.actions_taken = _ptr(out["actions"])
-        io = env._io(None, out)
-        opts = env._opts(T, noise_mode=_lib.MDPP_NOISE_PHILOX)
-        env._check(env._lib.mdpp_continuous_ars(
-            env._ctx, C.byref(env._state), C.byref(io), C.byref(ap),
-            C.byref(opts), env._stream()))
-        env._step_index += T
-        return out if record else None
+        return self._learn(env._lib.mdpp_continuous_ars, self._params(noise_std), T, record,
+                           (self.D,), env._real)
 
     def update(self):
         """One ARS step per config group from the fitness since the last

@@ -18,7 +18,7 @@ SOURCES = ["context.cu", "discrete.cu", "discrete_off.cu", "discrete_replay.cu",
            "jit.cu", "qlearn.cu", "ars.cu"]
 HEADERS = ["internal.h", "device_types.h", "philox.cuh", "discrete_kernels.cuh",
            "continuous_kernels.cuh", "ziggurat.cuh", "ziggurat_tables.h",
-           "discrete_launch.h", "../../include/mdpp_b200.h"]
+           "discrete_launch.h", "tabular_q.cuh", "../../include/mdpp_b200.h"]
 # device-side sources embedded into the library for the NVRTC specialisation
 EMBEDDED = ["discrete_kernels.cuh", "continuous_kernels.cuh", "device_types.h",
             "philox.cuh", "ziggurat.cuh",

@@ -29,9 +29,7 @@ constexpr int kArsMaxP = MDPP_MAX_DIM * (MDPP_MAX_DIM + 1);  // 272
 struct ArsDev {
   const double* theta;  // [G][P]
   double* fitness;
-  double* ep_return;
-  double* ret_sum;
-  int32_t* ret_count;
+  ReturnsDev ret;
   void* actions_taken;  // real [T][N][D] or NULL
   double noise_std;
   uint64_t iteration;
@@ -73,7 +71,7 @@ struct ArsAgent {
     if (!sel.active) return;
     env = sel.env;
     fit = p.a.fitness[env];
-    ep_ret = p.a.ep_return[env];
+    ep_ret = p.a.ret.ep_return[env];
     const uint32_t gid_plus = sel.gid - (uint32_t)(sel.local & 1);
     const double snu = (sel.local & 1) ? -p.a.noise_std : p.a.noise_std;
 #pragma unroll 1
@@ -110,20 +108,22 @@ struct ArsAgent {
     }
   }
 
+  // (the episode returns as TabularQ keeps them, written out here: through a
+  // shared inline helper the double kernels, which spill, compile differently)
   __device__ __forceinline__ void step(R out_r, bool reset) {
     const double r = (double)out_r;
     fit = __dadd_rn(fit, r);
     ep_ret = __dadd_rn(ep_ret, r);
     if (reset) {
-      p.a.ret_sum[env] = __dadd_rn(p.a.ret_sum[env], ep_ret);
-      p.a.ret_count[env] += 1;
+      p.a.ret.ret_sum[env] = __dadd_rn(p.a.ret.ret_sum[env], ep_ret);
+      p.a.ret.ret_count[env] += 1;
       ep_ret = 0.0;
     }
   }
 
   __device__ __forceinline__ void end(int64_t) {
     p.a.fitness[env] = fit;
-    p.a.ep_return[env] = ep_ret;
+    p.a.ret.ep_return[env] = ep_ret;
   }
 };
 
@@ -304,7 +304,7 @@ extern "C" int mdpp_continuous_ars(mdpp_ctx* ctx, const mdpp_continuous_state* s
   if (((uintptr_t)io->obs | (uintptr_t)io->final_obs) & 15)
     return fail(ctx, MDPP_EINVAL, "obs / final_obs must be 16-byte aligned");
   k.io = *io;
-  k.a = ArsDev{ap->theta, ap->fitness, ap->ep_return, ap->ret_sum, ap->ret_count,
+  k.a = ArsDev{ap->theta, ap->fitness, ReturnsDev{ap->ep_return, ap->ret_sum, ap->ret_count},
                ap->actions_taken, ap->noise_std, ap->iteration};
   MDPP_CUDA(ctx, cudaSetDevice(ctx->device));
   cudaStream_t s = (cudaStream_t)cuda_stream;

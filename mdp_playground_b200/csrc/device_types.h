@@ -87,15 +87,21 @@ struct StepOut {
   bool done, trunc;
 };
 
+// The per-env episode returns every learner keeps: the running episode's,
+// and the sum / count of the returns of those that ended in an auto-reset.
+struct ReturnsDev {
+  double* ep_return;
+  double* ret_sum;
+  int32_t* ret_count;
+};
+
 // Device view of mdpp_qlearn_params (qlearn.cu check_qlearn_params).
 struct QlearnDev {
   double* q;
   int32_t q_states, q_actions;
   double alpha, gamma;
   uint64_t explore_below;  // explore iff the exploring word < ceil(epsilon * 2^32)
-  double* ep_return;
-  double* ret_sum;
-  int32_t* ret_count;
+  ReturnsDev ret;
   int32_t* actions_taken;
 };
 

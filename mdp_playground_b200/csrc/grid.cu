@@ -19,6 +19,7 @@
 #include <vector>
 
 #include "internal.h"
+#include "tabular_q.cuh"
 #include "philox.cuh"
 #include "ziggurat.cuh"
 
@@ -501,54 +502,33 @@ grid_reset_kernel(const __grid_constant__ GridParams p) {
 //   w = philox(g, step >> 1, STREAM_GRID_ACTION), (x, y) / (z, w) = even / odd step
 //   a = first word < ceil(epsilon * 2^32) ? umulhi(second word, A) : argmax Q[s]
 //   step -> r, nxt (before any auto-reset), terminated
-//   target = terminated ? r : r + gamma * max_a' Q[nxt][a']
-//   Q[s][a] = q + alpha * (target - q)
-// in float64 with every operation rounded on its own, like QAgent (qlearn.cu).
+// then the update of TabularQ (tabular_q.cuh), like QAgent (qlearn.cu).
 // Action index a: 0 = no-op, 1 + 2k = -1 on dim k, 2 + 2k = +1 on dim k.
-// Q is float64 [N][q_states][q_actions], env-major; the host passes q_actions
-// = 8 for 2-D grids, so a row is one 64-byte line.
+// The host passes q_actions = 8 for 2-D grids, so a row is one 64-byte line.
 struct GridQlearnParams : GridParams {
   QlearnDev q;
 };
 
+__device__ __forceinline__ bool autoreset_of(const GridParams& p) { return p.autoreset != 0; }
+
 template <int ND>
-struct GridQAgent {
+struct GridQAgent : TabularQ<2 * ND + 1> {
+  using Q = TabularQ<2 * ND + 1>;
+  using Q::d; using Q::greedy; using Q::a;
   static constexpr bool kActs = true;
   // 65 536 envs are 512 CTAs of 128, 4 per SM on 148 SMs: at most 128
   // registers a thread keep them resident (one wave)
   static constexpr int kMinBlocks = 4;
   using Params = GridQlearnParams;
   static constexpr int A = 2 * ND + 1;
-  const QlearnDev& d;
-  double* tab;      // this env's Q-table
-  int32_t greedy;   // argmax of the current cell's row
-  int32_t s, a;     // the step's cell index and action
-  double ep_ret;    // return of the running episode
   uint64_t cached;  // step >> 1 of w
   U4 w;
 
-  __device__ __forceinline__ explicit GridQAgent(const GridQlearnParams& p) : d(p.q) {}
-
-  // (max, lowest argmax) of row st; numpy.argmax order
-  __device__ __forceinline__ int32_t row_argmax(int32_t st, double& m) const {
-    const double* row = tab + (int64_t)st * d.q_actions;
-    m = row[0];
-    int32_t am = 0;
-#pragma unroll
-    for (int k = 1; k < A; ++k) {
-      const double x = row[k];
-      if (x > m) { m = x; am = k; }
-    }
-    return am;
-  }
+  __device__ __forceinline__ explicit GridQAgent(const GridQlearnParams& p) : Q(p.q) {}
 
   __device__ __forceinline__ void begin(const mdpp_grid_config& c, int64_t env,
                                         const int32_t* pos) {
-    tab = d.q + env * (int64_t)d.q_states * d.q_actions;
-    s = cell_index<ND>(c, pos);
-    double m;
-    greedy = row_argmax(s, m);
-    ep_ret = d.ep_return[env];
+    Q::begin(env, [&] { return cell_index<ND>(c, pos); }, A);
     cached = ~0ull;
   }
 
@@ -571,38 +551,9 @@ struct GridQAgent {
   __device__ __forceinline__ void update(const GridParams& p, const mdpp_grid_config& c,
                                          const StepOut& o, const int32_t* pos_after,
                                          int64_t env, int64_t off) {
-    double* q_at = tab + (int64_t)s * d.q_actions + a;
-    const double q = *q_at;  // (loaded beside the row of nxt)
-    double m;
-    const int32_t am = row_argmax(o.nxt, m);
-    const double target = o.done ? o.r : __dadd_rn(o.r, __dmul_rn(d.gamma, m));
-    const double qn = __dadd_rn(q, __dmul_rn(d.alpha, __dsub_rn(target, q)));
-    *q_at = qn;
-    const bool reset = p.autoreset && (o.done || o.trunc);
-    if (reset) {
-      const int32_t s_after = cell_index<ND>(c, pos_after);
-      greedy = row_argmax(s_after, m);
-      s = s_after;
-    } else {
-      if (o.nxt != s) {
-        greedy = am;
-      } else if (a != am) {  // the row just loaded changed in entry a only
-        greedy = (qn > m || (qn == m && a < am)) ? a : am;
-      } else {  // the maximum itself changed: rescan unless it only grew
-        greedy = qn >= m ? am : row_argmax(s, m);
-      }
-      s = o.nxt;
-    }
-    ep_ret = __dadd_rn(ep_ret, o.r);
-    if (reset) {
-      d.ret_sum[env] = __dadd_rn(d.ret_sum[env], ep_ret);
-      d.ret_count[env] += 1;
-      ep_ret = 0.0;
-    }
+    Q::update(p, o, A, env, [&] { return cell_index<ND>(c, pos_after); });
     if (d.actions_taken) __stcs(d.actions_taken + off, a);
   }
-
-  __device__ __forceinline__ void end(int64_t env) { d.ep_return[env] = ep_ret; }
 };
 
 
@@ -711,28 +662,39 @@ static int fill_grid(mdpp_ctx* ctx, const mdpp_grid_state* st,
   return MDPP_OK;
 }
 
+// CTAs of a grid launch: the group set's, or one per kGBlock envs
+static unsigned grid_ctas(const mdpp_ctx* ctx, const GridParams& p) {
+  return p.groups ? (unsigned)ctx->g_set.n_ctas
+                  : (unsigned)((p.st.n_envs + kGBlock - 1) / kGBlock);
+}
+
+// The Philox-noise rollout with agent AG acting, one kernel per generator of
+// the reward normals (p.normal_mode)
+template <int ND, bool FAST, bool GROUPS, typename AG>
+static int launch_grid_philox(mdpp_ctx* ctx, const typename AG::Params& p, cudaStream_t s) {
+  const unsigned grid = grid_ctas(ctx, p);
+  if (p.normal_mode == MDPP_NORMAL_ZIGGURAT)
+    grid_rollout_kernel<ND, MDPP_NOISE_PHILOX, FAST, GROUPS, MDPP_NORMAL_ZIGGURAT, AG>
+        <<<grid, kGBlock, 0, s>>>(p);
+  else if (p.normal_mode == MDPP_NORMAL_FAST)
+    grid_rollout_kernel<ND, MDPP_NOISE_PHILOX, FAST, GROUPS, MDPP_NORMAL_FAST, AG>
+        <<<grid, kGBlock, 0, s>>>(p);
+  else
+    grid_rollout_kernel<ND, MDPP_NOISE_PHILOX, FAST, GROUPS, MDPP_NORMAL_F64, AG>
+        <<<grid, kGBlock, 0, s>>>(p);
+  MDPP_CUDA(ctx, cudaGetLastError());
+  return MDPP_OK;
+}
+
 template <int ND, bool FAST, bool GROUPS>
 static int launch_grid(mdpp_ctx* ctx, const GridParams& p, cudaStream_t s) {
-  const unsigned grid = GROUPS ? (unsigned)ctx->g_set.n_ctas
-                               : (unsigned)((p.st.n_envs + kGBlock - 1) / kGBlock);
-  switch (p.noise_mode) {
-    case MDPP_NOISE_OFF:
-      grid_rollout_kernel<ND, MDPP_NOISE_OFF, FAST, GROUPS><<<grid, kGBlock, 0, s>>>(p);
-      break;
-    case MDPP_NOISE_REPLAY:
-      grid_rollout_kernel<ND, MDPP_NOISE_REPLAY, FAST, GROUPS><<<grid, kGBlock, 0, s>>>(p);
-      break;
-    default:
-      if (p.normal_mode == MDPP_NORMAL_ZIGGURAT)
-        grid_rollout_kernel<ND, MDPP_NOISE_PHILOX, FAST, GROUPS, MDPP_NORMAL_ZIGGURAT>
-            <<<grid, kGBlock, 0, s>>>(p);
-      else if (p.normal_mode == MDPP_NORMAL_FAST)
-        grid_rollout_kernel<ND, MDPP_NOISE_PHILOX, FAST, GROUPS, MDPP_NORMAL_FAST>
-            <<<grid, kGBlock, 0, s>>>(p);
-      else
-        grid_rollout_kernel<ND, MDPP_NOISE_PHILOX, FAST, GROUPS, MDPP_NORMAL_F64>
-            <<<grid, kGBlock, 0, s>>>(p);
-  }
+  if (p.noise_mode == MDPP_NOISE_PHILOX)
+    return launch_grid_philox<ND, FAST, GROUPS, NoGridAgent>(ctx, p, s);
+  const unsigned grid = grid_ctas(ctx, p);
+  if (p.noise_mode == MDPP_NOISE_OFF)
+    grid_rollout_kernel<ND, MDPP_NOISE_OFF, FAST, GROUPS><<<grid, kGBlock, 0, s>>>(p);
+  else
+    grid_rollout_kernel<ND, MDPP_NOISE_REPLAY, FAST, GROUPS><<<grid, kGBlock, 0, s>>>(p);
   MDPP_CUDA(ctx, cudaGetLastError());
   return MDPP_OK;
 }
@@ -789,28 +751,12 @@ extern "C" int mdpp_grid_reset(mdpp_ctx* ctx, const mdpp_grid_state* st,
   p.init_states = init_states;
   p.reset_obs = obs;
   MDPP_CUDA(ctx, cudaSetDevice(ctx->device));
-  const unsigned grid = p.groups ? (unsigned)ctx->g_set.n_ctas
-                                 : (unsigned)((p.st.n_envs + kGBlock - 1) / kGBlock);
+  const unsigned grid = grid_ctas(ctx, p);
   cudaStream_t s = (cudaStream_t)cuda_stream;
   if (p.groups && ctx->g_cfg.n_dims == 4) grid_reset_kernel<4, true><<<grid, kGBlock, 0, s>>>(p);
   else if (p.groups) grid_reset_kernel<2, true><<<grid, kGBlock, 0, s>>>(p);
   else if (ctx->g_cfg.n_dims == 4) grid_reset_kernel<4><<<grid, kGBlock, 0, s>>>(p);
   else grid_reset_kernel<2><<<grid, kGBlock, 0, s>>>(p);
-  MDPP_CUDA(ctx, cudaGetLastError());
-  return MDPP_OK;
-}
-
-template <int ND, bool GROUPS>
-static int launch_grid_qlearn(mdpp_ctx* ctx, const GridQlearnParams& qp, int normal_mode,
-                              cudaStream_t s) {
-  const unsigned grid = GROUPS ? (unsigned)ctx->g_set.n_ctas
-                               : (unsigned)((qp.st.n_envs + kGBlock - 1) / kGBlock);
-  if (normal_mode == MDPP_NORMAL_ZIGGURAT)
-    grid_rollout_kernel<ND, MDPP_NOISE_PHILOX, false, GROUPS, MDPP_NORMAL_ZIGGURAT, GridQAgent<ND>><<<grid, kGBlock, 0, s>>>(qp);
-  else if (normal_mode == MDPP_NORMAL_FAST)
-    grid_rollout_kernel<ND, MDPP_NOISE_PHILOX, false, GROUPS, MDPP_NORMAL_FAST, GridQAgent<ND>><<<grid, kGBlock, 0, s>>>(qp);
-  else
-    grid_rollout_kernel<ND, MDPP_NOISE_PHILOX, false, GROUPS, MDPP_NORMAL_F64, GridQAgent<ND>><<<grid, kGBlock, 0, s>>>(qp);
   MDPP_CUDA(ctx, cudaGetLastError());
   return MDPP_OK;
 }
@@ -837,10 +783,9 @@ extern "C" int mdpp_grid_qlearn(mdpp_ctx* ctx, const mdpp_grid_state* st,
   k.io = *io;
   MDPP_CUDA(ctx, cudaSetDevice(ctx->device));
   cudaStream_t s = (cudaStream_t)cuda_stream;
-  const int normal = opts->normal_mode;
   if (k.groups)
-    return nd == 4 ? launch_grid_qlearn<4, true>(ctx, k, normal, s)
-                   : launch_grid_qlearn<2, true>(ctx, k, normal, s);
-  return nd == 4 ? launch_grid_qlearn<4, false>(ctx, k, normal, s)
-                 : launch_grid_qlearn<2, false>(ctx, k, normal, s);
+    return nd == 4 ? launch_grid_philox<4, false, true, GridQAgent<4>>(ctx, k, s)
+                   : launch_grid_philox<2, false, true, GridQAgent<2>>(ctx, k, s);
+  return nd == 4 ? launch_grid_philox<4, false, false, GridQAgent<4>>(ctx, k, s)
+                 : launch_grid_philox<2, false, false, GridQAgent<2>>(ctx, k, s);
 }

@@ -9,20 +9,15 @@
 //   explore = (double)w.z < epsilon * 2^32
 //   a = explore ? umulhi(w.x, A) : argmax_a' Q[s][a']  (lowest index on ties)
 //   step -> r, nxt (before any auto-reset), terminated
-//   target = terminated ? r : r + gamma * max_a' Q[nxt][a']
-//   Q[s][a] = q + alpha * (target - q)
-// with every float64 operation rounded on its own (no FMA contraction), so a
-// numpy restatement in the same order gives the same bits.
+// then the update of TabularQ (tabular_q.cuh).
 //
-// Q is float64 [N][q_states][q_actions], env-major: each env walks its own
-// contiguous table (64 rows of 64 B at 8 x 8; 32 MB for 65 536 envs, which
-// stays resident in the 126 MB L2).  One row load per step sits on the
-// dependent chain: Q[nxt] gives both the target's max and, when no
-// auto-reset follows, the next step's greedy action.
+// Each env walks its own contiguous table (64 rows of 64 B at 8 x 8; 32 MB
+// for 65 536 envs, which stays resident in the 126 MB L2).
 #include <algorithm>
 #include <cmath>
 
 #include "discrete_launch.h"
+#include "tabular_q.cuh"
 
 namespace mdpp {
 
@@ -31,38 +26,17 @@ struct QlearnParams {
   QlearnDev q;
 };
 
-struct QAgent {
+// The group's A bounds the row scans (a run-time value: TabularQ<0>).
+struct QAgent : TabularQ<0> {
   static constexpr bool kStepOut = true;
-  const QlearnDev& d;
-  double* tab;       // this env's Q-table
-  int32_t greedy;    // argmax of the current state's row
   uint32_t explore;  // bit j: step j of the chunk explores
-  int32_t s, a;      // the step's state and action
-  double ep_ret;     // return of the running episode
   // (the rest lives in the kernel parameters and the group view: registers
   // are what bounds the chain's occupancy)
 
-  __device__ __forceinline__ explicit QAgent(const QlearnDev& dev) : d(dev) {}
-
-  // (max, lowest argmax) of row st; numpy.argmax order
-  __device__ __forceinline__ int32_t row_argmax(const GroupView& v, int32_t st,
-                                                double& m) const {
-    const double* row = tab + (int64_t)st * d.q_actions;
-    m = row[0];
-    int32_t am = 0;
-#pragma unroll 4
-    for (int k = 1; k < v.A; ++k) {
-      const double x = row[k];
-      if (x > m) { m = x; am = k; }
-    }
-    return am;
-  }
+  __device__ __forceinline__ explicit QAgent(const QlearnDev& dev) : TabularQ(dev) {}
 
   __device__ __forceinline__ void begin(const GroupView& v, int64_t env, int32_t s0) {
-    tab = d.q + env * (int64_t)d.q_states * d.q_actions;
-    double m;
-    greedy = row_argmax(v, s0, m);
-    ep_ret = d.ep_return[env];
+    TabularQ::begin(env, [=] { return s0; }, v.A);
   }
 
   __device__ __forceinline__ void draw(int j, const U4& w) {
@@ -79,33 +53,9 @@ struct QAgent {
   __device__ __forceinline__ void update(const RolloutParams& p, const GroupView& v,
                                          const StepOut& o, int32_t s_after,
                                          int64_t env, int64_t off) {
-    double* q_at = tab + (int64_t)s * d.q_actions + a;
-    const double q = *q_at;  // (loaded beside the row of nxt)
-    double m;
-    const int32_t am = row_argmax(v, o.nxt, m);
-    const double target = o.done ? o.r : __dadd_rn(o.r, __dmul_rn(d.gamma, m));
-    const double qn = __dadd_rn(q, __dmul_rn(d.alpha, __dsub_rn(target, q)));
-    *q_at = qn;
-    const bool reset = autoreset_of(p) && (o.done || o.trunc);
-    if (reset) {
-      greedy = row_argmax(v, s_after, m);
-    } else if (o.nxt != s) {
-      greedy = am;
-    } else if (a != am) {  // the row just loaded changed in entry a only
-      greedy = (qn > m || (qn == m && a < am)) ? a : am;
-    } else {  // the maximum itself changed: rescan unless it only grew
-      greedy = qn >= m ? am : row_argmax(v, s, m);
-    }
-    ep_ret = __dadd_rn(ep_ret, o.r);
-    if (reset) {
-      d.ret_sum[env] = __dadd_rn(d.ret_sum[env], ep_ret);
-      d.ret_count[env] += 1;
-      ep_ret = 0.0;
-    }
+    TabularQ::update(p, o, v.A, env, [=] { return s_after; });
     if (d.actions_taken) st_stream(d.actions_taken + off, a);
   }
-
-  __device__ __forceinline__ void end(int64_t env) { d.ep_return[env] = ep_ret; }
 };
 
 // 65 536 envs are 1024 CTAs of 64, 7 per SM: 144 registers a thread keep 7
@@ -147,9 +97,7 @@ int check_qlearn_params(mdpp_ctx* ctx, const mdpp_qlearn_params* qp, int64_t n_s
   d->gamma = qp->gamma;
   // w < x for an integer w <=> w < ceil(x); x = epsilon * 2^32 is exact
   d->explore_below = (uint64_t)std::ceil(qp->epsilon * 4294967296.0);
-  d->ep_return = qp->ep_return;
-  d->ret_sum = qp->ret_sum;
-  d->ret_count = qp->ret_count;
+  d->ret = ReturnsDev{qp->ep_return, qp->ret_sum, qp->ret_count};
   d->actions_taken = qp->actions_taken;
   return MDPP_OK;
 }

@@ -49,10 +49,49 @@ def _unit(name, x):
 
 
 class EpisodeReturns:
-    """The per-env return bookkeeping every in-kernel learner keeps
-    (TabularQLearner, GridQLearner, ars.LinearARS): ep_return (the running
-    episode's), ret_sum / ret_count (the episodes that ended in an
-    auto-reset), all [N] on the device next to self.env."""
+    """The base of the learners that run inside a rollout kernel
+    (TabularQLearner, GridQLearner, ars.LinearARS): the checks they share,
+    the per-env return bookkeeping (ep_return, the running episode's;
+    ret_sum / ret_count, the episodes that ended in an auto-reset; all [N]
+    on the device next to self.env) and the launch of a learn call."""
+
+    def __init__(self, env):
+        if env.noise != "philox":
+            raise ValueError(f"{type(self).__name__} needs noise='philox' "
+                             f"(got {env.noise!r})")
+        if any(s_.image_representations for s_ in env._group_specs):
+            raise ValueError(f"{type(self).__name__} does not support "
+                             "image_representations")
+        self.env = env
+        N, dev = env.num_envs, env.device
+        self.ep_return = torch.zeros(N, dtype=torch.float64, device=dev)
+        self.ret_sum = torch.zeros(N, dtype=torch.float64, device=dev)
+        self.ret_count = torch.zeros(N, dtype=torch.int32, device=dev)
+
+    def _new_params(self, struct):
+        """A new parameter struct (_lib.QlearnParams / ArsParams) pointing
+        at the return counters."""
+        p = struct()
+        p.ep_return, p.ret_sum = _ptr(self.ep_return), _ptr(self.ret_sum)
+        p.ret_count = _ptr(self.ret_count)
+        return p
+
+    def _learn(self, entry, params, T, record, action_shape, action_dtype):
+        """One launch of the learner's entry point over T steps; with record,
+        the outputs and the actions taken ([T, N, *action_shape])."""
+        env = self.env
+        out = {}
+        if record:
+            out = env._alloc_out(T, env._obs_torch_dtype(), final_obs=False)
+            out["actions"] = torch.empty((T, env.num_envs) + action_shape,
+                                         dtype=action_dtype, device=env.device)
+            params.actions_taken = _ptr(out["actions"])
+        io = env._io(None, out)
+        opts = env._opts(T, noise_mode=_lib.MDPP_NOISE_PHILOX)
+        env._check(entry(env._ctx, C.byref(env._state), C.byref(io), C.byref(params),
+                         C.byref(opts), env._stream()))
+        env._step_index += T
+        return out if record else None
 
     def episode_returns(self, clear=False):
         """Per config group: "episodes" completed by an auto-reset since the
@@ -85,24 +124,13 @@ class TabularQLearner(EpisodeReturns):
 
     def __init__(self, env, alpha=0.1, gamma=0.99, epsilon=0.1, q_init=0.0):
         self._check_env(env)
-        if env.noise != "philox":
-            raise ValueError(f"{type(self).__name__} needs noise='philox' "
-                             f"(got {env.noise!r})")
-        if any(s_.image_representations for s_ in env._group_specs):
-            raise ValueError(f"{type(self).__name__} does not support "
-                             "image_representations")
-        self.env = env
+        super().__init__(env)
         self.alpha = _unit("alpha", alpha)
         self.gamma = _unit("gamma", gamma)
         self.epsilon = _unit("epsilon", epsilon)
-        N, dev = env.num_envs, env.device
         S, A = self._table_shape()
-        self.q = torch.full((N, S, A), float(q_init), dtype=torch.float64, device=dev)
-        # return of each env's running episode, and sum / count of the returns
-        # of the episodes that ended in an auto-reset
-        self.ep_return = torch.zeros(N, dtype=torch.float64, device=dev)
-        self.ret_sum = torch.zeros(N, dtype=torch.float64, device=dev)
-        self.ret_count = torch.zeros(N, dtype=torch.int32, device=dev)
+        self.q = torch.full((env.num_envs, S, A), float(q_init), dtype=torch.float64,
+                            device=env.device)
 
     # -- what differs between the env kinds -----------------------------------
     def _check_env(self, env):
@@ -117,8 +145,8 @@ class TabularQLearner(EpisodeReturns):
         tables = self.env.group_tables
         return max(t.n_states for t in tables), max(t.n_actions for t in tables)
 
-    def _launch(self, *args):
-        return self.env._lib.mdpp_discrete_qlearn(*args)
+    def _entry(self):
+        return self.env._lib.mdpp_discrete_qlearn
 
     def _before_launch(self):
         pass
@@ -134,32 +162,18 @@ class TabularQLearner(EpisodeReturns):
         action rows, which env.rollout(actions=...) accepts).  alpha / gamma
         / epsilon override the constructor's values for this call (e.g.
         epsilon=0, alpha=0 for a greedy evaluation that leaves q unchanged)."""
-        env = self.env
         T = int(n_steps)
         self._before_launch()
-        qp = _lib.QlearnParams()
+        qp = self._new_params(_lib.QlearnParams)
         qp.alpha = self.alpha if alpha is None else _unit("alpha", alpha)
         qp.gamma = self.gamma if gamma is None else _unit("gamma", gamma)
         qp.epsilon = self.epsilon if epsilon is None else _unit("epsilon", epsilon)
         qp.q = _ptr(self.q)
         qp.q_states, qp.q_actions = self.q.shape[1], self.q.shape[2]
-        qp.ep_return, qp.ret_sum = _ptr(self.ep_return), _ptr(self.ret_sum)
-        qp.ret_count = _ptr(self.ret_count)
-        out = {}
-        if record:
-            out = env._alloc_out(T, env._obs_torch_dtype(), final_obs=False)
-            out["actions"] = torch.empty((T, env.num_envs), dtype=torch.int32,
-                                         device=env.device)
-            qp.actions_taken = _ptr(out["actions"])
-        io = env._io(None, out)
-        opts = env._opts(T)
-        env._check(self._launch(
-            env._ctx, C.byref(env._state), C.byref(io), C.byref(qp),
-            C.byref(opts), env._stream()))
-        env._step_index += T
+        out = self._learn(self._entry(), qp, T, record, (), torch.int32)
         if record:
             out["actions"] = self._actions_out(out["actions"])
-        return out if record else None
+        return out
 
 
 class GridQLearner(TabularQLearner):
@@ -191,8 +205,8 @@ class GridQLearner(TabularQLearner):
         return (max(grid_cells(s_.grid_shape) for s_ in env._group_specs),
                 8 if env._nd == 2 else 9)
 
-    def _launch(self, *args):
-        return self.env._lib.mdpp_grid_qlearn(*args)
+    def _entry(self):
+        return self.env._lib.mdpp_grid_qlearn
 
     def _before_launch(self):
         pos = self.env._pos

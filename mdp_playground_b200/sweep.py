@@ -214,29 +214,30 @@ class Sweep:
         the episode counters' change over the iteration).  Discrete grids
         only (grid-world experiments: train_grid).  Calling train again
         continues with the same Q-tables."""
-        if self.kind != "discrete":
-            raise NotImplementedError(
-                "Sweep.train: tabular Q-learning runs on discrete grids only "
-                "(grid-world experiments: Sweep.train_grid)")
-        from .qlearning import TabularQLearner
-        return self._train(
-            lambda e: TabularQLearner(e, alpha=alpha, gamma=gamma, epsilon=epsilon),
-            iterations, steps_per_iteration, chunk,
-            dict(alpha=alpha, gamma=gamma, epsilon=epsilon), "TabularQLearning")
+        return self._train_q(
+            "discrete", "Sweep.train: tabular Q-learning runs on discrete grids only "
+            "(grid-world experiments: Sweep.train_grid)",
+            iterations, steps_per_iteration, alpha, gamma, epsilon, chunk)
 
     def train_grid(self, iterations, steps_per_iteration, alpha=0.1, gamma=0.99,
                    epsilon=0.1, chunk=256):
         """train() for grid-world experiments (GridQLearner): one learner on
         the grouped env, or one per cell when the cells differ in
         irrelevant_features; results in cell order either way."""
-        if self.kind != "grid":
-            raise NotImplementedError(
-                "Sweep.train_grid: runs grid-world experiments only")
-        from .qlearning import GridQLearner
-        return self._train(
-            lambda e: GridQLearner(e, alpha=alpha, gamma=gamma, epsilon=epsilon),
-            iterations, steps_per_iteration, chunk,
-            dict(alpha=alpha, gamma=gamma, epsilon=epsilon), "TabularQLearning")
+        return self._train_q("grid", "Sweep.train_grid: runs grid-world experiments only",
+                             iterations, steps_per_iteration, alpha, gamma, epsilon, chunk)
+
+    def _train_q(self, kind, refusal, iterations, steps_per_iteration, alpha, gamma,
+                 epsilon, chunk):
+        """train / train_grid: `refusal` is the NotImplementedError message
+        for experiments of another kind than `kind`."""
+        if self.kind != kind:
+            raise NotImplementedError(refusal)
+        from .qlearning import GridQLearner, TabularQLearner
+        learner = GridQLearner if kind == "grid" else TabularQLearner
+        kw = dict(alpha=alpha, gamma=gamma, epsilon=epsilon)
+        return self._train(lambda e: learner(e, **kw), iterations, steps_per_iteration,
+                           chunk, kw, "TabularQLearning")
 
     def train_continuous(self, iterations, steps_per_iteration, step_size=0.02,
                          noise_std=0.03, top_directions=None, chunk=256):

@@ -570,6 +570,47 @@ int mdpp_grid_qlearn(mdpp_ctx* ctx, const mdpp_grid_state* st,
 #endif
 
 /* ------------------------------------------------------------------------
+ * Evaluation of the learners' current policies: E episodes per env on an
+ * evaluation env, with nothing learned and no exploration.
+ *   mdpp_discrete_qeval / mdpp_grid_qeval: a = argmax_a' q[i][s][a'] (ties:
+ *     lowest index), with s and the table layout of mdpp_discrete_qlearn /
+ *     mdpp_grid_qlearn; q is only read.
+ *   mdpp_continuous_ars_eval: a = theta_g [obs; 1] with the product and sum
+ *     order, cast and clipping of mdpp_continuous_ars (noise_std = 0).
+ * The env steps exactly as the rollout with those actions.  The caller
+ * resets the env first, so every env starts a fresh episode; an episode
+ * ends on terminated or truncated.  Of each env, the first `episodes`
+ * episodes are counted: ret_sum[i] = the sum of their returns (fp64,
+ * sequential), ret_count[i] = how many completed (= episodes when
+ * n_steps >= episodes * horizon), len_sum[i] = the sum of their lengths; the
+ * steps after them are stepped and discarded.  Needs Philox noise,
+ * autoreset, horizon >= 1, episodes >= 1, n_steps >= episodes * horizon and
+ * io->actions == NULL (the other outputs of io may be NULL: skipped).
+ * mdpp_discrete_qeval: no irrelevant features.                              */
+typedef struct mdpp_eval_params {
+  const double* q;                /* qeval: [N][q_states][q_actions]         */
+  int32_t q_states, q_actions;    /* >= every group's S / A                  */
+  const double* theta;            /* ars_eval: [G][D][D+1] float64           */
+  int32_t episodes;               /* E >= 1 counted episodes per env         */
+  int32_t reserved0;
+  double* ret_sum;                /* [N] return sum of the first E episodes  */
+  int32_t* ret_count;             /* [N] episodes counted (<= E)             */
+  int64_t* len_sum;               /* [N] length sum of the counted episodes  */
+} mdpp_eval_params;
+
+#ifndef __CUDACC_RTC__ /* NVRTC sees the types only */
+int mdpp_discrete_qeval(mdpp_ctx* ctx, const mdpp_discrete_state* st,
+                        const mdpp_discrete_io* io, const mdpp_eval_params* ep,
+                        const mdpp_step_opts* opts, void* cuda_stream);
+int mdpp_grid_qeval(mdpp_ctx* ctx, const mdpp_grid_state* st, const mdpp_grid_io* io,
+                    const mdpp_eval_params* ep, const mdpp_step_opts* opts,
+                    void* cuda_stream);
+int mdpp_continuous_ars_eval(mdpp_ctx* ctx, const mdpp_continuous_state* st,
+                             const mdpp_continuous_io* io, const mdpp_eval_params* ep,
+                             const mdpp_step_opts* opts, void* cuda_stream);
+#endif
+
+/* ------------------------------------------------------------------------
  * Image observations (replaces ImageMultiDiscrete.generate_image,
  * spaces/image_multi_discrete.py:129-270, and ImageContinuous.generate_image
  * / get_image_representation, spaces/image_continuous.py:116-277).

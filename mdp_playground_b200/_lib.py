@@ -39,6 +39,7 @@ EXPORTED_SYMBOLS = (
     "mdpp_discrete_qlearn", "mdpp_grid_qlearn",
     "mdpp_continuous_ars", "mdpp_continuous_ars_update",
     "mdpp_continuous_ars_perturbations",
+    "mdpp_discrete_qeval", "mdpp_grid_qeval", "mdpp_continuous_ars_eval",
 )
 MDPP_MAX_DIM, MDPP_MAX_ORDER, MDPP_MAX_TERM_BOXES = 16, 4, 8
 
@@ -122,6 +123,14 @@ class ArsParams(C.Structure):
         ("iteration", C.c_uint64), ("seed", C.c_uint64),
         ("env_id_offset", C.c_int64), ("delta_out", C.c_void_p),
         ("group_stats", C.c_void_p),
+    ]
+
+
+class EvalParams(C.Structure):
+    _fields_ = [
+        ("q", C.c_void_p), ("q_states", C.c_int32), ("q_actions", C.c_int32),
+        ("theta", C.c_void_p), ("episodes", C.c_int32), ("reserved0", C.c_int32),
+        ("ret_sum", C.c_void_p), ("ret_count", C.c_void_p), ("len_sum", C.c_void_p),
     ]
 
 
@@ -323,6 +332,15 @@ def load():
         C.POINTER(StepOpts), P]
     lib.mdpp_continuous_ars.argtypes = [
         P, C.POINTER(ContinuousState), C.POINTER(ContinuousIO), C.POINTER(ArsParams),
+        C.POINTER(StepOpts), P]
+    lib.mdpp_continuous_ars_eval.argtypes = [
+        P, C.POINTER(ContinuousState), C.POINTER(ContinuousIO), C.POINTER(EvalParams),
+        C.POINTER(StepOpts), P]
+    lib.mdpp_discrete_qeval.argtypes = [
+        P, C.POINTER(DiscreteState), C.POINTER(DiscreteIO), C.POINTER(EvalParams),
+        C.POINTER(StepOpts), P]
+    lib.mdpp_grid_qeval.argtypes = [
+        P, C.POINTER(GridState), C.POINTER(GridIO), C.POINTER(EvalParams),
         C.POINTER(StepOpts), P]
     lib.mdpp_continuous_ars_update.argtypes = [P, C.c_int64, C.POINTER(ArsParams), P]
     lib.mdpp_continuous_ars_perturbations.argtypes = [

@@ -91,6 +91,24 @@ class LinearARS(EpisodeReturns):
         return self._learn(env._lib.mdpp_continuous_ars, self._params(noise_std), T, record,
                            (self.D,), env._real)
 
+    def _check_eval_layout(self, eval_env):
+        if eval_env.spec.state_space_dim != self.D or eval_env._real != self.env._real:
+            raise ValueError(f"LinearARS.evaluate: eval_env has D = "
+                             f"{eval_env.spec.state_space_dim} in {eval_env._real}, the "
+                             f"learner's env D = {self.D} in {self.env._real}")
+
+    def evaluate(self, eval_env, episodes=10, per_env=False):
+        """theta itself (no perturbation) on eval_env, an env built like the
+        learner's (typically without its noises): eval_env.reset(), then one
+        launch of episodes * eval_env.horizon steps in which the first
+        `episodes` episodes of every env are counted.  Leaves theta,
+        fitness, iteration, the training env and episode_returns untouched.
+        Returns what TabularQLearner.evaluate returns."""
+        ep = _lib.EvalParams()
+        ep.theta = _ptr(self.theta)
+        return self._evaluate(eval_env, episodes, self.env._lib.mdpp_continuous_ars_eval,
+                              ep, per_env)
+
     def update(self):
         """One ARS step per config group from the fitness since the last
         update; then fitness restarts at 0 and the iteration advances.

@@ -133,6 +133,69 @@ continuous_ars_kernel(const __grid_constant__ ArsParams p) {
   continuous_body<R, MDPP_NOISE_PHILOX, GROUPS, ArsAgent<R>>(p);
 }
 
+// ---- evaluation of theta (mdpp_continuous_ars_eval) -------------------------
+// a = theta_g [obs; 1]: ArsAgent's policy with noise_std = 0, read straight
+// from the shared-memory copy of theta_g (no delta, no per-thread weights, no
+// fitness); the first ev.episodes episodes go to EvalEpisodes.
+struct ArsEvalParams : ContinuousParams {
+  const double* theta;  // [G][P]
+  EvalDev ev;
+};
+
+template <typename R>
+struct ArsEvalAgent {
+  static constexpr bool kActs = true;
+  using Params = ArsEvalParams;
+  const ArsEvalParams& p;
+  const double* th;  // theta of the CTA's group, in shared memory
+  EvalEpisodes ep;
+
+  __device__ __forceinline__ explicit ArsEvalAgent(const ArsEvalParams& p_) : p(p_) {}
+
+  __device__ __forceinline__ void begin(const ContinuousGroupSel& sel,
+                                        const mdpp_continuous_config&, int D) {
+    __shared__ double th_s[kArsMaxP];
+    const int P = D * (D + 1);
+    const double* src = p.theta + (int64_t)sel.group * P;
+    for (int j = threadIdx.x; j < P; j += kCBlock) th_s[j] = src[j];
+    __syncthreads();
+    th = th_s;
+    ep.begin();
+  }
+
+  // ArsAgent::act's sums, casts and clipping, on theta (written out again:
+  // the learner's kernels keep their code as it was)
+  __device__ __forceinline__ void act(const R* em, int D, R amax, int64_t, R* out) const {
+    const bool bounded = isfinite((double)amax);
+#pragma unroll
+    for (int d = 0; d < MDPP_MAX_DIM; ++d)
+      if (d < D) {
+        const double* wd = th + d * (D + 1);
+        double acc = __dmul_rn(wd[0], (double)em[0]);
+#pragma unroll
+        for (int k = 1; k < MDPP_MAX_DIM; ++k)
+          if (k < D) acc = __dadd_rn(acc, __dmul_rn(wd[k], (double)em[k]));
+        acc = __dadd_rn(acc, wd[D]);
+        R a = (R)acc;
+        if (bounded) a = a < -amax ? -amax : (a > amax ? amax : a);
+        out[d] = a;
+      }
+  }
+
+  // (autoreset is required: `reset` is terminated or truncated)
+  __device__ __forceinline__ void step(R out_r, bool reset) {
+    ep.step(p.ev, (double)out_r, reset);
+  }
+
+  __device__ __forceinline__ void end(int64_t env) const { ep.end(p.ev, env); }
+};
+
+template <typename R, bool GROUPS>
+__global__ void __launch_bounds__(kCBlock)
+continuous_ars_eval_kernel(const __grid_constant__ ArsEvalParams p) {
+  continuous_body<R, MDPP_NOISE_PHILOX, GROUPS, ArsEvalAgent<R>>(p);
+}
+
 // ---- the update --------------------------------------------------------------
 struct ArsUpdateParams {
   const ContinuousGroupDev* groups;  // NULL: one group of all n_envs
@@ -317,6 +380,38 @@ extern "C" int mdpp_continuous_ars(mdpp_ctx* ctx, const mdpp_continuous_state* s
     const unsigned grid = (unsigned)((k.st.n_envs + kCBlock - 1) / kCBlock);
     if (f64) continuous_ars_kernel<double, false><<<grid, kCBlock, 0, s>>>(k);
     else continuous_ars_kernel<float, false><<<grid, kCBlock, 0, s>>>(k);
+  }
+  MDPP_CUDA(ctx, cudaGetLastError());
+  return MDPP_OK;
+}
+
+extern "C" int mdpp_continuous_ars_eval(mdpp_ctx* ctx, const mdpp_continuous_state* st,
+                                        const mdpp_continuous_io* io,
+                                        const mdpp_eval_params* ep,
+                                        const mdpp_step_opts* opts, void* cuda_stream) {
+  ArsEvalParams k;
+  int rc = fill_continuous_params(ctx, st, opts, &k);
+  if (rc) return rc;
+  if (!io) return fail(ctx, MDPP_EINVAL, "ars eval: io is NULL");
+  if (ctx->c_cfg.image_mode)
+    return fail(ctx, MDPP_EINVAL, "ars eval: image observations are not supported");
+  rc = check_eval_params(ctx, "ars eval", io->actions != nullptr, opts, ep, -1, 0, &k.ev);
+  if (rc) return rc;
+  if (((uintptr_t)io->obs | (uintptr_t)io->final_obs) & 15)
+    return fail(ctx, MDPP_EINVAL, "obs / final_obs must be 16-byte aligned");
+  k.io = *io;
+  k.theta = ep->theta;
+  MDPP_CUDA(ctx, cudaSetDevice(ctx->device));
+  cudaStream_t s = (cudaStream_t)cuda_stream;
+  const bool f64 = ctx->c_cfg.is_f64;
+  if (k.groups) {
+    const unsigned grid = (unsigned)ctx->c_set.n_ctas;
+    if (f64) continuous_ars_eval_kernel<double, true><<<grid, kCBlock, 0, s>>>(k);
+    else continuous_ars_eval_kernel<float, true><<<grid, kCBlock, 0, s>>>(k);
+  } else {
+    const unsigned grid = (unsigned)((k.st.n_envs + kCBlock - 1) / kCBlock);
+    if (f64) continuous_ars_eval_kernel<double, false><<<grid, kCBlock, 0, s>>>(k);
+    else continuous_ars_eval_kernel<float, false><<<grid, kCBlock, 0, s>>>(k);
   }
   MDPP_CUDA(ctx, cudaGetLastError());
   return MDPP_OK;

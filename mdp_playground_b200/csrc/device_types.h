@@ -95,6 +95,57 @@ struct ReturnsDev {
   int32_t* ret_count;
 };
 
+// Device view of the outputs of mdpp_eval_params (qlearn.cu check_eval_params):
+// per env, the return sum, count and length sum of the first `episodes`
+// episodes of an evaluation launch.
+struct EvalDev {
+  double* ret_sum;
+  int32_t* ret_count;
+  int64_t* len_sum;
+  int32_t episodes;
+};
+
+// One env's evaluation episodes, kept in registers over the launch.  The env
+// starts a fresh episode at the launch's first step (the caller resets it);
+// an episode ends on terminated or truncated (auto-reset), and only the
+// first `episodes` are added.
+struct EvalEpisodes {
+  double ret, sum;   // running episode's return; sum over the counted ones
+  int64_t len_sum;
+  int32_t len, count;
+
+  __device__ __forceinline__ void begin() {
+    ret = sum = 0.0;
+    len_sum = 0;
+    len = count = 0;
+  }
+  __device__ __forceinline__ void step(const EvalDev& d, double r, bool ended) {
+    if (count < d.episodes) {
+      ret = __dadd_rn(ret, r);
+      len += 1;
+      if (ended) {
+        sum = __dadd_rn(sum, ret);
+        len_sum += len;
+        count += 1;
+        ret = 0.0;
+        len = 0;
+      }
+    }
+  }
+  __device__ __forceinline__ void end(const EvalDev& d, int64_t env) const {
+    d.ret_sum[env] = sum;
+    d.ret_count[env] = count;
+    d.len_sum[env] = len_sum;
+  }
+};
+
+// Device view of mdpp_eval_params for the greedy tabular agents.
+struct QevalDev {
+  const double* q;
+  int32_t q_states, q_actions;
+  EvalDev ev;
+};
+
 // Device view of mdpp_qlearn_params (qlearn.cu check_qlearn_params).
 struct QlearnDev {
   double* q;

@@ -556,6 +556,42 @@ struct GridQAgent : TabularQ<2 * ND + 1> {
   }
 };
 
+// ---- greedy evaluation (mdpp_grid_qeval) ------------------------------------
+// a = argmax Q[s] (GreedyQ, tabular_q.cuh): no STREAM_GRID_ACTION draw.
+struct GridQevalParams : GridParams {
+  QevalDev q;
+};
+
+template <int ND>
+struct GridQEvalAgent : GreedyQ<2 * ND + 1> {
+  using Q = GreedyQ<2 * ND + 1>;
+  using Q::greedy;
+  static constexpr bool kActs = true;
+  static constexpr int kMinBlocks = 4;  // the learner's: one wave at 65 536 envs
+  using Params = GridQevalParams;
+  static constexpr int A = 2 * ND + 1;
+
+  __device__ __forceinline__ explicit GridQEvalAgent(const GridQevalParams& p) : Q(p.q) {}
+
+  __device__ __forceinline__ void begin(const mdpp_grid_config& c, int64_t env,
+                                        const int32_t* pos) {
+    Q::begin(env, [&] { return cell_index<ND>(c, pos); }, A);
+  }
+
+  // the greedy action, packed like pack_action
+  __device__ __forceinline__ uint32_t act(const GridParams&, uint32_t, uint64_t) const {
+    const int32_t a = greedy;
+    constexpr uint32_t noop = ND == 2 ? 0x5u : 0x55u;
+    const uint32_t one = 1u << (2 * ((a - 1) >> 1));
+    return a == 0 ? noop : (a & 1) ? noop - one : noop + one;
+  }
+
+  __device__ __forceinline__ void update(const GridParams& p, const mdpp_grid_config& c,
+                                         const StepOut& o, const int32_t* pos_after,
+                                         int64_t, int64_t) {
+    Q::update(p, o, A, [&] { return cell_index<ND>(c, pos_after); });
+  }
+};
 
 }  // namespace mdpp
 
@@ -788,4 +824,32 @@ extern "C" int mdpp_grid_qlearn(mdpp_ctx* ctx, const mdpp_grid_state* st,
                    : launch_grid_philox<2, false, true, GridQAgent<2>>(ctx, k, s);
   return nd == 4 ? launch_grid_philox<4, false, false, GridQAgent<4>>(ctx, k, s)
                  : launch_grid_philox<2, false, false, GridQAgent<2>>(ctx, k, s);
+}
+
+extern "C" int mdpp_grid_qeval(mdpp_ctx* ctx, const mdpp_grid_state* st,
+                               const mdpp_grid_io* io, const mdpp_eval_params* ep,
+                               const mdpp_step_opts* opts, void* cuda_stream) {
+  GridQevalParams k;
+  int rc = fill_grid(ctx, st, opts, &k);
+  if (rc) return rc;
+  if (!io) return fail(ctx, MDPP_EINVAL, "grid qeval: io is NULL");
+  if (ctx->g_states > INT32_MAX)
+    return fail(ctx, MDPP_EINVAL, "grid qeval: a group has more than 2^31 - 1 cells");
+  const int nd = ctx->g_cfg.n_dims;
+  rc = check_eval_params(ctx, "grid qeval", io->actions != nullptr, opts, ep, ctx->g_states,
+                         2 * nd + 1, &k.q.ev);
+  if (rc) return rc;
+  if (((uintptr_t)io->obs | (uintptr_t)io->final_obs) & 15)
+    return fail(ctx, MDPP_EINVAL, "grid rows must be 16-byte aligned");
+  k.q.q = ep->q;
+  k.q.q_states = ep->q_states;
+  k.q.q_actions = ep->q_actions;
+  k.io = *io;
+  MDPP_CUDA(ctx, cudaSetDevice(ctx->device));
+  cudaStream_t s = (cudaStream_t)cuda_stream;
+  if (k.groups)
+    return nd == 4 ? launch_grid_philox<4, false, true, GridQEvalAgent<4>>(ctx, k, s)
+                   : launch_grid_philox<2, false, true, GridQEvalAgent<2>>(ctx, k, s);
+  return nd == 4 ? launch_grid_philox<4, false, false, GridQEvalAgent<4>>(ctx, k, s)
+                 : launch_grid_philox<2, false, false, GridQEvalAgent<2>>(ctx, k, s);
 }

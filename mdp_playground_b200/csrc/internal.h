@@ -95,6 +95,13 @@ int fill_continuous_params(mdpp_ctx* ctx, const mdpp_continuous_state* st,
                            const mdpp_step_opts* opts, ContinuousParams* p);
 int check_qlearn_params(mdpp_ctx* ctx, const mdpp_qlearn_params* qp, int64_t n_states,
                         int64_t n_actions, QlearnDev* d);
+// The checks of the evaluation entry points (mdpp_discrete_qeval,
+// mdpp_grid_qeval, mdpp_continuous_ars_eval): the launch options, the episode
+// count and the output arrays, and the Q-table against the groups' S / A
+// (n_states >= 0) or theta (n_states < 0); then the outputs' device view
+int check_eval_params(mdpp_ctx* ctx, const char* who, bool has_actions,
+                      const mdpp_step_opts* opts, const mdpp_eval_params* ep,
+                      int64_t n_states, int64_t n_actions, EvalDev* d);
 
 // Checks that groups[0..n) cover [0, N) contiguously, in order, with N >= 1, and
 // that a set with an env -> group map has at most 65 535 groups (uint16).

@@ -8,6 +8,29 @@
 
 namespace mdpp {
 
+// (max, lowest argmax) of a Q row; numpy.argmax order.  A > 0: A entries
+// known at compile time, scanned fully unrolled; A == 0: `n` entries, a
+// run-time bound (unrolled by 4).
+template <int A>
+__device__ __forceinline__ int32_t row_argmax(const double* row, int n, double& m) {
+  m = row[0];
+  int32_t am = 0;
+  if constexpr (A > 0) {
+#pragma unroll
+    for (int k = 1; k < A; ++k) {
+      const double x = row[k];
+      if (x > m) { m = x; am = k; }
+    }
+  } else {
+#pragma unroll 4
+    for (int k = 1; k < n; ++k) {
+      const double x = row[k];
+      if (x > m) { m = x; am = k; }
+    }
+  }
+  return am;
+}
+
 // One env's tabular Q-learner.  Per step (state s, action a):
 //   target = terminated ? r : r + gamma * max_a' Q[nxt][a']
 //   Q[s][a] = q + alpha * (target - q)
@@ -33,23 +56,7 @@ struct TabularQ {
 
   // (max, lowest argmax) of row st; numpy.argmax order
   __device__ __forceinline__ int32_t row_argmax(int32_t st, int n, double& m) const {
-    const double* row = tab + (int64_t)st * d.q_actions;
-    m = row[0];
-    int32_t am = 0;
-    if constexpr (A > 0) {
-#pragma unroll
-      for (int k = 1; k < A; ++k) {
-        const double x = row[k];
-        if (x > m) { m = x; am = k; }
-      }
-    } else {
-#pragma unroll 4
-      for (int k = 1; k < n; ++k) {
-        const double x = row[k];
-        if (x > m) { m = x; am = k; }
-      }
-    }
-    return am;
+    return mdpp::row_argmax<A>(tab + (int64_t)st * d.q_actions, n, m);
   }
 
   // state(): the env's state at the start of the launch
@@ -99,6 +106,43 @@ struct TabularQ {
   }
 
   __device__ __forceinline__ void end(int64_t env) { d.ret.ep_return[env] = ep_ret; }
+};
+
+// One env's greedy policy over a fixed Q-table, for the evaluation launches
+// (mdpp_discrete_qeval, mdpp_grid_qeval): the action is always
+// argmax_a Q[s][a] (lowest index on ties), Q is only read, and the return and
+// length of the first ev.episodes episodes go to EvalEpisodes.  Per step one
+// row is loaded: that of the state the env is in after the step (o.nxt, or
+// state_after() after an auto-reset), whose argmax is the next action.
+template <int A>
+struct GreedyQ {
+  const QevalDev& d;
+  const double* tab;  // this env's Q-table
+  int32_t greedy;     // argmax of the current state's row
+  EvalEpisodes ep;
+
+  __device__ __forceinline__ explicit GreedyQ(const QevalDev& dev) : d(dev) {}
+
+  __device__ __forceinline__ int32_t argmax_of(int32_t st, int n) const {
+    double m;
+    return row_argmax<A>(tab + (int64_t)st * d.q_actions, n, m);
+  }
+
+  template <typename F>
+  __device__ __forceinline__ void begin(int64_t env, F state, int n) {
+    tab = d.q + env * (int64_t)d.q_states * d.q_actions;
+    greedy = argmax_of(state(), n);
+    ep.begin();
+  }
+
+  template <typename P, typename F>
+  __device__ __forceinline__ void update(const P& p, const StepOut& o, int n, F state_after) {
+    const bool ended = o.done || o.trunc;
+    greedy = argmax_of(autoreset_of(p) && ended ? state_after() : o.nxt, n);
+    ep.step(d.ev, o.r, ended);
+  }
+
+  __device__ __forceinline__ void end(int64_t env) const { ep.end(d.ev, env); }
 };
 
 }  // namespace mdpp

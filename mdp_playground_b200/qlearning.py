@@ -93,6 +93,72 @@ class EpisodeReturns:
         env._step_index += T
         return out if record else None
 
+    # -- evaluation -------------------------------------------------------------
+    def _check_eval_env(self, eval_env):
+        """ValueError unless eval_env has the training env's layout: class,
+        env count, group sizes and the learner's per-group shapes
+        (_check_eval_layout), Philox noise, no images, autoreset and a
+        horizon (which bounds every episode, so E * horizon steps complete
+        E episodes)."""
+        env, name = self.env, type(self).__name__
+        if type(eval_env) is not type(env):
+            raise ValueError(f"{name}.evaluate: eval_env is a {type(eval_env).__name__}, "
+                             f"the learner's env a {type(env).__name__}")
+        if eval_env.num_envs != env.num_envs or \
+                list(eval_env._group_sizes) != list(env._group_sizes):
+            raise ValueError(f"{name}.evaluate: eval_env has {eval_env.num_envs} envs in "
+                             f"groups {list(eval_env._group_sizes)}, the learner's env "
+                             f"{env.num_envs} in {list(env._group_sizes)}")
+        self._check_eval_layout(eval_env)
+        if eval_env.noise != "philox":
+            raise ValueError(f"{name}.evaluate: eval_env needs noise='philox' "
+                             f"(got {eval_env.noise!r})")
+        if any(s_.image_representations for s_ in eval_env._group_specs):
+            raise ValueError(f"{name}.evaluate: eval_env has image_representations")
+        if not eval_env.autoreset or eval_env.horizon < 1:
+            raise ValueError(f"{name}.evaluate: eval_env needs autoreset=True and a "
+                             "horizon >= 1")
+
+    def _evaluate(self, eval_env, episodes, entry, params, per_env):
+        """One evaluation launch of `entry` with `params` (an _lib.EvalParams
+        holding the policy) on eval_env, after eval_env.reset()."""
+        E = int(episodes)
+        if E < 1:
+            raise ValueError(f"episodes must be >= 1, got {episodes}")
+        self._check_eval_env(eval_env)
+        eval_env.reset()
+        N, dev = eval_env.num_envs, eval_env.device
+        T = E * eval_env.horizon
+        ret_sum = torch.empty(N, dtype=torch.float64, device=dev)
+        ret_count = torch.empty(N, dtype=torch.int32, device=dev)
+        len_sum = torch.empty(N, dtype=torch.int64, device=dev)
+        params.episodes = E
+        params.ret_sum, params.ret_count = _ptr(ret_sum), _ptr(ret_count)
+        params.len_sum = _ptr(len_sum)
+        io = eval_env._io(None, {})
+        opts = eval_env._opts(T, noise_mode=_lib.MDPP_NOISE_PHILOX)
+        eval_env._check(entry(eval_env._ctx, C.byref(eval_env._state), C.byref(io),
+                              C.byref(params), C.byref(opts), eval_env._stream()))
+        eval_env._step_index += T
+        # every episode is at most `horizon` steps long, so E * horizon steps
+        # complete E of them in every env
+        if not bool((ret_count == E).all()):
+            raise RuntimeError(f"evaluate: an env completed {int(ret_count.min())} of "
+                               f"{E} episodes in {T} steps")
+        group = torch.repeat_interleave(
+            torch.arange(eval_env.n_groups, device=dev),
+            torch.tensor(eval_env._group_sizes, device=dev))
+        per_group = torch.zeros((3, eval_env.n_groups), dtype=torch.float64, device=dev)
+        per_group[0].index_add_(0, group, ret_count.to(torch.float64))
+        per_group[1].index_add_(0, group, ret_sum)
+        per_group[2].index_add_(0, group, len_sum.to(torch.float64))
+        ep, tot, length = per_group.cpu().numpy()
+        out = {"episodes": ep, "episode_reward_mean": tot / ep,
+               "episode_len_mean": length / ep}
+        if per_env:
+            out.update(ret_sum=ret_sum, ret_count=ret_count, len_sum=len_sum)
+        return out
+
     def episode_returns(self, clear=False):
         """Per config group: "episodes" completed by an auto-reset since the
         last clear, and their mean return "episode_reward_mean" (NaN when
@@ -145,8 +211,20 @@ class TabularQLearner(EpisodeReturns):
         tables = self.env.group_tables
         return max(t.n_states for t in tables), max(t.n_actions for t in tables)
 
+    def _check_eval_layout(self, eval_env):
+        if eval_env._irr:
+            raise ValueError("TabularQLearner.evaluate: eval_env has irrelevant_features")
+        shapes = [[(t.n_states, t.n_actions) for t in e.group_tables]
+                  for e in (self.env, eval_env)]
+        if shapes[0] != shapes[1]:
+            raise ValueError("TabularQLearner.evaluate: eval_env's groups have (S, A) "
+                             f"{shapes[1]}, the learner's {shapes[0]}")
+
     def _entry(self):
         return self.env._lib.mdpp_discrete_qlearn
+
+    def _eval_entry(self):
+        return self.env._lib.mdpp_discrete_qeval
 
     def _before_launch(self):
         pass
@@ -161,7 +239,8 @@ class TabularQLearner(EpisodeReturns):
         truncated and the actions taken (GridQLearner: int64 [T, N, n_dims]
         action rows, which env.rollout(actions=...) accepts).  alpha / gamma
         / epsilon override the constructor's values for this call (e.g.
-        epsilon=0, alpha=0 for a greedy evaluation that leaves q unchanged)."""
+        epsilon=0, alpha=0 for a greedy run that leaves q unchanged; evaluate()
+        measures the greedy policy on a separate evaluation env)."""
         T = int(n_steps)
         self._before_launch()
         qp = self._new_params(_lib.QlearnParams)
@@ -174,6 +253,22 @@ class TabularQLearner(EpisodeReturns):
         if record:
             out["actions"] = self._actions_out(out["actions"])
         return out
+
+    def evaluate(self, eval_env, episodes=10, per_env=False):
+        """The greedy policy of the current q (argmax, lowest index on ties;
+        no exploration, q only read) on eval_env, an env built like the
+        learner's (typically without its noises): eval_env.reset(), then one
+        launch of episodes * eval_env.horizon steps in which the first
+        `episodes` episodes of every env are counted.  Leaves q, the
+        training env and episode_returns untouched.  Returns per config
+        group (numpy [G]): "episodes" counted, and their mean return
+        "episode_reward_mean" and mean length "episode_len_mean"; with
+        per_env=True also the per-env device tensors "ret_sum", "ret_count"
+        and "len_sum"."""
+        ep = _lib.EvalParams()
+        ep.q = _ptr(self.q)
+        ep.q_states, ep.q_actions = self.q.shape[1], self.q.shape[2]
+        return self._evaluate(eval_env, episodes, self._eval_entry(), ep, per_env)
 
 
 class GridQLearner(TabularQLearner):
@@ -205,8 +300,18 @@ class GridQLearner(TabularQLearner):
         return (max(grid_cells(s_.grid_shape) for s_ in env._group_specs),
                 8 if env._nd == 2 else 9)
 
+    def _check_eval_layout(self, eval_env):
+        shapes = [[tuple(s_.grid_shape) for s_ in e._group_specs]
+                  for e in (self.env, eval_env)]
+        if shapes[0] != shapes[1]:
+            raise ValueError(f"GridQLearner.evaluate: eval_env's grid shapes {shapes[1]} "
+                             f"differ from the learner's {shapes[0]}")
+
     def _entry(self):
         return self.env._lib.mdpp_grid_qlearn
+
+    def _eval_entry(self):
+        return self.env._lib.mdpp_grid_qeval
 
     def _before_launch(self):
         pos = self.env._pos

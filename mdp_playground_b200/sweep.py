@@ -107,6 +107,101 @@ def env_grid(module):
     return env_keys, out
 
 
+class _NormalProbe:
+    """Stands in for the numpy Generator that the reference passes to a noise
+    callable: records every call made on it."""
+
+    def __init__(self):
+        self.calls = []
+
+    def __getattr__(self, name):
+        if name.startswith("__"):
+            raise AttributeError(name)
+
+        def record(*args, **kwargs):
+            self.calls.append((name, args, kwargs))
+            return self
+        return record
+
+
+def noise_std(key, f):
+    """The sigma of a noise callable of the reference's evaluation configs,
+    `tune.function(lambda a: a.normal(0, sigma))`: one `normal(0, sigma)`
+    call with constant arguments, whose draw is the callable's value.
+    Anything else raises NotImplementedError naming `key`."""
+    probe = _NormalProbe()
+    try:
+        out = f(probe)
+    except Exception as e:
+        raise NotImplementedError(
+            f"evaluation env_config[{key!r}]: only lambda a: a.normal(0, sigma) is "
+            f"supported (calling it raised {type(e).__name__})") from None
+    ok = out is probe and len(probe.calls) == 1 and probe.calls[0][0] == "normal"
+    if ok:
+        _, args, kwargs = probe.calls[0]
+        names = ("loc", "scale")
+        ok = len(args) <= 2 and set(kwargs) <= set(names[len(args):])
+        if ok:
+            vals = dict(zip(names, args), **kwargs)
+            loc, scale = vals.get("loc", 0.0), vals.get("scale", 1.0)
+            ok = all(isinstance(v, (int, float, np.integer, np.floating))
+                     and not isinstance(v, bool) for v in (loc, scale)) \
+                and float(loc) == 0.0 and np.isfinite(scale) and float(scale) >= 0.0
+    if not ok:
+        raise NotImplementedError(
+            f"evaluation env_config[{key!r}]: only lambda a: a.normal(0, sigma) with "
+            f"constant sigma >= 0 is supported (got calls {probe.calls})")
+    return float(scale)
+
+
+# keys of the reference's evaluation_config that configure the agent, not the env
+_AGENT_EVAL_KEYS = ("explore",)
+
+
+def eval_settings(module, evaluation, horizon):
+    """The evaluation of an experiment: the module's `eval_config` (the
+    reference's RLlib layout: top-level "evaluation_interval", and in
+    "evaluation_config" "evaluation_num_episodes", "horizon" and the
+    "env_config" overrides; agent keys such as "explore" and
+    "exploration_*" are ignored), with the entries of a dict `evaluation`
+    on top (the same four names, "env_config" merged key by key).
+    Noise callables become their sigma (noise_std).  Returns a dict of
+    "interval", "episodes", "horizon" and "env_config"."""
+    ec = copy.deepcopy(getattr(module, "eval_config", None) or {})
+    inner = ec.get("evaluation_config", {}) or {}
+    out = {"interval": ec.get("evaluation_interval", 1),
+           "episodes": inner.get("evaluation_num_episodes",
+                                 ec.get("evaluation_num_episodes", 10)),
+           "horizon": inner.get("horizon", horizon),
+           "env_config": dict(inner.get("env_config", {}) or {})}
+    if isinstance(evaluation, dict):
+        known = {"evaluation_interval", "evaluation_num_episodes", "horizon", "env_config"}
+        if set(evaluation) - known:
+            raise ValueError(f"evaluation: unknown keys {sorted(set(evaluation) - known)} "
+                             f"(known: {sorted(known)})")
+        out["interval"] = evaluation.get("evaluation_interval", out["interval"])
+        out["episodes"] = evaluation.get("evaluation_num_episodes", out["episodes"])
+        out["horizon"] = evaluation.get("horizon", out["horizon"])
+        out["env_config"].update(evaluation.get("env_config", {}) or {})
+    for key in ("interval", "episodes", "horizon"):
+        v = out[key]
+        if isinstance(v, bool) or not isinstance(v, (int, np.integer)) or v < 1:
+            raise ValueError(f"evaluation {key} must be an integer >= 1, got {v!r}")
+        out[key] = int(v)
+    env_cfg = {}
+    for k, v in out["env_config"].items():
+        if k in _AGENT_EVAL_KEYS or k.startswith("exploration_"):
+            continue
+        env_cfg[k] = noise_std(k, v) if callable(v) else v
+    out["env_config"] = env_cfg
+    return out
+
+
+def eval_cell_configs(cell_configs, env_config):
+    """Each cell's config with the evaluation's env overrides on top."""
+    return [dict(copy.deepcopy(c), **copy.deepcopy(env_config)) for c in cell_configs]
+
+
 class Sweep:
     """All cells of an experiment's env grid in one VectorRLToyEnv."""
 
@@ -125,6 +220,7 @@ class Sweep:
                  for c in self.cell_configs}
         assert len(kinds) == 1, "one state_space_type per experiment file"
         self.kind = kinds.pop()
+        self._env_args = (device, shard, env_kwargs)
         if self.kind == "discrete":
             # the whole grid is ONE heterogeneous env: one launch per rollout
             self.env = VectorRLToyEnv(
@@ -140,19 +236,46 @@ class Sweep:
             # dimension or dtype; grid: irrelevant_features) take one
             # configuration per context: one env per cell, launched back to
             # back on the same stream
-            rank, world = shard
-            self.envs = [VectorRLToyEnv(
-                self.envs_per_cell, device=device, autoreset=True,
-                horizon=horizon,
-                env_id_offset=(i * world + rank) * self.envs_per_cell,
-                **env_kwargs, **copy.deepcopy(c))
-                for i, c in enumerate(self.cell_configs)]
+            self.envs = self._per_cell_envs(self.cell_configs, horizon)
             self.env = self.envs[0]
         self.timesteps = 0
         self._returned = np.zeros(self.n_cells)
         self.agents = None  # one learner per env of self.envs
         self.algorithm = None  # the learner's name in write_csv once one has trained
         self.train_results = []  # one dict per training iteration
+        self.eval_envs = None  # evaluation envs, laid out like self.envs
+        self.evaluation = None  # eval_settings() of the first train(evaluation=...)
+        self.eval_results = []  # one dict per evaluated training iteration
+
+    def _per_cell_envs(self, cell_configs, horizon):
+        from .vector_env import VectorRLToyEnv
+        device, (rank, world), env_kwargs = self._env_args
+        return [VectorRLToyEnv(
+            self.envs_per_cell, device=device, autoreset=True,
+            horizon=horizon,
+            env_id_offset=(i * world + rank) * self.envs_per_cell,
+            **env_kwargs, **copy.deepcopy(c))
+            for i, c in enumerate(cell_configs)]
+
+    def _build_eval_envs(self, evaluation):
+        """The evaluation envs, once: the layout of self.envs (one grouped
+        env, or one env per cell with the same env ids), each cell's config
+        with the evaluation's env overrides on top."""
+        if self.eval_envs is not None:
+            return
+        from .vector_env import VectorRLToyEnv
+        self.evaluation = eval_settings(self.module, evaluation, self.env.horizon)
+        cfgs = eval_cell_configs(self.cell_configs, self.evaluation["env_config"])
+        horizon = self.evaluation["horizon"]
+        device, shard, env_kwargs = self._env_args
+        if self.kind == "discrete" or getattr(self, "grouped", False):
+            self.eval_envs = [VectorRLToyEnv(
+                self.n_cells * self.envs_per_cell, device=device, autoreset=True,
+                horizon=horizon, config_groups=cfgs,
+                group_sizes=[self.envs_per_cell] * self.n_cells, shard=shard,
+                **env_kwargs)]
+        else:
+            self.eval_envs = self._per_cell_envs(cfgs, horizon)
 
     def _try_grouped(self, Env, device, horizon, shard, env_kwargs):
         """Continuous cells that share dim / dtype / reward function, and grid
@@ -205,7 +328,7 @@ class Sweep:
         return self.results()
 
     def train(self, iterations, steps_per_iteration, alpha=0.1, gamma=0.99,
-              epsilon=0.1, chunk=256):
+              epsilon=0.1, chunk=256, evaluation=None):
         """Tabular Q-learning (one agent per env; envs_per_cell seeds per
         cell), `iterations` times `steps_per_iteration` steps per env.  Each
         iteration appends to `train_results`, per cell: the cumulative
@@ -213,22 +336,34 @@ class Sweep:
         completed in the iteration; NaN if none) and episode_len_mean (from
         the episode counters' change over the iteration).  Discrete grids
         only (grid-world experiments: train_grid).  Calling train again
-        continues with the same Q-tables."""
+        continues with the same Q-tables.
+
+        evaluation: None (none), True (the experiment file's eval_config) or
+        a dict overriding it (eval_settings).  Every evaluation_interval-th
+        iteration then evaluates every agent's greedy policy
+        (TabularQLearner.evaluate) on evaluation envs built once like the
+        training envs, with the evaluation's env_config on top of each
+        cell's config, and appends to `eval_results`, per cell: the
+        training_iteration, its timesteps_total, and the evaluation
+        episodes' episode_reward_mean and episode_len_mean (write_eval_csv).
+        The settings and envs of the first evaluating call are kept.
+        Rank-local, like train_results."""
         return self._train_q(
             "discrete", "Sweep.train: tabular Q-learning runs on discrete grids only "
             "(grid-world experiments: Sweep.train_grid)",
-            iterations, steps_per_iteration, alpha, gamma, epsilon, chunk)
+            iterations, steps_per_iteration, alpha, gamma, epsilon, chunk, evaluation)
 
     def train_grid(self, iterations, steps_per_iteration, alpha=0.1, gamma=0.99,
-                   epsilon=0.1, chunk=256):
+                   epsilon=0.1, chunk=256, evaluation=None):
         """train() for grid-world experiments (GridQLearner): one learner on
         the grouped env, or one per cell when the cells differ in
         irrelevant_features; results in cell order either way."""
         return self._train_q("grid", "Sweep.train_grid: runs grid-world experiments only",
-                             iterations, steps_per_iteration, alpha, gamma, epsilon, chunk)
+                             iterations, steps_per_iteration, alpha, gamma, epsilon, chunk,
+                             evaluation)
 
     def _train_q(self, kind, refusal, iterations, steps_per_iteration, alpha, gamma,
-                 epsilon, chunk):
+                 epsilon, chunk, evaluation=None):
         """train / train_grid: `refusal` is the NotImplementedError message
         for experiments of another kind than `kind`."""
         if self.kind != kind:
@@ -237,10 +372,10 @@ class Sweep:
         learner = GridQLearner if kind == "grid" else TabularQLearner
         kw = dict(alpha=alpha, gamma=gamma, epsilon=epsilon)
         return self._train(lambda e: learner(e, **kw), iterations, steps_per_iteration,
-                           chunk, kw, "TabularQLearning")
+                           chunk, kw, "TabularQLearning", evaluation=evaluation)
 
     def train_continuous(self, iterations, steps_per_iteration, step_size=0.02,
-                         noise_std=0.03, top_directions=None, chunk=256):
+                         noise_std=0.03, top_directions=None, chunk=256, evaluation=None):
         """train() for continuous experiments: augmented random search
         (ars.LinearARS), one linear policy per cell whose envs_per_cell envs
         (an even number) are the perturbation population.  One learner on the
@@ -248,7 +383,9 @@ class Sweep:
         dtype.  Each iteration runs `steps_per_iteration` steps per env (the
         learn chunks), then one ARS update per cell, and appends the same
         per-cell results as train().  Calling it again continues with the
-        same policies.  Not for sharded sweeps (the update is per rank)."""
+        same policies.  Not for sharded sweeps (the update is per rank).
+        evaluation: as in train(), evaluating theta itself
+        (LinearARS.evaluate)."""
         if self.kind != "continuous":
             raise NotImplementedError(
                 "Sweep.train_continuous: runs continuous experiments only")
@@ -260,13 +397,17 @@ class Sweep:
         return self._train(
             lambda e: LinearARS(e, step_size=step_size, noise_std=noise_std,
                                 top_directions=top_directions),
-            iterations, steps_per_iteration, chunk, {}, "ARS", update=True)
+            iterations, steps_per_iteration, chunk, {}, "ARS", update=True,
+            evaluation=evaluation)
 
     def _train(self, make, iterations, steps_per_iteration, chunk, learn_kw,
-               algorithm, update=False):
+               algorithm, update=False, evaluation=None):
         if self.agents is None:
             self.agents = [make(e) for e in self.envs]
         self.algorithm = algorithm
+        evaluate = evaluation is not None and evaluation is not False
+        if evaluate:
+            self._build_eval_envs(evaluation)
 
         def per_cell(dicts, key):  # one value per group of each env, in cell order
             return np.concatenate([np.asarray(d[key]).reshape(-1) for d in dicts])
@@ -293,6 +434,15 @@ class Sweep:
                 "timesteps_total": per_cell(after, "transitions"),
                 "episode_reward_mean": per_cell(ret, "episode_reward_mean"),
                 "episode_len_mean": d_tr / np.maximum(d_ep, 1)})
+            it = len(self.train_results)
+            if evaluate and it % self.evaluation["interval"] == 0:
+                ev = [ag.evaluate(e, self.evaluation["episodes"])
+                      for ag, e in zip(self.agents, self.eval_envs)]
+                self.eval_results.append({
+                    "training_iteration": it,
+                    "timesteps_total": per_cell(after, "transitions"),
+                    "episode_reward_mean": per_cell(ev, "episode_reward_mean"),
+                    "episode_len_mean": per_cell(ev, "episode_len_mean")})
         return self.train_results
 
     def _random_actions(self, env, T, t0):
@@ -366,6 +516,20 @@ class Sweep:
                       "episode_reward_mean": res["episode_reward_mean"],
                       "episode_len_mean": res["episode_len_mean"]}]
             algorithm = algorithm or "RandomPolicy"
+        return self._write_rows(path, iters, algorithm)
+
+    def write_eval_csv(self, path, algorithm=None):
+        """The evaluation results (eval_results) in write_csv's column
+        layout: one row per (evaluated training iteration, cell) with the
+        training iteration, its timesteps_total, and the evaluation
+        episodes' mean return and mean length.  The reference's callbacks
+        write evaluation episodes to a stats file of their own, which its
+        analysis code loads next to the training file; whether that file
+        has exactly these columns has not been checked against the
+        reference.  Rank-local, like write_csv."""
+        return self._write_rows(path, self.eval_results, algorithm or self.algorithm)
+
+    def _write_rows(self, path, iters, algorithm):
         with open(path, "w") as f:
             f.write("# training_iteration, algorithm, "
                     + "".join(k + ", " for k in self.env_keys)
